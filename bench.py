@@ -7,7 +7,7 @@ size; the library gathers one 128-byte partial sum per rank over NCCL and folds 
 Every line also carries `strong_2p26`: BASELINE configs[4], 2^26 points in total split over the N ranks
 by point range (the >= 6x at 8 GPUs target), verified on the device at every N.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log-n 20]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log-n 20] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  `value` is timed with CUDA events on the library's stream with
 points and scalars resident in HBM; `e2e` is the same MSM through the reference-facing C-ABI call
@@ -381,6 +381,17 @@ def groth16_record(log_k, peak_tmacs, comm=None):
     return res
 
 
+def dump_g1_point(out_dir, name, point):
+    """Writes an affine G1 result as out_dir/<name>.npy: float64 of shape (2, 8), the 32-bit limbs of x and y,
+    least significant first (every limb is exact in float64).  The point at infinity is all zeros, as in the
+    library's byte encoding."""
+    import numpy as np
+    x, y = point if point is not None else (0, 0)
+    limbs = [[(v >> (32 * j)) & 0xFFFFFFFF for j in range(8)] for v in (x, y)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), np.array(limbs, dtype=np.float64))
+
+
 # ------------------------------------------------------------------ our arm (GPU)
 def run_ours(args):
     rank = int(os.environ.get("RANK", "0"))
@@ -514,7 +525,7 @@ def run_ours(args):
     msm_us = 0.0
     nat.timer_start()
     for i in range(steps):
-        step_resident(warmup + i)
+        last = step_resident(warmup + i)
         acc_us += nat.msm_last_profile("accumulate")
         msm_us += nat.msm_last_profile(None)
     ms = nat.timer_stop()
@@ -527,6 +538,8 @@ def run_ours(args):
     value = total_points * steps / (ms * 1e-3) / 1e6
 
     nat.msm_profile(False)
+    if args.dump_outputs and rank == 0:
+        dump_g1_point(args.dump_outputs, "g1_msm", last)
 
     # for the record: the same MSMs submitted as ONE pipelined batch call (two streams: the tail of MSM k
     # overlaps the accumulation of MSM k+1), the call shape of a prover that commits in groups
@@ -748,7 +761,9 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline MSM and of its e2e record (the pipelined batch takes min(steps, 8)); "
+                         "the other sub-records (strong scaling, Groth16, PLONK, G2, NTT) time their own fixed counts")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--log-n", type=int, default=20, help="log2 of the points per GPU")
@@ -757,7 +772,15 @@ def main():
     ap.add_argument("--plain", action="store_true", help="do not precompute the window table")
     ap.add_argument("--no-extras", dest="extras", action="store_false", help="skip the Groth16 / PLONK / G2 / NTT sub-records")
     ap.add_argument("--no-cpu", dest="cpu", action="store_false", help="skip the CPU baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the affine point of the last timed headline MSM to DIR/g1_msm.npy (see dump_g1_point); "
+                         "the inputs depend only on the arguments, so two builds can be compared output for output. "
+                         "GPU arm only: --impl reference times a different, smaller sample and is refused")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":
