@@ -286,6 +286,23 @@ int zkp_fr_ap_interpolate_dev(uint64_t values, uint64_t off, uint64_t k, const u
 int zkp_fr_ap_vanishing_dev(uint64_t k, uint64_t out, uint64_t out_off);
 int zkp_fr_ap_lagrange_dev(uint64_t k, const uint8_t x[32], uint64_t out, uint64_t out_off);
 
+/* ---- pairings (verifier side) -------------------------------------------------------------------
+ * The BN254 optimal-Ate pairing of py_ecc's bn128.pairing(Q, P), Q in G2, P in G1, in the encodings above
+ * (csrc/pairing.cu).  Replaces the pairings of zkp/groth16/verifying.py:29-40 (e(A, B) == e(alpha, beta)
+ * e(sum r_i sigma1_3[i], gamma) e(C, delta)), zkp/plonk/verifier.py:42-208 (e(A, [tau]_2) == e(B, [1]_2)) and
+ * zkp/plonk/kzg.py:117-160 (verify_opening).  An input point that is not on its curve (or has a coordinate not
+ * below p) fails with ZKP_ERR_INVALID_ARGUMENT, as py_ecc's `assert is_on_curve` does.
+ * zkp_pairing: e(Q, P) as py_ecc's FQ12, 12 x 32 B canonical coefficients of w^0..w^11 (mod w^12 - 18 w^6 + 82);
+ * either input at infinity -> 1.
+ * zkp_pairing_check: *out_ok = [ prod_i e(Q_i, k_i P_i) == 1 ] over `count` pairs (g2s: count x 128 B, g1s:
+ * count x 64 B); scalars == NULL means k_i = 1, otherwise count x 32 B, reduced mod r; a pair with infinity on
+ * either side (also k_i P_i = infinity) contributes 1.  g2_subgroup_check != 0: any Q_i outside G2 ([r] Q_i !=
+ * infinity) makes *out_ok = 0.  count == 0 -> *out_ok = 1.  One Miller loop per pair on the device, one final
+ * exponentiation per call: the batch verifiers (verify_batch) check k proofs with one call. */
+int zkp_pairing(const uint8_t g2_xy[128], const uint8_t g1_xy[64], uint8_t out_fq12[384]);
+int zkp_pairing_check(const uint8_t* g2s, const uint8_t* g1s, const uint8_t* scalars, uint64_t count,
+                      int g2_subgroup_check, int* out_ok);
+
 /* ---- measurement helpers (bench.py) -----------------------------------------------------------
  * Per-stage CUDA-event profile of the most recent MSM (events recorded on the library stream).
  * zkp_msm_last_profile sums the stages whose name contains `stage` ("accumulate", "ws", "horner",

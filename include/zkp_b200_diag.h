@@ -37,6 +37,11 @@ int zkp_dbg_field_op(int field, int op, const uint8_t* a, const uint8_t* b, uint
 /* out[i] = a[i] + b[i] (group: 0 = G1, 1 = G2; 2 / 3 = the same through the quad-lane operations of
  * csrc/ec_quad.cuh) via XYZZ, result affine; exercises all edge cases */
 int zkp_dbg_point_add(int group, const uint8_t* a, const uint8_t* b, uint64_t n, uint8_t* out);
+/* Fp12 self-test hook (csrc/pairing.cu): n elements of 384 B each in py_ecc's FQ12 basis (12 canonical
+ * coefficients of w^0..w^11); op: 0 a * b, 1 a^2, 2 cyclotomic squaring (valid for a in the cyclotomic subgroup),
+ * 3 1 / a, 4 / 5 / 6 the Frobenius maps pi, pi^2, pi^3, 7 the final exponentiation a^((p^12 - 1) / r).
+ * b is read by op 0 only. */
+int zkp_dbg_fp12_op(int op, const uint8_t* a, const uint8_t* b, uint64_t n, uint8_t* out);
 /* Guarded allocation (start the process with ZKP_B200_GUARD=1): every device block of the library carries a
  * 512-byte canary zone on both sides; this checks the zones of all live blocks (blocks are also checked when
  * freed) and returns the number of live blocks and of blocks found damaged so far.  compute-sanitizer is closed

@@ -124,11 +124,14 @@ PROTOTYPES = {
     "zkp_msm_last_profile": (c_int, [ctypes.c_char_p, f32p]),
     "zkp_pinned_alloc": (c_int, [u64, ctypes.POINTER(ctypes.c_void_p)]),
     "zkp_pinned_free": (c_int, [vp]),
+    "zkp_pairing": (c_int, [vp, vp, vp]),
+    "zkp_pairing_check": (c_int, [vp, vp, vp, u64, c_int, intp]),
     "zkp_imad_peak": (c_int, [c_int, f64p, f64p]),
     "zkp_latency_probe": (c_int, [c_int, f64p]),
     "zkp_debug_check_guards": (c_int, [u64p, u64p]),
     "zkp_dbg_field_op": (c_int, [c_int, c_int, vp, vp, u64, vp]),
     "zkp_dbg_point_add": (c_int, [c_int, vp, vp, u64, vp]),
+    "zkp_dbg_fp12_op": (c_int, [c_int, vp, vp, u64, vp]),
 }
 
 ZKP_ERR_NOT_DIVISIBLE = -5

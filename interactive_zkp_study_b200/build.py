@@ -17,7 +17,7 @@ OBJ = os.path.join(HERE, "_build")
 LIB = os.path.join(HERE, "libzkp_b200.so")
 ROOT = os.path.dirname(HERE)
 
-UNITS = ["capi_core.cu", "comm.cu", "diag.cu", "msm_g1.cu", "msm_g2.cu", "ntt.cu", "poly.cu"]
+UNITS = ["capi_core.cu", "comm.cu", "diag.cu", "msm_g1.cu", "msm_g2.cu", "ntt.cu", "pairing.cu", "poly.cu"]
 
 NVCC_FLAGS = [
     "-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

@@ -13,7 +13,7 @@ field_modulus = 2188824287183927522224640574525727508869631115729782366268903789
 curve_order = 21888242871839275222246405745257275088548364400416034343698204186575808495617
 
 try:  # pragma: no cover - exercised only where py_ecc is installed
-    from py_ecc.fields import bn128_FQ as FQ, bn128_FQ2 as FQ2
+    from py_ecc.fields import bn128_FQ as FQ, bn128_FQ2 as FQ2, bn128_FQ12 as FQ12
     from py_ecc import bn128 as _bn128
     HAVE_PY_ECC = True
     G1, G2 = _bn128.G1, _bn128.G2
@@ -117,6 +117,56 @@ except ImportError:
 
         def __repr__(self):
             return repr(self.coeffs)
+
+    class FQ12(object):
+        """Element of Fp[w]/(w^12 - 18 w^6 + 82), py_ecc's pairing target: a value container for what
+        zkp.pairing.pairing returns, with the product and the equality the verifiers' e(..) * e(..) == e(..)
+        needs.  The pairings themselves run on the GPU (native.pairing)."""
+        degree = 12
+
+        def __init__(self, coeffs):
+            if len(coeffs) != 12:
+                raise Exception("FQ12 takes twelve coefficients")
+            self.coeffs = tuple(FQ(c) for c in coeffs)
+
+        def __mul__(self, o):
+            if isinstance(o, (int, FQ)):
+                return FQ12([c * o for c in self.coeffs])
+            if not isinstance(o, FQ12):
+                raise TypeError("Expected an FQ12, FQ or int")
+            a = [c.n for c in self.coeffs]
+            b = [c.n for c in o.coeffs]
+            t = [0] * 23
+            for i in range(12):
+                for j in range(12):
+                    t[i + j] += a[i] * b[j]
+            for k in range(22, 11, -1):      # w^12 = 18 w^6 - 82
+                t[k - 6] += 18 * t[k]
+                t[k - 12] -= 82 * t[k]
+            return FQ12(t[:12])
+
+        __rmul__ = __mul__
+
+        def __eq__(self, o):
+            if not isinstance(o, FQ12):
+                raise TypeError("Expected an FQ12 object")
+            return all(x == y for x, y in zip(self.coeffs, o.coeffs))
+
+        def __ne__(self, o):
+            return not self == o
+
+        __hash__ = None
+
+        def __repr__(self):
+            return repr(self.coeffs)
+
+        @classmethod
+        def one(cls):
+            return cls([1] + [0] * 11)
+
+        @classmethod
+        def zero(cls):
+            return cls([0] * 12)
 
     G1 = (FQ(1), FQ(2))
     G2 = (

@@ -511,6 +511,29 @@ def groth16_quotient(a_bytes, b_bytes, c_bytes, length, z_bytes, z_len):
     return bytes(h), bytes(r[:32 * (z_len - 1)])
 
 
+# ------------------------------------------------------------------ pairings (verifier side)
+def pairing(g2_b, g1_b):
+    """e(Q, P) for one G2 point (128 B) and one G1 point (64 B) -> py_ecc's FQ12 coefficients (12 ints, w^0..w^11)."""
+    out = bytearray(384)
+    check(_lib.lib().zkp_pairing(buf(bytes(g2_b)), buf(bytes(g1_b)), buf(out)))
+    return fr_vec_from_bytes(bytes(out), 12)
+
+
+def pairing_check(g2_b, g1_b, n, scalars=None, g2_subgroup_check=False):
+    """[ prod_i e(Q_i, k_i P_i) == 1 ] over n pairs (n x 128 B, n x 64 B; scalars: n x 32 B or None for k_i = 1)."""
+    ok = ctypes.c_int()
+    check(_lib.lib().zkp_pairing_check(buf(bytes(g2_b)) if n else None, buf(bytes(g1_b)) if n else None,
+                                       buf(bytes(scalars)) if scalars is not None and n else None, n,
+                                       1 if g2_subgroup_check else 0, ctypes.byref(ok)))
+    return bool(ok.value)
+
+
+def dbg_fp12_op(op, a_bytes, b_bytes, n):
+    out = bytearray(384 * n)
+    check(_lib.lib().zkp_dbg_fp12_op(op, buf(a_bytes), buf(b_bytes), n, buf(out)))
+    return bytes(out)
+
+
 # ------------------------------------------------------------------ diagnostics (tests)
 def debug_check_guards():
     """(live device blocks, blocks whose canaries were overwritten) -- needs ZKP_B200_GUARD=1 in the environment."""

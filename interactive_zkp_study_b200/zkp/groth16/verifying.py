@@ -1,9 +1,13 @@
 """Drop-in for /root/reference/zkp/groth16/verifying.py (SURVEY.md 8f-4: verifier-side group work).
 
 The public-wire combination sum_i r_i * sigma1_3[i] (:34-37) is one GPU MSM; the four pairings and the
-GT product stay on the CPU (O(1) per proof) and come from py_ecc -- where py_ecc is not installed a
-caller passes `pairing=` (the tests hand in the oracle's restatement)."""
+GT product of `verify` come from py_ecc -- where py_ecc is not installed a caller passes `pairing=`
+(zkp.pairing.pairing runs them on the GPU).
+
+`verify_batch` checks k proofs of one circuit at once: a random linear combination turns the k equations into
+one product of k + 3 pairings, decided by a single device call (zkp.pairing.pairing_check)."""
 from ... import native
+from ..pairing import batch_weights, pairing_check
 from ...compat import FQ, FR, G1, G2, HAVE_PY_ECC, curve_order, g1_from_ints  # noqa: F401
 
 g1 = G1
@@ -40,3 +44,34 @@ def verify(prf_A, prf_B, prf_C, sigma1_1, sigma1_3, sigma2_1, rx_pub, pairing=No
     """e(A, B) == e(alpha, beta) * e(sum r_i sigma1_3[i], gamma) * e(C, delta)   (reference :29-40);
     rx_pub = [(index_i, r_i), ...]."""
     return lhs(prf_A, prf_B, pairing) == rhs(prf_C, sigma1_1, sigma1_3, sigma2_1, rx_pub, pairing)
+
+
+def verify_batch(proofs, sigma1_1, sigma1_3, sigma2_1, rx_pubs, rng=None):
+    """True iff every proof j in `proofs` = [(A_j, B_j, C_j)] satisfies `verify` with public input rx_pubs[j]
+    (a list of (index, r_i) as for `verify`), up to a 2^-128 chance of accepting a bad batch.  With random
+    non-zero 128-bit weights rho_j (from `secrets`, or from rng.getrandbits for reproducible runs) it checks
+
+        prod_j e(rho_j A_j, B_j) * e(-(sum rho_j) alpha, beta) * e(-sum_j rho_j P_j, gamma) * e(-sum_j rho_j C_j, delta) == 1
+
+    (alpha = sigma1_1[0], (beta, gamma, delta) = sigma2_1[0..2], P_j = proof j's public-wire term): one GPU MSM
+    over sigma1_3 with the weights folded into the per-index scalars, one over the C_j, and one pairing check
+    with k + 3 pairs.  The B_j come from provers, so the check also tests that each lies in G2."""
+    proofs = list(proofs)
+    rx_pubs = list(rx_pubs)
+    k = len(proofs)
+    if len(rx_pubs) != k:
+        raise ValueError("verify_batch: one public input list per proof")
+    if k == 0:
+        return True
+    rho = batch_weights(k, rng)
+    pub = {}
+    for w, rx_pub in zip(rho, rx_pubs):
+        for i, ri in rx_pub:
+            pub[i] = (pub.get(i, 0) + w * int(ri)) % curve_order
+    idx = sorted(pub)
+    P = _public_term(sigma1_3, [(i, pub[i]) for i in idx])
+    C = g1_from_ints(native.g1_msm(native.g1_vec_bytes([c for _, _, c in proofs]), native.fr_vec_bytes(rho), k))
+    pairs = [(b, a) for a, b, _ in proofs] + [(sigma2_1[0], sigma1_1[0]), (sigma2_1[1], P), (sigma2_1[2], C)]
+    minus_one = curve_order - 1
+    scalars = rho + [(-sum(rho)) % curve_order, minus_one, minus_one]
+    return pairing_check(pairs, scalars, g2_subgroup_check=True)

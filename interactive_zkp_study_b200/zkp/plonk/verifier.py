@@ -9,9 +9,14 @@ are two GPU MSMs (2 and 18 terms):
     F = [t_lo] + zeta^n [t_mid] + zeta^2n [t_hi] + v D + v r0 G1 + v^2 [a] + v^3 [b] + v^4 [c] + v^5 [s1] + v^6 [s2]
     D = (a b)[q_m] + a [q_l] + b [q_r] + c [q_o] + [q_c] + (perm_z + alpha^2 L1) [z] - perm_s3 [s3]
 
-and the check is e(A, [tau]_2) == e(B, [1]_2): the two pairings need py_ecc (or a `pairing=` callable).
+and the check is e(A, [tau]_2) == e(B, [1]_2): the two pairings need py_ecc (or a `pairing=` callable;
+zkp.pairing.pairing runs them on the GPU).
+
+`verify_batch` checks k proofs against one SRS with e(sum rho_j A_j, [tau]_2) e(-sum rho_j B_j, [1]_2) == 1:
+the same two MSMs (over all proofs' terms at once) and two pairings for any k.
 """
 from ... import native
+from ..pairing import batch_weights, pairing_check
 from ...compat import HAVE_PY_ECC, g1_from_ints
 from .field import FR, G1, CURVE_ORDER
 from .transcript import Transcript
@@ -25,7 +30,8 @@ def _msm(terms):
     return g1_from_ints(native.g1_msm(native.g1_vec_bytes(pts), native.fr_vec_bytes(sc), len(pts)))
 
 
-def verify(proof, public_inputs, preprocessed, srs, pairing=None):
+def _pairing_terms(proof, public_inputs, preprocessed):
+    """(point, scalar) terms of the two G1 points A and B of the final check e(A, [tau]_2) == e(B, [1]_2)."""
     pp = preprocessed
     n, omega = pp.n, pp.omega
     t = Transcript()
@@ -59,10 +65,10 @@ def verify(proof, public_inputs, preprocessed, srs, pairing=None):
         e_scalar = e_scalar + vp * val
     e_scalar = e_scalar + u * zw
 
-    A = _msm([(proof.W_zeta_comm, FR(1)), (proof.W_zeta_omega_comm, u)])
+    A = [(proof.W_zeta_comm, FR(1)), (proof.W_zeta_omega_comm, u)]
     v2 = v * v
     v4 = v2 * v2
-    B = _msm([
+    B = [
         (proof.W_zeta_comm, zeta), (proof.W_zeta_omega_comm, u * zeta * omega),
         (proof.t_lo_comm, FR(1)), (proof.t_mid_comm, zeta_n), (proof.t_hi_comm, zeta_n * zeta_n),
         (pp.q_m_comm, v * a * b), (pp.q_l_comm, v * a), (pp.q_r_comm, v * b), (pp.q_o_comm, v * c), (pp.q_c_comm, v),
@@ -70,10 +76,33 @@ def verify(proof, public_inputs, preprocessed, srs, pairing=None):
         (G1, v * r0 - e_scalar),
         (proof.a_comm, v2), (proof.b_comm, v2 * v), (proof.c_comm, v4),
         (pp.s_sigma1_comm, v4 * v), (pp.s_sigma2_comm, v4 * v2),
-    ])
+    ]
+    return A, B
+
+
+def verify(proof, public_inputs, preprocessed, srs, pairing=None):
+    a_terms, b_terms = _pairing_terms(proof, public_inputs, preprocessed)
+    A = _msm(a_terms)
+    B = _msm(b_terms)
     if pairing is None:
         if not HAVE_PY_ECC:
             raise NotImplementedError("pairings are outside the GPU hot path; install py_ecc or pass pairing=")
         from py_ecc import bn128  # pragma: no cover
         pairing = bn128.pairing   # pragma: no cover
     return pairing(srs.g2_powers[1], A) == pairing(srs.g2_powers[0], B)
+
+
+def verify_batch(items, srs, rng=None):
+    """True iff every (proof, public_inputs, preprocessed) in `items` passes `verify` against the one `srs`, up
+    to a 2^-128 chance of accepting a bad batch: with random non-zero 128-bit weights rho_j (from `secrets`, or
+    from rng.getrandbits for reproducible runs) it checks e(sum rho_j A_j, [tau]_2) e(-sum rho_j B_j, [1]_2) == 1,
+    i.e. two GPU MSMs over the terms of all proofs and one pairing check with two pairs."""
+    items = list(items)
+    if not items:
+        return True
+    a_all, b_all = [], []
+    for rho, (proof, public_inputs, pp) in zip(batch_weights(len(items), rng), items):
+        a_terms, b_terms = _pairing_terms(proof, public_inputs, pp)
+        a_all += [(p, int(s) * rho) for p, s in a_terms]
+        b_all += [(p, int(s) * rho) for p, s in b_terms]
+    return pairing_check([(srs.g2_powers[1], _msm(a_all)), (srs.g2_powers[0], _msm(b_all))], [1, CURVE_ORDER - 1])
