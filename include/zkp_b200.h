@@ -162,6 +162,20 @@ int zkp_g1_fixed_base_mul(const uint8_t base_xy[64], const uint8_t* scalars, uin
 int zkp_g2_fixed_base_mul(const uint8_t base_xy[128], const uint8_t* scalars, uint64_t n, uint64_t* out_table);
 int zkp_g1_fixed_base_mul_dev(const uint8_t base_xy[64], uint64_t scalars, uint64_t n, uint64_t* out_table);
 int zkp_g2_fixed_base_mul_dev(const uint8_t base_xy[128], uint64_t scalars, uint64_t n, uint64_t* out_table);
+/* Variable-base form for a powers-of-tau contribution (zkp/plonk/srs.py:50-87 makes [tau^i]_1; a participant with
+ * secret s turns it into [(s tau)^i]_1 = s^i [tau^i]_1):
+ * out[i] = scalars[sc_offset + i] * T[offset + i], i < n, as a new plain table handle (affine, same encoding).
+ * Scalars are any 256-bit values, reduced mod r; a zero scalar or an infinity point gives infinity.  T may be plain
+ * or window-precomputed (the points are its first row).  One thread per point: a 4-bit fixed-window ladder over
+ * a per-thread table of 1..15 P.  n == 0 gives an empty table. */
+int zkp_g1_table_scale(uint64_t table, uint64_t offset, uint64_t scalars, uint64_t sc_offset, uint64_t n, uint64_t* out_table);
+int zkp_g2_table_scale(uint64_t table, uint64_t offset, uint64_t scalars, uint64_t sc_offset, uint64_t n, uint64_t* out_table);
+/* *first_bad = lowest index in [offset, offset+n) whose point is not on its curve (G2: or, with subgroup_check,
+ * not in the order-r subgroup), UINT64_MAX if none.  Infinity (0,0) counts as valid.  Validation judges the point
+ * as stored: zkp_g1/g2_table_load reduces every coordinate mod p on upload, so a coordinate c >= p is checked as
+ * c mod p. */
+int zkp_g1_table_validate(uint64_t table, uint64_t offset, uint64_t n, uint64_t* first_bad);
+int zkp_g2_table_validate(uint64_t table, uint64_t offset, uint64_t n, int subgroup_check, uint64_t* first_bad);
 int zkp_table_download(uint64_t table, uint64_t offset, uint64_t n, uint8_t* out_pts);
 int zkp_scalars_download(uint64_t scalars, uint64_t offset, uint64_t n, uint8_t* out);
 

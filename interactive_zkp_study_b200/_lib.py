@@ -80,6 +80,10 @@ PROTOTYPES = {
     "zkp_g1_fixed_base_mul": (c_int, [vp, vp, u64, u64p]),
     "zkp_g2_fixed_base_mul": (c_int, [vp, vp, u64, u64p]),
     "zkp_g1_fixed_base_mul_dev": (c_int, [vp, u64, u64, u64p]),
+    "zkp_g1_table_scale": (c_int, [u64, u64, u64, u64, u64, u64p]),
+    "zkp_g2_table_scale": (c_int, [u64, u64, u64, u64, u64, u64p]),
+    "zkp_g1_table_validate": (c_int, [u64, u64, u64, u64p]),
+    "zkp_g2_table_validate": (c_int, [u64, u64, u64, c_int, u64p]),
     "zkp_table_download": (c_int, [u64, u64, u64, vp]),
     "zkp_scalars_download": (c_int, [u64, u64, u64, vp]),
     "zkp_scalars_generate": (c_int, [u64, u64, u64p]),

@@ -1,23 +1,16 @@
 // Group-generic implementation of the MSM / table entry points; instantiated for G1 (msm_g1.cu)
 // and G2 (msm_g2.cu).  See include/zkp_b200.h for the contract of each function.
 #pragma once
+#include <type_traits>
 #include "comm.cuh"
+#include "curve_check.cuh"
 #include "msm.cuh"
 #include "registry.cuh"
 
 namespace zkp {
 
-
-// out[i] = scalars[i] * base: MSB-first double-and-add in XYZZ with mixed additions, one thread per
-// scalar, then one inversion per point.  Replaces the n sequential Python scalar-muls of
-// SRS.generate (/root/reference/zkp/plonk/srs.py:78-82) and sigma12/15/22 (setup.py:18-23,56-69).
-template <class F>
-__global__ void __launch_bounds__(128) fixed_base_mul_kernel(Affine<F> base_canon, const uint32_t* __restrict__ scalars,
-                                                              uint64_t n, Affine<F>* __restrict__ out) {
-  uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  Affine<F> base = {base_canon.x.to_mont(), base_canon.y.to_mont()};
-  uint32_t s[8];
+// s = scalars[i] mod r: any 256-bit value, 32 B canonical little-endian (2^256 < 6 r: at most five subtractions)
+ZKP_DEVINL void load_scalar_mod_r(const uint32_t* __restrict__ scalars, uint64_t i, uint32_t s[8]) {
   const uint4* sp = reinterpret_cast<const uint4*>(scalars + 8 * i);
   uint4 lo = sp[0], hi = sp[1];
   s[0] = lo.x; s[1] = lo.y; s[2] = lo.z; s[3] = lo.w;
@@ -34,6 +27,19 @@ __global__ void __launch_bounds__(128) fixed_base_mul_kernel(Affine<F> base_cano
 #pragma unroll
     for (int k = 0; k < 8; k++) s[k] = t[k];
   }
+}
+
+// out[i] = scalars[i] * base: MSB-first double-and-add in XYZZ with mixed additions, one thread per
+// scalar, then one inversion per point.  Replaces the n sequential Python scalar-muls of
+// SRS.generate (/root/reference/zkp/plonk/srs.py:78-82) and sigma12/15/22 (setup.py:18-23,56-69).
+template <class F>
+__global__ void __launch_bounds__(128) fixed_base_mul_kernel(Affine<F> base_canon, const uint32_t* __restrict__ scalars,
+                                                              uint64_t n, Affine<F>* __restrict__ out) {
+  uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  Affine<F> base = {base_canon.x.to_mont(), base_canon.y.to_mont()};
+  uint32_t s[8];
+  load_scalar_mod_r(scalars, i, s);
   XYZZ<F> acc = XYZZ<F>::inf();
   for (int w = 7; w >= 0; w--) {
     uint32_t word = s[w];
@@ -66,22 +72,7 @@ __global__ void __launch_bounds__(128) fixed_base_windowed_kernel(const Affine<F
   uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   uint32_t s[8];
-  const uint4* sp = reinterpret_cast<const uint4*>(scalars + 8 * i);
-  uint4 lo = sp[0], hi = sp[1];
-  s[0] = lo.x; s[1] = lo.y; s[2] = lo.z; s[3] = lo.w;
-  s[4] = hi.x; s[5] = hi.y; s[6] = hi.z; s[7] = hi.w;
-  for (int it = 0; it < 6; it++) {
-    uint32_t t[8], borrow = 0;
-#pragma unroll
-    for (int k = 0; k < 8; k++) {
-      uint64_t d = (uint64_t)s[k] - FrParams::MOD_(k) - borrow;
-      t[k] = (uint32_t)d;
-      borrow = (uint32_t)(d >> 63);
-    }
-    if (borrow) break;
-#pragma unroll
-    for (int k = 0; k < 8; k++) s[k] = t[k];
-  }
+  load_scalar_mod_r(scalars, i, s);
   XYZZ<F> acc = XYZZ<F>::inf();
 #pragma unroll 1
   for (int j = 0; j < 32; j++) {
@@ -89,6 +80,75 @@ __global__ void __launch_bounds__(128) fixed_base_windowed_kernel(const Affine<F
     if (d) acc.madd(tab[j * 256 + d]);
   }
   out[i] = acc.to_affine();
+}
+
+// out[i] = scalars[i] * pts[i], a different base per thread (zkp_g1/g2_table_scale; the powers-of-tau update
+// [tau^i]_1 -> [(s tau)^i]_1 = s^i [tau^i]_1).  Table and result are Montgomery affine, (0,0) for infinity.
+//   - tab[d - 1] = d P for d = 1..15, built in XYZZ (one doubling, 13 mixed additions) and made affine with one
+//     inversion shared by the 15 entries (Montgomery's trick: 1/(ZZ ZZZ) gives 1/ZZ and 1/ZZZ).
+//   - k mod r in 4-bit windows from the top: 4 doublings and at most one mixed addition of tab[d - 1] per window
+//     (~252 doublings + <= 64 additions, against 254 doublings + ~127 additions bit by bit), one inversion at the end.
+// The table is indexed by a data-dependent digit and so lives in local memory (L1-resident: 15 x 64 B in G1).
+template <class F>
+__global__ void __launch_bounds__(128) table_scale_kernel(const Affine<F>* __restrict__ pts,
+                                                          const uint32_t* __restrict__ scalars, uint64_t n,
+                                                          Affine<F>* __restrict__ out) {
+  uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const Affine<F> p = pts[i];
+  if (p.is_inf()) {
+    out[i] = Affine<F>::inf();
+    return;
+  }
+  uint32_t s[8];
+  load_scalar_mod_r(scalars, i, s);
+  constexpr int TAB = 15;
+  Affine<F> tab[TAB];
+  F zz[TAB], zzz[TAB], pre[TAB];  // pre[j] = prod_{m <= j} zz[m] zzz[m]
+  XYZZ<F> acc = XYZZ<F>::from_affine(p);
+  F prod = F::one();
+#pragma unroll 1
+  for (int j = 0; j < TAB; j++) {
+    if (j) acc.madd(p);  // (j + 1) P; an entry at infinity (P of small order off G2) stays (0,0) below
+    const bool inf = acc.is_inf();
+    tab[j] = {acc.x, acc.y};
+    zz[j] = inf ? F::one() : acc.zz;
+    zzz[j] = inf ? F::one() : acc.zzz;
+    prod = prod * (zz[j] * zzz[j]);
+    pre[j] = prod;
+  }
+  F inv = prod.inv();  // 1 / prod_{m <= j} for the current j, walking down
+#pragma unroll 1
+  for (int j = TAB - 1; j >= 0; j--) {
+    const F im = j ? inv * pre[j - 1] : inv;  // 1 / (zz[j] zzz[j])
+    inv = inv * (zz[j] * zzz[j]);
+    tab[j] = {tab[j].x * (im * zzz[j]), tab[j].y * (im * zz[j])};
+  }
+  XYZZ<F> r = XYZZ<F>::inf();
+#pragma unroll 1
+  for (int w = 63; w >= 0; w--) {
+    if (!r.is_inf()) r = r.dbl().dbl().dbl().dbl();
+    const uint32_t d = (s[w >> 3] >> ((w & 7) * 4)) & 15u;
+    if (d) r.madd(tab[d - 1]);
+  }
+  out[i] = r.to_affine();
+}
+
+// *first_bad = min(first_bad, base + i) for every pts[i], i < n, that is not on its curve (Montgomery coordinates as
+// stored in a table) or, with `subgroup` (G2 only), not in the order-r subgroup.  Infinity (0,0) is valid.
+template <class F>
+__global__ void __launch_bounds__(64) table_validate_kernel(const Affine<F>* __restrict__ pts, uint64_t n, uint64_t base,
+                                                            bool subgroup, unsigned long long* __restrict__ first_bad) {
+  using FC = typename CompactOf<F>::type;  // same layout, out-of-line products: this is not a hot loop
+  uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const Affine<FC> a = reinterpret_cast<const Affine<FC>*>(pts)[i];
+  if (a.is_inf()) return;
+  bool ok = on_curve_mont(a);
+  if constexpr (std::is_same<FC, Fp2>::value) {
+    if (ok && subgroup) ok = g2_in_subgroup(a);
+  }
+  if (!ok) atomicMin(first_bad, (unsigned long long)(base + i));
 }
 
 template <class F>
@@ -429,6 +489,53 @@ struct GroupApi {
       if (!base_xy || !out_table) throw InvalidArgument("fixed_base_mul_dev: null argument");
       if (n > s->n) throw InvalidArgument("fixed_base_mul_dev: n exceeds the scalar vector");
       fixed_base_run(c, base_xy, s->buf.as<uint32_t>(), n, out_table);
+    });
+  }
+
+  // Points [offset, offset + n) of either layout: a precomputed table keeps the points themselves in row 0.
+  static const Affine<F>* table_points(Resource* t, uint64_t offset) { return t->buf.as<Affine<F>>() + offset; }
+
+  static int table_scale(uint64_t table, uint64_t offset, uint64_t scalars, uint64_t sc_offset, uint64_t n,
+                         uint64_t* out_table) {
+    return guarded([&](Context& c) {
+      Resource* t = need(table, KIND, "table_scale");
+      Resource* s = need(scalars, HandleKind::Scalars, "table_scale");
+      if (!out_table) throw InvalidArgument("table_scale: null output");
+      if (!range_ok(offset, n, t->n) || !range_ok(sc_offset, n, s->n)) throw InvalidArgument("table_scale: range out of bounds");
+      auto r = std::make_unique<Resource>();
+      r->kind = KIND;
+      r->n = n;
+      r->buf.reserve_pooled(n ? n * PT : PT);
+      if (n) {
+        table_scale_kernel<F><<<ceil_div(n, 128), 128, 0, c.stream>>>(table_points(t, offset),
+                                                                     s->buf.as<uint32_t>() + 8 * sc_offset, n,
+                                                                     r->buf.as<Affine<F>>());
+        CUDA_CHECK_LAUNCH();
+        c.launches++;
+      }
+      CUDA_CHECK(cudaStreamSynchronize(c.stream));
+      *out_table = registry().put(std::move(r));
+    });
+  }
+
+  static int table_validate(uint64_t table, uint64_t offset, uint64_t n, int subgroup, uint64_t* first_bad) {
+    return guarded([&](Context& c) {
+      Resource* t = need(table, KIND, "table_validate");
+      if (!first_bad) throw InvalidArgument("table_validate: null output");
+      if (!range_ok(offset, n, t->n)) throw InvalidArgument("table_validate: range out of bounds");
+      unsigned long long bad = ~0ull;
+      if (n) {
+        ScopedDevBuf flag;
+        flag.reserve(sizeof bad);
+        CUDA_CHECK(cudaMemsetAsync(flag.p, 0xff, sizeof bad, c.stream));
+        table_validate_kernel<F><<<ceil_div(n, 64), 64, 0, c.stream>>>(table_points(t, offset), n, offset, subgroup != 0,
+                                                                       flag.as<unsigned long long>());
+        CUDA_CHECK_LAUNCH();
+        c.launches++;
+        CUDA_CHECK(cudaMemcpyAsync(&bad, flag.p, sizeof bad, cudaMemcpyDeviceToHost, c.stream));
+        CUDA_CHECK(cudaStreamSynchronize(c.stream));
+      }
+      *first_bad = bad;
     });
   }
 

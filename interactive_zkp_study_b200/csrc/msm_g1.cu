@@ -100,6 +100,14 @@ int zkp_g1_fixed_base_mul_dev(const uint8_t base_xy[64], uint64_t scalars, uint6
   return Api::fixed_base_dev(base_xy, scalars, n, out_table);
 }
 
+int zkp_g1_table_scale(uint64_t table, uint64_t offset, uint64_t scalars, uint64_t sc_offset, uint64_t n,
+                       uint64_t* out_table) {
+  return Api::table_scale(table, offset, scalars, sc_offset, n, out_table);
+}
+int zkp_g1_table_validate(uint64_t table, uint64_t offset, uint64_t n, uint64_t* first_bad) {
+  return Api::table_validate(table, offset, n, 0, first_bad);
+}
+
 int zkp_g1_msm_dev_batch(uint64_t table, uint32_t count, const uint64_t* scalars, const uint64_t* sc_offsets,
                          const uint64_t* offsets, const uint64_t* lens, uint8_t* out_xy, int* out_is_inf) {
   return Api::msm_batch(table, count, scalars, sc_offsets, offsets, lens, out_xy, out_is_inf);

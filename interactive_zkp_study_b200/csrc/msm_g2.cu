@@ -53,6 +53,13 @@ int zkp_g2_msm_multi_end(uint8_t out_xy[128], int* out_is_inf) { return Api::msm
 int zkp_g2_fixed_base_mul_dev(const uint8_t base_xy[128], uint64_t scalars, uint64_t n, uint64_t* out_table) {
   return Api::fixed_base_dev(base_xy, scalars, n, out_table);
 }
+int zkp_g2_table_scale(uint64_t table, uint64_t offset, uint64_t scalars, uint64_t sc_offset, uint64_t n,
+                       uint64_t* out_table) {
+  return Api::table_scale(table, offset, scalars, sc_offset, n, out_table);
+}
+int zkp_g2_table_validate(uint64_t table, uint64_t offset, uint64_t n, int subgroup_check, uint64_t* first_bad) {
+  return Api::table_validate(table, offset, n, subgroup_check, first_bad);
+}
 int zkp_g2_table_precompute(uint64_t table, int window_bits) { return Api::table_precompute(table, window_bits); }
 int zkp_g2_fixed_base_mul(const uint8_t base_xy[128], const uint8_t* scalars, uint64_t n, uint64_t* out_table) {
   return Api::fixed_base_host(base_xy, scalars, n, out_table);

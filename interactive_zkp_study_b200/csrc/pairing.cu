@@ -14,57 +14,14 @@
 // tests/tower_model.py states every formula on integers; the CPU suite checks it against py_ecc.
 #include <cstring>
 #include "../../include/zkp_b200_diag.h"
-#include "ec.cuh"
+#include "curve_check.cuh"
 #include "fp12.cuh"
 #include "registry.cuh"
 
 namespace zkp {
 
-using G1A = Affine<FpC>;  // same layout as G1Affine: x || y, 8 limbs each
-using G2A = Affine<Fp2>;
-
 constexpr uint64_t ATE_LOW = 11347224129447541672ull;  // 6x + 2 - 2^64: the 64 bits below the implicit top bit
 constexpr uint64_t NONE = ~0ull;
-
-ZKP_DEVINL bool fp_canonical(const FpC& a) {
-  uint32_t borrow = 0;
-#pragma unroll
-  for (int k = 0; k < 8; k++) {
-    uint64_t d = (uint64_t)a.v[k] - FpParams::MOD_(k) - borrow;
-    borrow = (uint32_t)(d >> 63);
-  }
-  return borrow != 0;
-}
-
-ZKP_DEVINL Fp2 twist_b() {
-  Fp2 b;
-#pragma unroll
-  for (int k = 0; k < 8; k++) {
-    b.c0.v[k] = FpParams::B2_C0_(k);
-    b.c1.v[k] = FpParams::B2_C1_(k);
-  }
-  return b;
-}
-
-// canonical input -> Montgomery form; false when a coordinate is not below p or the point is not on its curve
-// (infinity, all zeros, is valid)
-ZKP_DEVINL bool load_g1(const G1A& in, G1A& out) {
-  out = in;
-  if (in.is_inf()) return true;
-  if (!fp_canonical(in.x) || !fp_canonical(in.y)) return false;
-  out = {in.x.to_mont(), in.y.to_mont()};
-  FpC b;
-#pragma unroll
-  for (int k = 0; k < 8; k++) b.v[k] = FpParams::B3_(k);
-  return out.y.sqr() == out.x.sqr() * out.x + b;
-}
-ZKP_DEVINL bool load_g2(const G2A& in, G2A& out) {
-  out = in;
-  if (in.is_inf()) return true;
-  if (!fp_canonical(in.x.c0) || !fp_canonical(in.x.c1) || !fp_canonical(in.y.c0) || !fp_canonical(in.y.c1)) return false;
-  out = {in.x.to_mont(), in.y.to_mont()};
-  return out.y.sqr() == out.x.sqr() * out.x + twist_b();
-}
 
 // first_bad[0] / [1]: lowest index of a G1 / G2 input that fails load_g1 / load_g2
 __global__ void pairing_validate_kernel(const G2A* q, const G1A* p, uint64_t n, unsigned long long* first_bad) {
@@ -83,13 +40,7 @@ __global__ void g2_subgroup_kernel(const G2A* q, uint64_t n, unsigned long long*
   if (i >= n) return;
   G2A a;
   if (!load_g2(q[i], a) || a.is_inf()) return;
-  XYZZ<Fp2> acc = XYZZ<Fp2>::from_affine(a);
-#pragma unroll 1
-  for (int bit = 252; bit >= 0; bit--) {  // r < 2^254, bit 253 is set: acc starts there
-    acc = acc.dbl();
-    if ((FrParams::MOD_(bit >> 5) >> (bit & 31)) & 1) acc.madd(a);
-  }
-  if (!acc.is_inf()) atomicMin(first_bad + 2, (unsigned long long)i);
+  if (!g2_in_subgroup(a)) atomicMin(first_bad + 2, (unsigned long long)i);
 }
 
 struct G2Proj {

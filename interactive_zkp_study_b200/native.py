@@ -302,6 +302,40 @@ def g1_fixed_base_mul_dev(base_bytes, scalars, n):
     return DeviceHandle(h.value, n, "g1")
 
 
+def _table_scale(fn_name, table, offset, scalars, sc_offset, n):
+    h = ctypes.c_uint64()
+    check(getattr(_lib.lib(), fn_name)(table.handle, offset, scalars.handle, sc_offset, n, ctypes.byref(h)))
+    return DeviceHandle(h.value, n, table.kind)
+
+
+def g1_table_scale(table, offset, scalars, sc_offset, n):
+    """New plain G1 table: out[i] = scalars[sc_offset + i] * table[offset + i] (scalars reduced mod r)."""
+    return _table_scale("zkp_g1_table_scale", table, offset, scalars, sc_offset, n)
+
+
+def g2_table_scale(table, offset, scalars, sc_offset, n):
+    return _table_scale("zkp_g2_table_scale", table, offset, scalars, sc_offset, n)
+
+
+def _first_bad(v):
+    return None if v == (1 << 64) - 1 else v
+
+
+def g1_table_validate(table, offset, n):
+    """Lowest index in [offset, offset + n) whose point is not on the curve, or None (infinity is valid)."""
+    bad = ctypes.c_uint64()
+    check(_lib.lib().zkp_g1_table_validate(table.handle, offset, n, ctypes.byref(bad)))
+    return _first_bad(bad.value)
+
+
+def g2_table_validate(table, offset, n, subgroup_check=False):
+    """Lowest index in [offset, offset + n) whose point is not on the twist or, with subgroup_check, not in G2;
+    None if every point passes."""
+    bad = ctypes.c_uint64()
+    check(_lib.lib().zkp_g2_table_validate(table.handle, offset, n, 1 if subgroup_check else 0, ctypes.byref(bad)))
+    return _first_bad(bad.value)
+
+
 # ------------------------------------------------------------------ MSM
 def _msm_out(group):
     return bytearray(64 if group == 1 else 128), ctypes.c_int()

@@ -12,7 +12,7 @@ written and read without ever becoming Python integers:
     G2      x.c0 | x.c1 | y.c0 | y.c1, 128 bytes; None is 128 zero bytes
     vectors the elements back to back
 
-Composite objects (SRS, PreprocessedData, Proof) are a flat container: magic, then (name, tag, length,
+Composite objects (SRS, PreprocessedData, Proof, ceremony Contribution) are a flat container: magic, then (name, tag, length,
 payload) records.  `to_text` / `from_text` wrap any payload as base64 for stores that only take strings
 (TinyDB, JSON responses).
 """
@@ -21,6 +21,7 @@ import struct
 
 from ... import native
 from ...compat import FQ, FQ2, curve_order
+from .ceremony import Contribution
 from .field import FR
 from .polynomial import Polynomial
 from .preprocessor import PreprocessedData
@@ -168,6 +169,17 @@ def deserialize_srs(blob):
     g1 = [deserialize_g1(g1b[i:i + 64]) for i in range(0, len(g1b), 64)]
     g2 = [deserialize_g2(g2b[i:i + 128]) for i in range(0, len(g2b), 128)]
     return SRS(g1, g2, struct.unpack("<q", rec["max_degree"][1])[0])
+
+
+# ------------------------------------------------------------------ powers-of-tau Contribution (ceremony.py)
+def serialize_contribution(contribution):
+    return dumps([_g1f("s_g1", contribution.s_g1), _g1f("R", contribution.R), _frf("z", contribution.z)])
+
+
+def deserialize_contribution(blob):
+    rec = loads(blob)
+    z = _get_fr(rec, "z")
+    return Contribution(_get_g1(rec, "s_g1"), _get_g1(rec, "R"), 0 if z is None else int(z))
 
 
 # ------------------------------------------------------------------ PreprocessedData
