@@ -102,6 +102,17 @@ int zkp_g2_msm_dev_end(uint8_t out_xy[128], int* out_is_inf);
  * commitments in groups: kzg.commit x3 in round1.py:80-82, round3.py:178-180, x2 in round5.py:174-175). */
 int zkp_g1_msm_dev_batch(uint64_t table, uint32_t count, const uint64_t* scalars, const uint64_t* sc_offsets,
                          const uint64_t* offsets, const uint64_t* lens, uint8_t* out_xy, int* out_is_inf);
+/* Many MSMs over ONE point range, for batch proving (count proofs of one circuit: the per-proof MSMs of
+ * zkp/groth16/proving.py:23-75 share their points).  MSM j = sum_i s[sc_offset + j*n + i] * T[offset + i], j < count:
+ * the scalar vectors lie back to back in one handle.  Plain and window-precomputed tables.  One Pippenger pass over
+ * all count*n scalars (MSM j owns its own buckets), so the launch count does not depend on count.  out_xy holds
+ * count x 64 (G1) / 128 (G2) bytes; out_is_inf (may be NULL) count flags.  count = 0 returns at once; n = 0 gives
+ * count points at infinity.  ZKP_ERR_INVALID_ARGUMENT before any launch when count*W*n >= 2^32 (W = windows of the
+ * table's width), count * (buckets per MSM) >= 2^31, or a range runs past its table / handle. */
+int zkp_g1_msm_dev_many(uint64_t table, uint64_t offset, uint64_t n, uint32_t count, uint64_t scalars,
+                        uint64_t sc_offset, uint8_t* out_xy, int* out_is_inf);
+int zkp_g2_msm_dev_many(uint64_t table, uint64_t offset, uint64_t n, uint32_t count, uint64_t scalars,
+                        uint64_t sc_offset, uint8_t* out_xy, int* out_is_inf);
 /* Shard form for the multi-GPU path (SURVEY 8e): the un-normalised XYZZ partial sum of this rank's
  * point range, 4 coordinates x 32 B Montgomery for G1 (128 B); combine folds `count` partials
  * (gathered from all ranks) into the affine result.  `out_xyzz` and `partials` may be host memory or
@@ -225,6 +236,18 @@ int zkp_groth16_quotient(const uint8_t* a, const uint8_t* b, const uint8_t* c, u
  * remainder (zero for a satisfied instance; three more transforms) is then not computed. */
 int zkp_groth16_quotient_dev(uint64_t a, uint64_t b, uint64_t c, uint64_t len, uint64_t z, uint64_t z_len,
                              uint64_t* h_out, uint64_t* rem_out);
+/* count quotients at once: proof j's coefficients at offset j*len of a, b and c.  Creates one handle of
+ * count x (2*len - z_len) coefficients, proof j's quotient at offset j*(2*len - z_len); equal to
+ * zkp_groth16_quotient_dev per proof (quotient only; shares its divisor cache).  Launches do not grow with count. */
+int zkp_groth16_quotient_batch_dev(uint64_t a, uint64_t b, uint64_t c, uint64_t len, uint32_t count, uint64_t z,
+                                   uint64_t z_len, uint64_t* h_out);
+/* The three scalar vectors of count proofs (zkp/groth16/device_prover.py _scalars_ab / _scalars_c), one launch:
+ * A_j = uA_j | 1 | r_j, B_j = uB_j | 1 | s_j (k + 2 each), C_j = r_j uB_j + s_j uA_j | r_j | rx_j | H_j | s_j | s_j r_j
+ * (2k + 2 + m_priv).  uA, uB: count*k; h: count*(k-1) (ignored for k = 1); rx: count*m_priv (ignored for m_priv = 0);
+ * rs, ss: count x 32 B canonical.  Creates three handles, proof j's vector at offset j * (its length). */
+int zkp_groth16_batch_scalars_dev(uint64_t ua, uint64_t ub, uint64_t h, uint64_t rx, uint64_t k, uint64_t m_priv,
+                                  uint32_t count, const uint8_t* rs, const uint8_t* ss, uint64_t* out_a,
+                                  uint64_t* out_b, uint64_t* out_c);
 /* The three MSMs of one proof (proving.py:23-75 as one MSM per element): A = <sa, ta> and C' = <sc, tc>
  * in G1 on one stream, B = <sb, tb2> in G2 on a second one, so the G2 work overlaps the G1 work.
  * Whole tables from index 0, na / nb / nc entries; out_is_inf = {A, B, C'} flags (may be NULL). */
@@ -297,6 +320,12 @@ int zkp_sparse_load(const uint32_t* row_ptr, const uint32_t* col_idx, const uint
 int zkp_sparse_matvec_dev(uint64_t matrix, uint64_t vec, uint64_t vec_off, uint64_t out, uint64_t out_off);
 int zkp_fr_ap_interpolate_dev(uint64_t values, uint64_t off, uint64_t k, const uint8_t* scale, uint64_t out,
                               uint64_t out_off);
+/* The same over count vectors in the same launches: witness j at vec_off + j*cols, output j at out_off + j*rows;
+ * values j at off + j*k, coefficients j at out_off + j*k. */
+int zkp_sparse_matvec_many_dev(uint64_t matrix, uint64_t vec, uint64_t vec_off, uint64_t out, uint64_t out_off,
+                               uint32_t count);
+int zkp_fr_ap_interpolate_many_dev(uint64_t values, uint64_t off, uint64_t k, uint32_t count, const uint8_t* scale,
+                                   uint64_t out, uint64_t out_off);
 int zkp_fr_ap_vanishing_dev(uint64_t k, uint64_t out, uint64_t out_off);
 int zkp_fr_ap_lagrange_dev(uint64_t k, const uint8_t x[32], uint64_t out, uint64_t out_off);
 

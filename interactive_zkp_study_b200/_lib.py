@@ -56,6 +56,8 @@ PROTOTYPES = {
     "zkp_g1_msm_dev": (c_int, [u64, u64, u64, u64, u64, vp, intp]),
     "zkp_g2_msm_dev": (c_int, [u64, u64, u64, u64, u64, vp, intp]),
     "zkp_g1_msm_dev_batch": (c_int, [u64, u32, u64p, u64p, u64p, u64p, vp, intp]),
+    "zkp_g1_msm_dev_many": (c_int, [u64, u64, u64, u32, u64, u64, vp, intp]),
+    "zkp_g2_msm_dev_many": (c_int, [u64, u64, u64, u32, u64, u64, vp, intp]),
     "zkp_g1_msm_dev_partial": (c_int, [u64, u64, u64, u64, u64, vp]),
     "zkp_g1_combine_partials": (c_int, [vp, u32, vp, intp]),
     "zkp_msm_set_window_bits": (c_int, [c_int]),
@@ -96,6 +98,8 @@ PROTOTYPES = {
     "zkp_fr_vec_matrix": (c_int, [vp, vp, u64, u64, vp]),
     "zkp_groth16_quotient": (c_int, [vp, vp, vp, u64, vp, u64, vp, vp]),
     "zkp_groth16_quotient_dev": (c_int, [u64, u64, u64, u64, u64, u64, u64p, u64p]),
+    "zkp_groth16_quotient_batch_dev": (c_int, [u64, u64, u64, u64, u32, u64, u64, u64p]),
+    "zkp_groth16_batch_scalars_dev": (c_int, [u64, u64, u64, u64, u64, u64, u32, vp, vp, u64p, u64p, u64p]),
     "zkp_scalars_alloc": (c_int, [u64, u64p]),
     "zkp_scalars_copy": (c_int, [u64, u64, u64, u64, u64]),
     "zkp_scalars_upload": (c_int, [u64, u64, vp, u64]),
@@ -120,6 +124,8 @@ PROTOTYPES = {
     "zkp_sparse_load": (c_int, [vp, vp, vp, u64, u64, u64, u64p]),
     "zkp_sparse_matvec_dev": (c_int, [u64, u64, u64, u64, u64]),
     "zkp_fr_ap_interpolate_dev": (c_int, [u64, u64, u64, vp, u64, u64]),
+    "zkp_sparse_matvec_many_dev": (c_int, [u64, u64, u64, u64, u64, u32]),
+    "zkp_fr_ap_interpolate_many_dev": (c_int, [u64, u64, u64, u32, vp, u64, u64]),
     "zkp_fr_ap_vanishing_dev": (c_int, [u64, u64, u64]),
     "zkp_fr_ap_lagrange_dev": (c_int, [u64, vp, u64, u64]),
     "zkp_fr_poly_mul": (c_int, [vp, u64, vp, u64, vp]),

@@ -180,6 +180,21 @@ static __global__ void msm_scatter_kernel(const uint32_t* __restrict__ codes, ui
   sorted[pos] = i | ((code & 1u) << 31);
 }
 
+// The same for the codes of msm_digits_many_kernel: entry idx = w * N + j * n + i is point i of window w, shared by
+// all MSMs.
+static __global__ void msm_scatter_many_kernel(const uint32_t* __restrict__ codes, uint64_t total, uint64_t N, uint64_t n,
+                                               uint32_t* __restrict__ cursor, uint32_t* __restrict__ sorted,
+                                               uint32_t pre_stride, uint32_t pre_offset) {
+  uint64_t idx = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= total) return;
+  uint32_t code = codes[idx];
+  if (code == MSM_INVALID) return;
+  uint32_t i = (uint32_t)((idx % N) % n);
+  if (pre_stride) i += (uint32_t)(idx / N) * pre_stride + pre_offset;
+  uint32_t pos = atomicAdd(&cursor[code >> 1], 1u);
+  sorted[pos] = i | ((code & 1u) << 31);
+}
+
 // ---------------------------------------------------------------- digit recoding helpers
 // Canonical scalar i reduced mod r into s[0..8] (s[8] = 0): the group has order r, so
 // k*P == (k mod r)*P (field.py:88).  2^256 / r < 6.
@@ -238,6 +253,27 @@ static __global__ void msm_digits_kernel(const uint32_t* __restrict__ scalars, u
     uint32_t code = msm_digit_code(s, w, c, B, wstride, carry);
     codes[(uint64_t)w * n + i] = code;
     if (code != MSM_INVALID) atomicAdd(&hist[code >> 1], 1u);
+  }
+}
+
+// Many MSMs over one point range (MsmEngine::run_many): scalar q = j * n + i of the N = count * n back-to-back
+// vectors belongs to MSM j and point i; MSM j owns buckets [j * per_msm, (j + 1) * per_msm).  codes[w * N + q].
+static __global__ void msm_digits_many_kernel(const uint32_t* __restrict__ scalars, uint64_t n, uint64_t N, int c, int W,
+                                              uint32_t B, uint32_t wstride, uint32_t per_msm,
+                                              uint32_t* __restrict__ codes, uint32_t* __restrict__ hist) {
+  uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= N) return;
+  const uint32_t base = (uint32_t)(q / n) * per_msm;
+  uint32_t s[9];
+  msm_load_scalar(scalars, q, s);
+  uint32_t carry = 0;
+  for (int w = 0; w < W; w++) {
+    uint32_t code = msm_digit_code(s, w, c, B, wstride, carry);
+    if (code != MSM_INVALID) {
+      code += base << 1;
+      atomicAdd(&hist[code >> 1], 1u);
+    }
+    codes[(uint64_t)w * N + q] = code;
   }
 }
 
@@ -731,6 +767,28 @@ __global__ void __launch_bounds__(32) msm_final_kernel(const XYZZ<F>* __restrict
   }
 }
 
+// One warp per MSM of a run_many pass: block j runs the Horner chain over its W window sums (W = 1 for a
+// precomputed table: only the affine conversion is left) and writes out[j] / inf_flag[j] as msm_final_kernel does.
+template <class F>
+__global__ void __launch_bounds__(32) msm_final_many_kernel(const XYZZ<F>* __restrict__ window_sums, int W, int c,
+                                                            Affine<F>* __restrict__ out, int* __restrict__ inf_flag) {
+  const int ql = threadIdx.x & 3;
+  const XYZZ<F>* ws = window_sums + (uint64_t)blockIdx.x * W;
+  XYZZ<F> r = ws[W - 1];
+  for (int w = W - 2; w >= 0; w--) {
+    if (!r.is_inf())
+      for (int k = 0; k < c; k++) r = Quad<F>::dbl(r, ql);
+    r = Quad<F>::add(r, ws[w], ql);
+  }
+  Affine<F> a = r.to_affine();
+  a.x = a.x.from_mont();
+  a.y = a.y.from_mont();
+  if (threadIdx.x == 0) {
+    inf_flag[blockIdx.x] = r.is_inf() ? 1 : 0;
+    out[blockIdx.x] = a;
+  }
+}
+
 // canonical <-> Montgomery conversion of coordinate arrays (n_fe field elements of the base field)
 template <class FE>
 __global__ void fe_to_mont_kernel(FE* __restrict__ v, uint64_t n) {
@@ -1172,6 +1230,73 @@ struct MsmEngine {
     tr.mark("horner+affine");
     return launches;
   }
+
+  // `count` MSMs over the same n points, scalar vector j at scalars[8 * j * n ...]: ONE Pippenger pass whose bucket
+  // sets are the MSMs' own (MSM j owns buckets [j * per_msm, (j + 1) * per_msm)).  Tasks, accumulation and fold run
+  // unchanged over count times as many buckets; the reduction treats every (MSM, window) as a segment; one warp per
+  // MSM finishes.  Leaves count canonical affine points in `many_out` and the infinity flags in `many_flag`.
+  // The launch count does not depend on count.  The caller has checked count * W * n < 2^32 and
+  // count * per_msm < 2^31 (GroupApi::msm_dev_many).
+  int run_many(const Affine<F>* pts, const uint32_t* scalars, uint64_t n, uint32_t count, cudaStream_t st, int force_c,
+               uint32_t pre_stride, uint32_t pre_offset) {
+    many_out.reserve((size_t)(count ? count : 1) * sizeof(Affine<F>));
+    many_flag.reserve((size_t)(count ? count : 1) * sizeof(int));
+    if (!count) return 0;
+    if (n == 0) {  // every MSM is empty: count points at infinity
+      CUDA_CHECK(cudaMemsetAsync(many_out.p, 0, (size_t)count * sizeof(Affine<F>), st));
+      std::vector<int> ones(count, 1);
+      CUDA_CHECK(cudaMemcpyAsync(many_flag.p, ones.data(), (size_t)count * sizeof(int), cudaMemcpyHostToDevice, st));
+      CUDA_CHECK(cudaStreamSynchronize(st));
+      return 0;
+    }
+    const MsmPlan pl = msm_plan(n, force_c);
+    const uint32_t per_msm = pre_stride ? pl.B : pl.nbuckets;
+    const uint32_t wstride = pre_stride ? 0u : pl.B;
+    const uint64_t N = (uint64_t)count * n;
+    const uint64_t total = (uint64_t)pl.W * N;
+    const uint32_t nbuckets = count * per_msm;
+    const int n_windows = pre_stride ? (int)count : (int)count * pl.W;
+    int launches = 0;
+    StageTrace tr(st);
+    buckets.reserve((size_t)nbuckets * sizeof(XYZZ<F>));
+    codes.reserve(total * 4);
+    sorted.reserve(total * 4);
+    hist.reserve((size_t)nbuckets * 4);
+    offsets.reserve(((size_t)nbuckets + 1) * 4);
+    cursor.reserve(((size_t)nbuckets + 1) * 4);
+    CUDA_CHECK(cudaMemsetAsync(hist.p, 0, (size_t)nbuckets * 4, st));
+    msm_digits_many_kernel<<<ceil_div(N, 256), 256, 0, st>>>(scalars, n, N, pl.c, pl.W, pl.B, wstride, per_msm,
+                                                            codes.as<uint32_t>(), hist.as<uint32_t>());
+    CUDA_CHECK_LAUNCH();
+    launches += 1 + scan_u32(hist.as<uint32_t>(), nbuckets, offsets.as<uint32_t>(), st);
+    tr.mark("digits+scan");
+    CUDA_CHECK(cudaMemcpyAsync(cursor.p, offsets.p, ((size_t)nbuckets + 1) * 4, cudaMemcpyDeviceToDevice, st));
+    msm_scatter_many_kernel<<<ceil_div(total, 256), 256, 0, st>>>(codes.as<uint32_t>(), total, N, n, cursor.as<uint32_t>(),
+                                                                 sorted.as<uint32_t>(), pre_stride, pre_offset);
+    CUDA_CHECK_LAUNCH();
+    launches++;
+    tr.mark("scatter");
+    const uint32_t max_tasks = (uint32_t)(total / MSM_TASK_LEN) + nbuckets + 1;
+    launches += build_tasks(nbuckets, max_tasks, st);
+    tr.mark("tasks");
+    msm_accumulate_kernel<F, MSM_ACC_OUTLINE><<<ceil_div(max_tasks, 128), 128, 0, st>>>(
+        pts, sorted.as<uint32_t>(), tasks.as<uint4>(), task_base.as<uint32_t>() + nbuckets, partials.as<XYZZ<F>>(),
+        buckets.as<XYZZ<F>>(), false);
+    CUDA_CHECK_LAUNCH();
+    launches++;
+    tr.mark("accumulate");
+    launches += fold_buckets(nbuckets, total / nbuckets, st, false, false);
+    tr.mark("fold");
+    const XYZZ<FC>* wsum = nullptr;
+    launches += reduce_buckets(nbuckets, n_windows, st, tr, &wsum);
+    const int W = pre_stride ? 1 : pl.W;
+    msm_final_many_kernel<FC><<<count, 32, 0, st>>>(wsum, W, pl.c, many_out.as<Affine<FC>>(), many_flag.as<int>());
+    CUDA_CHECK_LAUNCH();
+    launches++;
+    tr.mark("horner+affine");
+    return launches;
+  }
+  DevBuf many_out, many_flag;
 };
 
 }  // namespace zkp

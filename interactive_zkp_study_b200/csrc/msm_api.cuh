@@ -258,6 +258,42 @@ struct GroupApi {
     });
   }
 
+  // `count` MSMs over the same points [offset, offset + n), scalar vector j at sc_offset + j * n: one Pippenger pass
+  // (MsmEngine::run_many).  The limits are checked on the host before anything is launched.
+  static int msm_dev_many(uint64_t table, uint64_t offset, uint64_t n, uint32_t count, uint64_t scalars, uint64_t sc_offset,
+                          uint8_t* out_xy, int* out_is_inf) {
+    return guarded([&](Context& c) {
+      Resource* t = need(table, KIND, "msm_dev_many");
+      Resource* s = need(scalars, HandleKind::Scalars, "msm_dev_many");
+      if (count && !out_xy) throw InvalidArgument("msm_dev_many: null output");
+      if (!range_ok(offset, n, t->n)) throw InvalidArgument("msm_dev_many: point range exceeds the table");
+      if (!count) return;
+      const int force_c = t->pre_c ? t->pre_c : msm_options().window_bits;
+      const MsmPlan pl = msm_plan(n ? n : 1, force_c);
+      if ((uint64_t)count * pl.W * n >= (1ull << 32)) throw InvalidArgument("msm_dev_many: count * W * n must be < 2^32");
+      const uint64_t per_msm = t->pre_c ? pl.B : (uint64_t)pl.W * pl.B;
+      if (n && (uint64_t)count * per_msm >= (1ull << 31))
+        throw InvalidArgument("msm_dev_many: count * buckets per MSM must be < 2^31");
+      if (!range_ok(sc_offset, (uint64_t)count * n, s->n)) throw InvalidArgument("msm_dev_many: scalar range exceeds the handle");
+      MsmEngine<F>& e = engine();
+      const uint32_t* sc = s->buf.as<uint32_t>() + 8 * sc_offset;
+      if (t->pre_c)
+        c.launches += e.run_many(t->buf.as<Affine<F>>(), sc, n, count, c.stream, t->pre_c, (uint32_t)t->n, (uint32_t)offset);
+      else
+        c.launches += e.run_many(t->buf.as<Affine<F>>() + offset, sc, n, count, c.stream, force_c, 0, 0);
+      std::vector<uint8_t> host((size_t)count * (PT + sizeof(int)));
+      int* flags = reinterpret_cast<int*>(host.data() + (size_t)count * PT);
+      CUDA_CHECK(cudaMemcpyAsync(host.data(), e.many_out.p, (size_t)count * PT, cudaMemcpyDeviceToHost, c.stream));
+      CUDA_CHECK(cudaMemcpyAsync(flags, e.many_flag.p, (size_t)count * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
+      CUDA_CHECK(cudaStreamSynchronize(c.stream));
+      for (uint32_t j = 0; j < count; j++) {
+        if (flags[j]) memset(out_xy + (size_t)j * PT, 0, PT);
+        else memcpy(out_xy + (size_t)j * PT, host.data() + (size_t)j * PT, PT);
+        if (out_is_inf) out_is_inf[j] = flags[j];
+      }
+    });
+  }
+
   static int table_precompute(uint64_t table, int window_bits) {
     return guarded([&](Context& c) {
       Resource* t = need(table, KIND, "table_precompute");

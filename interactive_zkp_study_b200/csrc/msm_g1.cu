@@ -113,6 +113,10 @@ int zkp_g1_msm_dev_batch(uint64_t table, uint32_t count, const uint64_t* scalars
   return Api::msm_batch(table, count, scalars, sc_offsets, offsets, lens, out_xy, out_is_inf);
 }
 int zkp_g1_table_precompute(uint64_t table, int window_bits) { return Api::table_precompute(table, window_bits); }
+int zkp_g1_msm_dev_many(uint64_t table, uint64_t offset, uint64_t n, uint32_t count, uint64_t scalars, uint64_t sc_offset,
+                        uint8_t* out_xy, int* out_is_inf) {
+  return Api::msm_dev_many(table, offset, n, count, scalars, sc_offset, out_xy, out_is_inf);
+}
 
 // G1 or G2 table -> canonical affine points on the host
 int zkp_table_download(uint64_t table, uint64_t offset, uint64_t n, uint8_t* out_pts) {

@@ -61,6 +61,10 @@ int zkp_g2_table_validate(uint64_t table, uint64_t offset, uint64_t n, int subgr
   return Api::table_validate(table, offset, n, subgroup_check, first_bad);
 }
 int zkp_g2_table_precompute(uint64_t table, int window_bits) { return Api::table_precompute(table, window_bits); }
+int zkp_g2_msm_dev_many(uint64_t table, uint64_t offset, uint64_t n, uint32_t count, uint64_t scalars, uint64_t sc_offset,
+                        uint8_t* out_xy, int* out_is_inf) {
+  return Api::msm_dev_many(table, offset, n, count, scalars, sc_offset, out_xy, out_is_inf);
+}
 int zkp_g2_fixed_base_mul(const uint8_t base_xy[128], const uint8_t* scalars, uint64_t n, uint64_t* out_table) {
   return Api::fixed_base_host(base_xy, scalars, n, out_table);
 }

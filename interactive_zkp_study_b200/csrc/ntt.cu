@@ -337,12 +337,18 @@ static constexpr uint32_t NTT_ELEMS_PER_THREAD = 8;
 
 int ntt_device(Context& c, Fr* data, Fr* scratch, uint32_t log_n, const FrBytes& omega, bool inverse,
                const FrBytes* coset_shift, uint32_t log_batch) {
-  if (log_n > FrParams::TWO_ADICITY) throw InvalidArgument("ntt: log_n exceeds the 2-adicity of Fr (28)");
   if (log_n + log_batch > 31) throw InvalidArgument("ntt: batch * n must be < 2^32");
+  return ntt_device_count(c, data, scratch, log_n, omega, inverse, coset_shift, uint64_t(1) << log_batch);
+}
+
+int ntt_device_count(Context& c, Fr* data, Fr* scratch, uint32_t log_n, const FrBytes& omega, bool inverse,
+                     const FrBytes* coset_shift, uint64_t count) {
+  if (log_n > FrParams::TWO_ADICITY) throw InvalidArgument("ntt: log_n exceeds the 2-adicity of Fr (28)");
+  if (count == 0 || (count << log_n) >= (uint64_t(1) << 32)) throw InvalidArgument("ntt: batch * n must be < 2^32");
   int launches = 0;
-  // 2^log_batch independent transforms of 2^log_n contiguous elements: the same passes over a longer
+  // `count` independent transforms of 2^log_n contiguous elements: the same passes over a longer
   // array (tile indices simply run on into the next transform; twiddles depend on the position inside one)
-  const uint32_t n = 1u << (log_n + log_batch);
+  const uint32_t n = (uint32_t)(count << log_n);
   const Fr* tw = twiddle_table(c, omega, inverse, log_n, &launches);
   const Fr* pre = nullptr;
   const Fr* post = nullptr;
@@ -368,7 +374,8 @@ int ntt_device(Context& c, Fr* data, Fr* scratch, uint32_t log_n, const FrBytes&
   a.log_g = 0;
   if (log_n < (uint32_t)NTT_LOG_TILE) {
     a.log_g = (uint32_t)NTT_LOG_TILE - log_n;
-    if (a.log_g > log_batch) a.log_g = log_batch;
+    // a first-pass tile holds 2^log_g whole transforms: 2^log_g must divide the batch
+    while (count & ((uint64_t(1) << a.log_g) - 1)) a.log_g--;
   }
   a.bitrev_in = 1;
   // a single-pass transform lives entirely inside one tile, which is read completely before it is

@@ -20,6 +20,9 @@ struct FrBytes {
 // log_batch: transform 2^log_batch contiguous vectors of n elements each in the same launches.
 int ntt_device(Context& c, Fr* data, Fr* scratch, uint32_t log_n, const FrBytes& omega, bool inverse,
                const FrBytes* coset_shift, uint32_t log_batch = 0);
+// The same for any number `count` of contiguous transforms (count * 2^log_n < 2^32).
+int ntt_device_count(Context& c, Fr* data, Fr* scratch, uint32_t log_n, const FrBytes& omega, bool inverse,
+                     const FrBytes* coset_shift, uint64_t count);
 
 // x^(2^k), k < 32, in Montgomery form on the device (cached per x); `inverted`: of x^-1 instead.
 const Fr* pow2_table(Context& c, const FrBytes& x, bool inverted, int* launches);

@@ -1385,3 +1385,4 @@ int zkp_groth16_quotient(const uint8_t* a, const uint8_t* b, const uint8_t* cc, 
 }  // extern "C"
 
 #include "qap.cuh"
+#include "groth16_batch.cuh"

@@ -286,6 +286,27 @@ def groth16_quotient_dev(a, b, c, length, z, z_len, want_remainder=True):
             DeviceHandle(hr.value, z_len - 1, "fr") if want_remainder else None)
 
 
+def groth16_quotient_batch_dev(a, b, c, length, count, z, z_len):
+    """Handle of count quotients (2 * length - z_len coefficients each, back to back); proof j's a, b, c at j * length."""
+    hq = ctypes.c_uint64()
+    check(_lib.lib().zkp_groth16_quotient_batch_dev(a.handle, b.handle, c.handle, length, count, z.handle, z_len,
+                                                    ctypes.byref(hq)))
+    return DeviceHandle(hq.value, count * (2 * length - z_len), "fr")
+
+
+def groth16_batch_scalars_dev(uA, uB, h, rx, k, m_priv, rs, ss):
+    """(scA, scB, scC) handles of len(rs) proofs: uA | 1 | r, uB | 1 | s and r uB + s uA | r | rx | H | s | s r."""
+    count = len(rs)
+    ha, hb, hc = ctypes.c_uint64(), ctypes.c_uint64(), ctypes.c_uint64()
+    check(_lib.lib().zkp_groth16_batch_scalars_dev(uA.handle, uB.handle, h.handle if h is not None else 0,
+                                                   rx.handle if rx is not None else 0, k, m_priv, count,
+                                                   buf(fr_vec_bytes(rs)), buf(fr_vec_bytes(ss)), ctypes.byref(ha),
+                                                   ctypes.byref(hb), ctypes.byref(hc)))
+    nC = 2 * k + 2 + m_priv
+    return (DeviceHandle(ha.value, count * (k + 2), "fr"), DeviceHandle(hb.value, count * (k + 2), "fr"),
+            DeviceHandle(hc.value, count * nC, "fr"))
+
+
 def groth16_msms_dev(ta, sa, na, tb2, sb, nb, tc, sc, nc):
     """A (G1), B (G2), C' (G1) of one proof with the G2 MSM overlapped on a second stream."""
     oa, ob, oc = bytearray(64), bytearray(128), bytearray(64)
@@ -388,6 +409,19 @@ def g1_msm_dev_batch(table, items):
     check(_lib.lib().zkp_g1_msm_dev_batch(table.handle, k, arr([it[0].handle for it in items]), arr([it[1] for it in items]),
                                           arr([it[2] for it in items]), arr([it[3] for it in items]), buf(out), inf))
     return [g1_from_bytes(bytes(out[64 * i:64 * i + 64]), bool(inf[i])) for i in range(k)]
+
+
+def msm_dev_many(table, offset, n, count, scalars, sc_offset=0):
+    """count MSMs over the points [offset, offset + n) of `table` (G1 or G2 by its kind), vector j of scalars at
+    sc_offset + j * n -> list of count points.  One Pippenger pass for the whole batch."""
+    g1 = table.kind == "g1"
+    sz = 64 if g1 else 128
+    out = bytearray(sz * max(count, 1))
+    inf = (ctypes.c_int * max(count, 1))()
+    fn = _lib.lib().zkp_g1_msm_dev_many if g1 else _lib.lib().zkp_g2_msm_dev_many
+    check(fn(table.handle, offset, n, count, scalars.handle, sc_offset, buf(out), inf))
+    dec = g1_from_bytes if g1 else g2_from_bytes
+    return [dec(bytes(out[sz * j:sz * j + sz]), bool(inf[j])) for j in range(count)]
 
 
 def g1_msm_dev_partial(table, offset, scalars, sc_offset, n, out_addr=None):
@@ -710,6 +744,17 @@ def fr_ap_interpolate_dev(values, k, out, scale=None, off=0, out_off=0):
     """out[0..k) = coefficients of the polynomial p of degree < k with p(j + 1) = values[j], times scale."""
     sc = fe_bytes(scale) if scale is not None else None
     check(_lib.lib().zkp_fr_ap_interpolate_dev(values.handle, off, k, buf(sc), out.handle, out_off))
+
+
+def sparse_matvec_many_dev(matrix, vec, out, count, vec_off=0, out_off=0):
+    """sparse_matvec_dev over count vectors: witness j at vec_off + j * cols, result j at out_off + j * rows."""
+    check(_lib.lib().zkp_sparse_matvec_many_dev(matrix.handle, vec.handle, vec_off, out.handle, out_off, count))
+
+
+def fr_ap_interpolate_many_dev(values, k, count, out, scale=None, off=0, out_off=0):
+    """fr_ap_interpolate_dev over count value vectors of k entries each, back to back."""
+    sc = fe_bytes(scale) if scale is not None else None
+    check(_lib.lib().zkp_fr_ap_interpolate_many_dev(values.handle, off, k, count, buf(sc), out.handle, out_off))
 
 
 def fr_ap_vanishing_dev(k):

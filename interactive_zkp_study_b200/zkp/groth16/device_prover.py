@@ -113,6 +113,96 @@ def prove(key, uA, uB, uC, Z, rx_priv, r, s, keep_quotient=False):
     return out
 
 
+# ------------------------------------------------------------------ many proofs of one circuit per pass
+def _many_msm_shape(table, n):
+    """(windows W, buckets per MSM) of a many-MSM pass over n rows of `table`: the table's own width when it is
+    window-precomputed (all windows share one bucket set), else the automatic width of csrc/msm.cuh msm_plan."""
+    c = getattr(table, "pre_c", 0)
+    if not c:
+        c = min(max(max(n, 1).bit_length() - 1 - 4, 4), 16)
+    W = -(-255 // c)
+    B = 1 << (c - 1)
+    return W, (B if getattr(table, "pre_c", 0) else W * B)
+
+
+def plan_chunk(key, count, free_bytes):
+    """Largest number of proofs per pass of prove_batch: within the 32-bit entry and 31-bit bucket numbering of the
+    many-MSM (count * W * n < 2^32, count * buckets < 2^31), the 32-bit batched transforms of the quotient, and half
+    of `free_bytes` of device memory at the working set estimated below.  At least 1, at most count."""
+    k, mp = key.k, key.m_priv
+    nC = tc_rows(k, mp)
+    lg1 = (2 * k - 2).bit_length()                     # transforms of 2^lg1 >= 2k - 1 points
+    limit = ((1 << 32) - 1) >> lg1
+    g1_ws = g2_ws = 0
+    for table, n, xyzz in ((key.TA, k + 2, 128), (key.TB2, k + 2, 256), (key.TC, nC, 128)):
+        W, per = _many_msm_shape(table, n)
+        limit = min(limit, ((1 << 32) - 1) // (W * n), ((1 << 31) - 1) // per)
+        ws = 8 * W * n + per * (3 * xyzz + 12)          # codes + sorted entries; buckets, partials, levels, counts
+        if xyzz == 256:
+            g2_ws = max(g2_ws, ws)
+        else:
+            g1_ws = max(g1_ws, ws)
+    per_proof = (g1_ws + g2_ws                            # the G1 and the G2 engine keep their own workspace
+                 + 32 * (2 * (k + 2) + nC)                # scalar vectors
+                 + 32 * (5 << lg1)                        # quotient transforms
+                 + 32 * (4 * k + mp))                     # chunk copies of uA, uB, uC, rx_priv and H
+    limit = min(limit, (free_bytes // 2) // per_proof)
+    return int(max(1, min(limit, count)))
+
+
+def _slice(h, off, n):
+    out = native.scalars_alloc(n)
+    if n:
+        native.scalars_copy(out, 0, h, off, n)
+    return out
+
+
+def prove_batch(key, uA, uB, uC, Z, rx_priv, rs, ss, keep_quotient=False, chunk=None):
+    """count = len(rs) proofs of the circuit of `key`, bit-identical to count calls of prove: proof j from uA, uB, uC
+    at offset j * k, rx_priv at offset j * m_priv, and (rs[j], ss[j]).  Per chunk of proofs: one batched quotient,
+    one scalar assembly and three many-MSMs (TA, TB2, TC), so the launch count does not grow with count.
+    chunk=None picks the largest chunk the 32-bit limits and the free device memory allow (plan_chunk); the
+    result does not depend on it.  Returns the list of (A, B, C), and with keep_quotient also the handle of the
+    count quotients (k - 1 coefficients each, back to back)."""
+    k, mp = key.k, key.m_priv
+    count = len(rs)
+    if len(ss) != count:
+        raise ValueError("prove_batch: rs and ss differ in length (%d, %d)" % (count, len(ss)))
+    if chunk is not None and int(chunk) <= 0:
+        raise ValueError("prove_batch: chunk must be positive")
+    for name, h, need in (("uA", uA, count * k), ("uB", uB, count * k), ("uC", uC, count * k),
+                          ("rx_priv", rx_priv, count * mp), ("Z", Z, k + 1)):
+        if h is None or h.n < need:
+            raise ValueError("prove_batch: %s holds %s values, needs %d" % (name, None if h is None else h.n, need))
+    if count == 0:
+        return []
+    rs = [int(r) % R for r in rs]
+    ss = [int(s) % R for s in ss]
+    step = min(int(chunk), count) if chunk is not None else plan_chunk(key, count, native.device_mem_info()[0])
+    nC = tc_rows(k, mp)
+    H = native.scalars_alloc(count * (k - 1)) if keep_quotient else None
+    proofs = []
+    for j0 in range(0, count, step):
+        cnt = min(step, count - j0)
+        whole = cnt == count
+        a, b, c = (h if whole else _slice(h, j0 * k, cnt * k) for h in (uA, uB, uC))
+        x = rx_priv if whole or not mp else _slice(rx_priv, j0 * mp, cnt * mp)
+        hq = native.groth16_quotient_batch_dev(a, b, c, k, cnt, Z, k + 1)
+        scA, scB, scC = native.groth16_batch_scalars_dev(a, b, hq, x, k, mp, rs[j0:j0 + cnt], ss[j0:j0 + cnt])
+        As = native.msm_dev_many(key.TA, 0, k + 2, cnt, scA)
+        Bs = native.msm_dev_many(key.TB2, 0, k + 2, cnt, scB)
+        Cs = native.msm_dev_many(key.TC, 0, nC, cnt, scC)
+        if H is not None and k > 1:
+            native.scalars_copy(H, j0 * (k - 1), hq, 0, cnt * (k - 1))
+        for h in (scA, scB, scC, hq):
+            h.free()
+        if not whole:
+            for h in (a, b, c) + ((x,) if mp else ()):
+                h.free()
+        proofs.extend((g1_from_ints(A), g2_from_ints(B), g1_from_ints(C)) for A, B, C in zip(As, Bs, Cs))
+    return (proofs, H) if keep_quotient else proofs
+
+
 # ------------------------------------------------------------------ the same proof over the GPUs of one box
 class ShardedDeviceKey:
     """This rank's contiguous row range of each of the three CRS tables (sharded.shard_range of the

@@ -116,6 +116,22 @@ def witness_polys(dev, w, lcm=True):
     return tuple(out)
 
 
+def witness_polys_batch(dev, W, count, lcm=True, off=0):
+    """witness_polys for count witnesses at once: witness j at W[off + j * m]; returns uA, uB, uC handles of
+    count * k coefficients, proof j's at j * k.  Two launches of sparse products and two batched interpolations
+    per matrix, whatever count is."""
+    k = dev.k
+    out = []
+    ev = native.scalars_alloc(count * k)
+    for mat, sc in zip(dev.mats, _scales(k, lcm)):
+        native.sparse_matvec_many_dev(mat, W, ev, count, vec_off=off)
+        u = native.scalars_alloc(count * k)
+        native.fr_ap_interpolate_many_dev(ev, k, count, u, scale=sc if lcm else None)
+        out.append(u)
+    ev.free()
+    return tuple(out)
+
+
 class Keys:
     """Proving key (device tables of device_prover.DeviceKey) + the verifier's small CRS part."""
 
@@ -229,3 +245,42 @@ def prove(keys, dev, w, r, s, keep=False):
     for h in (uA, uB, uC):
         h.free()
     return out
+
+
+def _selection_matrix(keys, m):
+    """The private-wire selection as an m_priv x m 0/1 sparse matrix (cached on keys): one sparse product gathers the
+    private wires of every witness of a batch."""
+    if getattr(keys, "_sel_mat", None) is None:
+        idx = keys.priv_idx
+        keys._sel_mat = native.sparse_load(list(range(len(idx) + 1)), idx, [1] * len(idx), len(idx), m)
+    return keys._sel_mat
+
+
+def prove_batch(keys, dev, W, rs, ss, chunk=None):
+    """[prove(keys, dev, w_j, rs[j], ss[j]) for each witness w_j = W[j * m : (j + 1) * m]] in batched passes:
+    witness polynomials, private-wire gathers, quotients and the three MSMs of a chunk of proofs each run in a
+    fixed number of launches (device_prover.prove_batch).  chunk=None: device_prover.plan_chunk."""
+    count = len(rs)
+    if len(ss) != count:
+        raise ValueError("prove_batch: rs and ss differ in length (%d, %d)" % (count, len(ss)))
+    if chunk is not None and int(chunk) <= 0:
+        raise ValueError("prove_batch: chunk must be positive")
+    if W is None or W.n < count * dev.m:
+        raise ValueError("prove_batch: W holds %s values, needs %d" % (None if W is None else W.n, count * dev.m))
+    if count == 0:
+        return []
+    key = keys.device_key
+    mp = len(keys.priv_idx)
+    step = min(int(chunk), count) if chunk is not None else device_prover.plan_chunk(key, count, native.device_mem_info()[0])
+    sel = _selection_matrix(keys, dev.m) if mp else None
+    proofs = []
+    for j0 in range(0, count, step):
+        cnt = min(step, count - j0)
+        uA, uB, uC = witness_polys_batch(dev, W, cnt, keys.lcm, off=j0 * dev.m)
+        rx = native.scalars_alloc(cnt * mp)
+        if mp:
+            native.sparse_matvec_many_dev(sel, W, rx, cnt, vec_off=j0 * dev.m)
+        proofs.extend(device_prover.prove_batch(key, uA, uB, uC, keys.Z, rx, rs[j0:j0 + cnt], ss[j0:j0 + cnt], chunk=cnt))
+        for h in (uA, uB, uC, rx):
+            h.free()
+    return proofs
