@@ -296,6 +296,57 @@ int zkp_plonk_coset_setup_dev(uint64_t n, uint32_t ext, const uint8_t g[32], con
                               uint64_t zh8_out);
 int zkp_plonk_quotient_dev(const uint64_t evals[12], uint64_t n, uint32_t ext, uint64_t x, uint64_t l1f, uint64_t zh8,
                            const uint8_t beta[32], const uint8_t gamma[32], const uint8_t alpha[32], uint64_t t_out);
+/* ---- batch PLONK proving: count proofs of one circuit per call (zkp/plonk/device_prover.py prove_batch) ----------
+ * The rounds of zkp/plonk/prover/round1..5.py for count witnesses in launches whose number does not depend on
+ * count.  Every proof has its own challenges: betas, gammas, alphas, zetas are count x 32 B canonical arrays.  Each
+ * entry gives, per proof, exactly what its single-proof counterpart above gives.  Ranges are checked before any
+ * launch (ZKP_ERR_INVALID_ARGUMENT).
+ * zkp_fr_ntt_many_dev: count contiguous transforms of 2^log_n at offset (zkp_fr_ntt_dev each; fft / ifft /
+ *   coset_fft of zkp/plonk/polynomial.py:292-378, utils.py:145-205); count * 2^log_n < 2^32.
+ * zkp_plonk_blind_many_dev: dst_v = src_v + (b_v0 + .. + b_v,k-1 x^(k-1))(x^n - 1) at dst_stride >= n + k, v < nvec,
+ *   src_v = n coefficients at src_off + v * src_stride, blinds nvec x k (round1.py:38-108 / round2.py:45-85 blinding).
+ * zkp_plonk_perm_terms_many_dev: zkp_plonk_perm_terms_dev per proof (permutation.py:120-135), witness j at
+ *   off + j * n of a, b, c; sigma shared; num / den: count * n.
+ * zkp_fr_scan_many_dev: zkp_fr_scan_dev over count segments of seg elements, each starting afresh (the accumulator
+ *   z_j of permutation.py:120-135 starts at 1 in every proof).
+ * zkp_plonk_coset_inputs_many_dev: the round-3 transform inputs: 3 count wire blocks (stride n + 2) and count z
+ *   blocks (stride n + 3) zero-padded to 2^log_N, Montgomery, in the order a_*, b_*, c_*, z_* (round3.py:56-184).
+ * zkp_plonk_quotient_many_dev: zkp_plonk_quotient_dev per proof on those 4 count blocks; circuit = the 8 shared
+ *   coset evaluations q_l, q_r, q_o, q_m, q_c, s_sigma1..3; t_out: count blocks of N = ext * n (round3.py:114-147).
+ * zkp_plonk_divisible_many_dev: lowest j whose t_j has a non-zero coefficient at 3n + 6 or above, UINT64_MAX if
+ *   none (the divisibility check of round3.py:150-155).
+ * zkp_plonk_split_t_many_dev: t_lo | t_mid | t_hi of every proof from Montgomery t blocks, canonical, each at stride
+ *   n + 6 with t_lo, t_mid zero-padded; vector part * count + j (round3.py:169-171).
+ * zkp_fr_poly_eval_many_dev: groups x count Horner evaluations (round4.py:39-81, polynomial.py:85-106): group g's
+ *   vector of proof j at offs[g] + j * strides[g] (0: one vector shared by all proofs), lens[g] coefficients, at
+ *   points[sel[g] * count + j]; out[g * count + j]; at most 16 groups.
+ * zkp_fr_lincomb_many_dev: dst_j[i] = sum_k coeffs[j][k] src_k,j[i] + (i == 0 ? coeffs[j][K] : 0), i < n, sources
+ *   shared or per proof as above, coeffs count x (K + 1) (round5.py:90-160); dst must not overlap a source.
+ * zkp_fr_div_linear_many_dev: zkp_fr_div_linear_dev per proof (round5.py:165-171, kzg.py:95-104), p_j at
+ *   src_off + j * src_stride (len coefficients), quotient j at dst_off + j * dst_stride; zeta_j = 0 is a shift. */
+int zkp_fr_ntt_many_dev(uint64_t scalars, uint64_t offset, uint32_t log_n, const uint8_t omega[32], int inverse,
+                        const uint8_t* coset_shift, uint32_t count);
+int zkp_plonk_blind_many_dev(uint64_t src, uint64_t src_off, uint64_t src_stride, uint64_t n, uint32_t nvec,
+                             const uint8_t* blinds, uint32_t k, uint64_t dst, uint64_t dst_off, uint64_t dst_stride);
+int zkp_plonk_perm_terms_many_dev(uint64_t a, uint64_t b, uint64_t c, uint64_t off, uint64_t s1, uint64_t s2, uint64_t s3,
+                                  uint64_t n, uint32_t count, const uint8_t omega[32], const uint8_t* betas,
+                                  const uint8_t* gammas, uint64_t num, uint64_t den);
+int zkp_fr_scan_many_dev(int op, uint64_t dst, uint64_t dst_off, uint64_t src, uint64_t src_off, uint64_t seg,
+                         uint32_t count);
+int zkp_plonk_coset_inputs_many_dev(uint64_t wires, uint64_t z, uint64_t n, uint32_t count, uint32_t log_N, uint64_t out);
+int zkp_plonk_quotient_many_dev(uint64_t evals, const uint64_t circuit[8], uint64_t n, uint32_t ext, uint32_t count,
+                                uint64_t x, uint64_t l1f, uint64_t zh8, const uint8_t* betas, const uint8_t* gammas,
+                                const uint8_t* alphas, uint64_t t_out);
+int zkp_plonk_divisible_many_dev(uint64_t t, uint64_t n, uint32_t ext, uint32_t count, uint64_t* first_bad);
+int zkp_plonk_split_t_many_dev(uint64_t t, uint64_t n, uint32_t ext, uint32_t count, uint64_t out);
+int zkp_fr_poly_eval_many_dev(uint32_t groups, const uint64_t* handles, const uint64_t* offs, const uint64_t* strides,
+                              const uint64_t* lens, const uint32_t* sel, uint32_t count, uint32_t npsets,
+                              const uint8_t* points, uint8_t* out);
+int zkp_fr_lincomb_many_dev(uint64_t dst, uint64_t dst_off, uint64_t dst_stride, uint64_t n, uint32_t count, uint32_t K,
+                            const uint64_t* handles, const uint64_t* offs, const uint64_t* strides, const uint64_t* lens,
+                            const uint8_t* coeffs);
+int zkp_fr_div_linear_many_dev(uint64_t src, uint64_t src_off, uint64_t src_stride, uint64_t len, uint32_t count,
+                               const uint8_t* zetas, uint64_t dst, uint64_t dst_off, uint64_t dst_stride);
 /* General product and exact/long division over Fr in coefficient form
  * (Polynomial.__mul__ polynomial.py:144-159; poly_div polynomial.py:385-435). */
 int zkp_fr_poly_mul(const uint8_t* a, uint64_t a_len, const uint8_t* b, uint64_t b_len, uint8_t* out);

@@ -121,6 +121,17 @@ PROTOTYPES = {
     "zkp_plonk_perm_terms_dev": (c_int, [u64, u64, u64, u64, u64, u64, u64, vp, vp, vp, u64, u64]),
     "zkp_plonk_coset_setup_dev": (c_int, [u64, u32, vp, vp, vp, vp, u64, u64, u64]),
     "zkp_plonk_quotient_dev": (c_int, [u64p, u64, u32, u64, u64, u64, vp, vp, vp, u64]),
+    "zkp_fr_ntt_many_dev": (c_int, [u64, u64, u32, vp, c_int, vp, u32]),
+    "zkp_plonk_blind_many_dev": (c_int, [u64, u64, u64, u64, u32, vp, u32, u64, u64, u64]),
+    "zkp_plonk_perm_terms_many_dev": (c_int, [u64, u64, u64, u64, u64, u64, u64, u64, u32, vp, vp, vp, u64, u64]),
+    "zkp_fr_scan_many_dev": (c_int, [c_int, u64, u64, u64, u64, u64, u32]),
+    "zkp_plonk_coset_inputs_many_dev": (c_int, [u64, u64, u64, u32, u32, u64]),
+    "zkp_plonk_quotient_many_dev": (c_int, [u64, u64p, u64, u32, u32, u64, u64, u64, vp, vp, vp, u64]),
+    "zkp_plonk_divisible_many_dev": (c_int, [u64, u64, u32, u32, u64p]),
+    "zkp_plonk_split_t_many_dev": (c_int, [u64, u64, u32, u32, u64]),
+    "zkp_fr_poly_eval_many_dev": (c_int, [u32, u64p, u64p, u64p, u64p, ctypes.POINTER(u32), u32, u32, vp, vp]),
+    "zkp_fr_lincomb_many_dev": (c_int, [u64, u64, u64, u64, u32, u32, u64p, u64p, u64p, u64p, vp]),
+    "zkp_fr_div_linear_many_dev": (c_int, [u64, u64, u64, u64, u32, vp, u64, u64, u64]),
     "zkp_sparse_load": (c_int, [vp, vp, vp, u64, u64, u64, u64p]),
     "zkp_sparse_matvec_dev": (c_int, [u64, u64, u64, u64, u64]),
     "zkp_fr_ap_interpolate_dev": (c_int, [u64, u64, u64, vp, u64, u64]),

@@ -714,6 +714,108 @@ def plonk_quotient_dev(evals12, n, ext, x, l1f, zh8, beta, gamma, alpha, t_out):
                                             buf(fe_bytes(gamma)), buf(fe_bytes(alpha)), t_out.handle))
 
 
+# ------------------------------------------------------------------ batch PLONK proving (count proofs per call)
+def _u64s(vals):
+    return (ctypes.c_uint64 * max(len(vals), 1))(*vals)
+
+
+def _fr_rows(what, rows, count, width):
+    """count rows of `width` scalars -> bytes (reduced mod r); the C side reads exactly count * width of them."""
+    rows = [list(r) for r in rows]
+    if len(rows) != count or any(len(r) != width for r in rows):
+        raise ValueError("%s: expected %d rows of %d scalars" % (what, count, width))
+    return fr_vec_bytes([int(x) % R_MOD for r in rows for x in r])
+
+
+def ntt_many_dev(h, off, log_n, count, omega, inverse=False, coset_shift=None):
+    """count contiguous transforms of 2^log_n elements from h[off] (ntt_dev each)."""
+    cs = fe_bytes(coset_shift) if coset_shift is not None else None
+    check(_lib.lib().zkp_fr_ntt_many_dev(h.handle, off, log_n, buf(fe_bytes(omega)), 1 if inverse else 0, buf(cs), count))
+
+
+def plonk_blind_many_dev(src, src_off, src_stride, n, nvec, blinds, dst, dst_off, dst_stride):
+    """dst_v = src_v + (b_v0 + b_v1 x + ...)(x^n - 1) at dst_stride, v < nvec; blinds: nvec lists of k scalars."""
+    k = len(blinds[0]) if nvec else 0
+    flat = _fr_rows("plonk_blind_many_dev: blinds", blinds, nvec, k)
+    check(_lib.lib().zkp_plonk_blind_many_dev(src.handle, src_off, src_stride, n, nvec, buf(flat) if k else None, k,
+                                              dst.handle, dst_off, dst_stride))
+
+
+def plonk_perm_terms_many_dev(a, b, c, off, s1, s2, s3, n, omega, betas, gammas, num, den):
+    """plonk_perm_terms_dev for len(betas) proofs, witness j at off + j * n of a, b, c."""
+    count = len(betas)
+    ch = _fr_rows("plonk_perm_terms_many_dev: betas, gammas", [betas, gammas], 2, count)
+    check(_lib.lib().zkp_plonk_perm_terms_many_dev(a.handle, b.handle, c.handle, off, s1.handle, s2.handle, s3.handle, n,
+                                                   count, buf(fe_bytes(omega)), buf(ch[:32 * count]),
+                                                   buf(ch[32 * count:]), num.handle, den.handle))
+
+
+def scan_many_dev(op, dst, dst_off, src, src_off, seg, count):
+    """scan_dev over count segments of seg elements, each starting afresh (op 0 product, 1 sum)."""
+    check(_lib.lib().zkp_fr_scan_many_dev(op, dst.handle, dst_off, src.handle, src_off, seg, count))
+
+
+def plonk_coset_inputs_many_dev(wires, z, n, count, log_N, out):
+    check(_lib.lib().zkp_plonk_coset_inputs_many_dev(wires.handle, z.handle, n, count, log_N, out.handle))
+
+
+def plonk_quotient_many_dev(evals, circuit8, n, ext, x, l1f, zh8, betas, gammas, alphas, t_out):
+    """plonk_quotient_dev for len(betas) proofs: evals holds the blocks a_*, b_*, c_*, z_* of N = ext * n each."""
+    count = len(betas)
+    if len(circuit8) != 8:
+        raise ValueError("plonk_quotient_many_dev: 8 circuit coset evaluations, got %d" % len(circuit8))
+    ch = _fr_rows("plonk_quotient_many_dev: betas, gammas, alphas", [betas, gammas, alphas], 3, count)
+    check(_lib.lib().zkp_plonk_quotient_many_dev(evals.handle, _u64s([h.handle for h in circuit8]), n, ext, count,
+                                                 x.handle, l1f.handle, zh8.handle, buf(ch[:32 * count]),
+                                                 buf(ch[32 * count:64 * count]), buf(ch[64 * count:]), t_out.handle))
+
+
+def plonk_divisible_many_dev(t, n, ext, count):
+    """Lowest proof index whose quotient block has a non-zero coefficient at 3n + 6 or above, or None."""
+    bad = ctypes.c_uint64()
+    check(_lib.lib().zkp_plonk_divisible_many_dev(t.handle, n, ext, count, ctypes.byref(bad)))
+    return _first_bad(bad.value)
+
+
+def plonk_split_t_many_dev(t, n, ext, count, out):
+    check(_lib.lib().zkp_plonk_split_t_many_dev(t.handle, n, ext, count, out.handle))
+
+
+def fr_poly_eval_many_dev(groups, count, point_sets):
+    """groups = [(handle, offset, stride, length, point_set)] (stride 0: shared by every proof), point_sets = lists of
+    count points -> values[g][j] = p_g,j(point_sets[sel_g][j]).  One batched set of Horner launches."""
+    g = len(groups)
+    if not g or not count:
+        return [[] for _ in range(g)]
+    if any(not 0 <= it[4] < len(point_sets) for it in groups):
+        raise ValueError("fr_poly_eval_many_dev: a group names a point set that is not given")
+    out = bytearray(32 * g * count)
+    sel = (ctypes.c_uint32 * g)(*[it[4] for it in groups])
+    pts = _fr_rows("fr_poly_eval_many_dev: point_sets", point_sets, len(point_sets), count)
+    check(_lib.lib().zkp_fr_poly_eval_many_dev(g, _u64s([it[0].handle for it in groups]), _u64s([it[1] for it in groups]),
+                                               _u64s([it[2] for it in groups]), _u64s([it[3] for it in groups]), sel, count,
+                                               len(point_sets), buf(pts), buf(out)))
+    vals = fr_vec_from_bytes(bytes(out))
+    return [vals[i * count:(i + 1) * count] for i in range(g)]
+
+
+def lincomb_many_dev(dst, dst_off, dst_stride, n, count, sources, coeffs):
+    """dst_j[i] = sum_k coeffs[j][k] * src_k,j[i] (+ coeffs[j][K] at i = 0), i < n; sources = [(handle, offset, stride,
+    length)] with stride 0 for a vector shared by every proof; coeffs: count rows of K + 1 scalars."""
+    K = len(sources)
+    flat = _fr_rows("lincomb_many_dev: coeffs", coeffs, count, K + 1)
+    check(_lib.lib().zkp_fr_lincomb_many_dev(dst.handle, dst_off, dst_stride, n, count, K, _u64s([s[0].handle for s in sources]),
+                                             _u64s([s[1] for s in sources]), _u64s([s[2] for s in sources]),
+                                             _u64s([s[3] for s in sources]), buf(flat) if count else None))
+
+
+def div_linear_many_dev(src, src_off, src_stride, length, zetas, dst, dst_off, dst_stride):
+    """div_linear_dev for len(zetas) polynomials of `length` coefficients at src_off + j * src_stride."""
+    zs = fr_vec_bytes([int(z) % R_MOD for z in zetas])
+    check(_lib.lib().zkp_fr_div_linear_many_dev(src.handle, src_off, src_stride, length, len(zetas),
+                                                buf(zs) if zetas else None, dst.handle, dst_off, dst_stride))
+
+
 # ------------------------------------------------------------------ QAP over {1..k} at scale (SURVEY 8 f2)
 def sparse_load(row_ptr, col_idx, values, rows, cols):
     """CSR matrix with Fr values -> device handle.  row_ptr: rows+1 offsets, col_idx: column of each

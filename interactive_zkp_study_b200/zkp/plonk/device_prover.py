@@ -239,3 +239,177 @@ def prove(key, a_vals, b_vals, c_vals, blinds=None, keep=False):
     for h in (wires["a"], wires["b"], wires["c"], z, t, r, W, Ww, P):
         h.free()
     return proof
+
+
+# ------------------------------------------------------------------ many proofs of one circuit per pass
+_NOT_DIVISIBLE = "제약 다항식이 Z_H(x)로 나누어 떨어지지 않습니다. 회로 또는 witness에 오류가 있습니다."
+# the many-MSMs of one pass: (scalar vectors per proof, padded length - n) -- rounds 1, 2, 3 and 5
+_PASS_MSMS = ((3, 2), (1, 3), (3, 6), (2, 5))
+
+
+def plan_chunk(key, count, free_bytes):
+    """Largest number of proofs per pass of prove_batch: within the 32-bit entry and 31-bit bucket numbering of the
+    many-MSM (vectors * W * L < 2^32, vectors * buckets < 2^31 at the padded length L of each round's vectors), the
+    32-bit batched coset transforms (4 * count * N8 < 2^32), and half of `free_bytes` of device memory at the working
+    set estimated below.  At least 1, at most count."""
+    from ..groth16.device_prover import _many_msm_shape
+    n, N = key.n, key.N8
+    limit = ((1 << 32) - 1) // (4 * N)
+    msm_ws = 0
+    for vecs, pad in _PASS_MSMS:
+        W, per = _many_msm_shape(key.srs_table, n + pad)
+        limit = min(limit, ((1 << 32) - 1) // (vecs * W * (n + pad)), ((1 << 31) - 1) // (vecs * per))
+        msm_ws = max(msm_ws, vecs * (8 * W * (n + pad) + per * (3 * 128 + 12)))   # entries; buckets and levels
+    per_proof = msm_ws + 32 * (9 * N + 20 * n + 64)     # coset blocks, transform scratch and the per-round vectors
+    limit = min(limit, (free_bytes // 2) // per_proof)
+    return int(max(1, min(limit, count)))
+
+
+def prove_batch(key, a_vals, b_vals, c_vals, count, blinds=None, chunk=None):
+    """count proofs of the circuit of `key`, proof j from the wire values at offset j * n of a_vals, b_vals, c_vals
+    and blinds[j] (9 scalars in the order of prove; fresh ones from `secrets` when blinds is None).  Proof j is
+    bit-identical to prove(key, a_j, b_j, c_j, blinds=blinds[j]).  Per chunk of proofs every round is a fixed number of
+    launches whatever the chunk size: batched transforms, per-proof challenge arrays, segmented scans and one many-MSM
+    per commitment group.  The transcripts stay on the host, one per proof.  chunk=None picks the largest chunk
+    plan_chunk allows; the result does not depend on it.  An unsatisfied witness raises the ValueError of prove,
+    naming the first failing proof, before any round-3 commitment of its chunk."""
+    n = key.n
+    count = int(count)
+    if key.ranks is not None:
+        raise ValueError("prove_batch: a sharded key is not supported (batch over one GPU's SRS)")
+    if chunk is not None and int(chunk) <= 0:
+        raise ValueError("prove_batch: chunk must be positive")
+    if count < 0:
+        raise ValueError("prove_batch: count must be >= 0")
+    for name, h in (("a_vals", a_vals), ("b_vals", b_vals), ("c_vals", c_vals)):
+        if h is None or h.n < count * n:
+            raise ValueError("prove_batch: %s holds %s values, needs %d" % (name, None if h is None else h.n, count * n))
+    if blinds is not None:
+        blinds = [list(b) for b in blinds]
+        if len(blinds) != count or any(len(b) != 9 for b in blinds):
+            raise ValueError("prove_batch: blinds must be %d lists of 9 scalars" % count)
+    if count == 0:
+        return []
+    if blinds is None:
+        blinds = [[secrets.randbelow(R) for _ in range(9)] for _ in range(count)]
+    blinds = [[int(b) % R for b in bl] for bl in blinds]
+    step = min(int(chunk), count) if chunk is not None else plan_chunk(key, count, native.device_mem_info()[0])
+    proofs = []
+    for j0 in range(0, count, step):
+        proofs.extend(_prove_chunk(key, a_vals, b_vals, c_vals, j0, min(step, count - j0), blinds))
+    return proofs
+
+
+def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds):
+    n, log_n, w, N = key.n, key.log_n, key.omega, key.N8
+    bl = blinds[j0:j0 + cnt]
+    trs = [Transcript() for _ in range(cnt)]
+    proofs = [Proof() for _ in range(cnt)]
+    tmp = []
+
+    def alloc(m):
+        h = native.scalars_alloc(m)
+        tmp.append(h)
+        return h
+
+    try:
+        # ---- round 1: 3 cnt inverse transforms, blinding at stride n + 2 (vector i * cnt + j: wire i of proof j)
+        ev = alloc(3 * cnt * n)
+        for i, vals in enumerate((a_vals, b_vals, c_vals)):
+            native.scalars_copy(ev, i * cnt * n, vals, j0 * n, cnt * n)
+        native.ntt_many_dev(ev, 0, log_n, 3 * cnt, w, inverse=True)
+        wires = alloc(3 * cnt * (n + 2))
+        native.plonk_blind_many_dev(ev, 0, n, n, 3 * cnt, [b[2 * i:2 * i + 2] for i in range(3) for b in bl], wires, 0, n + 2)
+        pts = native.msm_dev_many(key.srs_table, 0, n + 2, 3 * cnt, wires)
+        for j, (prf, tr) in enumerate(zip(proofs, trs)):
+            for i, name in enumerate("abc"):
+                setattr(prf, name + "_comm", g1_from_ints(pts[i * cnt + j]))
+                tr.append_point(name.encode() + b"_comm", getattr(prf, name + "_comm"))
+        # ---- round 2: grand products with per-proof beta, gamma; segmented scan; blinding at stride n + 3
+        betas = [int(tr.challenge_scalar(b"beta")) for tr in trs]
+        gammas = [int(tr.challenge_scalar(b"gamma")) for tr in trs]
+        zc = alloc(cnt * n)
+        if n > 1:
+            num, den = alloc(cnt * n), alloc(cnt * n)
+            native.plonk_perm_terms_many_dev(a_vals, b_vals, c_vals, j0 * n, *key.sigma_evals, n, w, betas, gammas, num, den)
+            native.batch_inverse_dev(den, 0, cnt * n)
+            native.vec_op_dev(2, num, 0, num, 0, den, 0, cnt * n)
+            native.scan_many_dev(0, zc, 0, num, 0, n, cnt)  # z_j,0 = 1 in every proof
+        else:                                               # n = 1: z = [1], as in prove
+            native.scalars_upload(zc, 0, native.fr_vec_bytes([1] * cnt), cnt)
+        native.ntt_many_dev(zc, 0, log_n, cnt, w, inverse=True)
+        z = alloc(cnt * (n + 3))
+        native.plonk_blind_many_dev(zc, 0, n, n, cnt, [b[6:9] for b in bl], z, 0, n + 3)
+        for prf, tr, pt in zip(proofs, trs, native.msm_dev_many(key.srs_table, 0, n + 3, cnt, z)):
+            prf.z_comm = g1_from_ints(pt)
+            tr.append_point(b"z_comm", prf.z_comm)
+        # ---- round 3: 4 cnt coset transforms, the quotient with per-proof challenges, cnt inverse transforms
+        alphas = [int(tr.challenge_scalar(b"alpha")) for tr in trs]
+        ext = alloc(4 * cnt * N)
+        native.plonk_coset_inputs_many_dev(wires, z, n, cnt, key.log_n + key.log_ext, ext)
+        native.ntt_many_dev(ext, 0, log_n + key.log_ext, 4 * cnt, key.omega8, coset_shift=COSET_SHIFT)
+        t = alloc(cnt * N)
+        native.plonk_quotient_many_dev(ext, [key.coset[k] for k in CIRCUIT_POLYS], n, key.ext, key.x, key.l1f, key.zh8,
+                                       betas, gammas, alphas, t)
+        native.ntt_many_dev(t, 0, log_n + key.log_ext, cnt, key.omega8, inverse=True, coset_shift=COSET_SHIFT)
+        bad = native.plonk_divisible_many_dev(t, n, key.ext, cnt)
+        if bad is not None:
+            raise ValueError(_NOT_DIVISIBLE + " (proof %d of the batch)" % (j0 + bad))
+        ts = alloc(3 * cnt * (n + 6))                       # t_lo | t_mid | t_hi, vector part * cnt + j
+        native.plonk_split_t_many_dev(t, n, key.ext, cnt, ts)
+        pts = native.msm_dev_many(key.srs_table, 0, n + 6, 3 * cnt, ts)
+        for j, (prf, tr) in enumerate(zip(proofs, trs)):
+            for i, part in enumerate(("t_lo", "t_mid", "t_hi")):
+                setattr(prf, part + "_comm", g1_from_ints(pts[i * cnt + j]))
+                tr.append_point(part.encode() + b"_comm", getattr(prf, part + "_comm"))
+        # ---- round 4: 6 cnt evaluations in one batched set of Horner launches
+        zetas = [int(tr.challenge_scalar(b"zeta")) for tr in trs]
+        zws = [zeta * w % R for zeta in zetas]
+        wl = cnt * (n + 2)
+        evals = native.fr_poly_eval_many_dev(
+            [(wires, 0, n + 2, n + 2, 0), (wires, wl, n + 2, n + 2, 0), (wires, 2 * wl, n + 2, n + 2, 0),
+             (key.coeffs["s_sigma1"], 0, 0, n, 0), (key.coeffs["s_sigma2"], 0, 0, n, 0), (z, 0, n + 3, n + 3, 1)],
+            cnt, [zetas, zws])
+        names = ("a_eval", "b_eval", "c_eval", "s_sigma1_eval", "s_sigma2_eval", "z_omega_eval")
+        for j, (prf, tr) in enumerate(zip(proofs, trs)):
+            for g, name in enumerate(names):
+                setattr(prf, name, FR(evals[g][j]))
+                tr.append_scalar(name.encode(), evals[g][j])
+        # ---- round 5: linearisation and opening polynomials as batched lincombs, segmented divisions by (x - zeta)
+        vs = [int(tr.challenge_scalar(b"v")) for tr in trs]
+        r_rows, p_rows = [], []
+        for j in range(cnt):
+            beta, gamma, alpha, zeta, v = betas[j], gammas[j], alphas[j], zetas[j], vs[j]
+            a_e, b_e, c_e, s1_e, s2_e, zw_e = (evals[g][j] for g in range(6))
+            zh_zeta = (pow(zeta, n, R) - 1) % R
+            l1_zeta = 1 if zeta == 1 else pow(n, -1, R) * zh_zeta % R * pow((zeta - 1) % R, -1, R) % R
+            perm_z = alpha * (a_e + beta * zeta + gamma) % R * (b_e + beta * K1 * zeta + gamma) % R * (c_e + beta * K2 * zeta + gamma) % R
+            ab = (a_e + beta * s1_e + gamma) * (b_e + beta * s2_e + gamma) % R
+            perm_s3 = alpha * ab % R * beta % R * zw_e % R
+            const = (-alpha * ab % R * zw_e % R * (c_e + gamma) - alpha * alpha % R * l1_zeta) % R
+            r_rows.append([a_e * b_e % R, a_e, b_e, c_e, 1, (-perm_s3) % R, (perm_z + alpha * alpha % R * l1_zeta) % R, const])
+            zeta_n = pow(zeta, n, R)
+            p_rows.append([1, zeta_n, zeta_n * zeta_n % R, v] + [pow(v, e, R) for e in range(2, 7)] + [0])
+        r = alloc(cnt * (n + 3))
+        native.lincomb_many_dev(r, 0, n + 3, n + 3, cnt,
+                                [(key.coeffs[k], 0, 0, n) for k in ("q_m", "q_l", "q_r", "q_o", "q_c", "s_sigma3")]
+                                + [(z, 0, n + 3, n + 3)], r_rows)
+        r_evals = native.fr_poly_eval_many_dev([(r, 0, n + 3, n + 3, 0)], cnt, [zetas])[0]
+        tl = cnt * (n + 6)
+        P = alloc(cnt * (n + 6))
+        native.lincomb_many_dev(P, 0, n + 6, n + 6, cnt,
+                                [(ts, 0, n + 6, n), (ts, tl, n + 6, n), (ts, 2 * tl, n + 6, n + 6), (r, 0, n + 3, n + 3),
+                                 (wires, 0, n + 2, n + 2), (wires, wl, n + 2, n + 2), (wires, 2 * wl, n + 2, n + 2),
+                                 (key.coeffs["s_sigma1"], 0, 0, n), (key.coeffs["s_sigma2"], 0, 0, n)], p_rows)
+        # W_j (n + 5) and Ww_j (n + 2, zero-padded to n + 5: a zero scalar adds nothing) in one many-MSM
+        Wb = alloc(2 * cnt * (n + 5))
+        native.div_linear_many_dev(P, 0, n + 6, n + 6, zetas, Wb, 0, n + 5)
+        native.div_linear_many_dev(z, 0, n + 3, n + 3, zws, Wb, cnt * (n + 5), n + 5)
+        pts = native.msm_dev_many(key.srs_table, 0, n + 5, 2 * cnt, Wb)
+        for j, prf in enumerate(proofs):
+            prf.r_eval = FR(r_evals[j])
+            prf.W_zeta_comm, prf.W_zeta_omega_comm = g1_from_ints(pts[j]), g1_from_ints(pts[cnt + j])
+        return proofs
+    finally:
+        for h in tmp:
+            h.free()
