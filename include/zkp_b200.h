@@ -380,6 +380,24 @@ int zkp_fr_ap_interpolate_many_dev(uint64_t values, uint64_t off, uint64_t k, ui
 int zkp_fr_ap_vanishing_dev(uint64_t k, uint64_t out, uint64_t out_off);
 int zkp_fr_ap_lagrange_dev(uint64_t k, const uint8_t x[32], uint64_t out, uint64_t out_off);
 
+/* ---- witness solving: count witnesses of one circuit per call (zkp/witness.py, csrc/witness.cuh) ---------------
+ * Replaces the host witness computation of the reference (zkp/groth16/code_to_r1cs.py variable assignment,
+ * zkp/plonk/circuit.py wire values).  A program has `vars` variables (v_0 = 1, in_var[n_in] from the caller) and
+ * `steps` steps sorted by level (level_ptr[levels + 1]); step s has four linear forms, rows 4s..4s+3 of a CSR matrix
+ * over the variables (row_ptr[4 steps + 1], col_idx[nnz], values nnz x 32 B canonical): alpha, beta, gamma, delta.
+ * N = (alpha.v)(beta.v) + gamma.v, D = delta.v.  out_var[s] = 0xFFFFFFFF: a check step (N must be 0); otherwise
+ * v[out_var[s]] = N / D (delta = 1 v_0: no inversion).  Load checks that every variable other than v_0 and the inputs
+ * is written by exactly one step and that each step reads only variables of lower levels.
+ * zkp_witness_solve_many_dev: witness j reads its n_in inputs at in_off + j*n_in and writes its `vars` canonical
+ * values at out_off + j*vars.  *first_bad = lowest j*steps + s whose step failed (D = 0, or N != 0 in a check), or
+ * UINT64_MAX.  One launch whatever count and depth are; count = 0 launches nothing.  Ranges are checked before any
+ * launch (ZKP_ERR_INVALID_ARGUMENT). */
+int zkp_witness_program_load(const uint32_t* row_ptr, const uint32_t* col_idx, const uint8_t* values, uint64_t nnz,
+                             const uint32_t* out_var, uint64_t steps, const uint32_t* level_ptr, uint64_t levels,
+                             const uint32_t* in_var, uint64_t n_in, uint64_t vars, uint64_t* handle);
+int zkp_witness_solve_many_dev(uint64_t program, uint64_t inputs, uint64_t in_off, uint32_t count, uint64_t out,
+                               uint64_t out_off, uint64_t* first_bad);
+
 /* ---- pairings (verifier side) -------------------------------------------------------------------
  * The BN254 optimal-Ate pairing of py_ecc's bn128.pairing(Q, P), Q in G2, P in G1, in the encodings above
  * (csrc/pairing.cu).  Replaces the pairings of zkp/groth16/verifying.py:29-40 (e(A, B) == e(alpha, beta)

@@ -139,6 +139,8 @@ PROTOTYPES = {
     "zkp_fr_ap_interpolate_many_dev": (c_int, [u64, u64, u64, u32, vp, u64, u64]),
     "zkp_fr_ap_vanishing_dev": (c_int, [u64, u64, u64]),
     "zkp_fr_ap_lagrange_dev": (c_int, [u64, vp, u64, u64]),
+    "zkp_witness_program_load": (c_int, [vp, vp, vp, u64, vp, u64, vp, u64, vp, u64, u64, u64p]),
+    "zkp_witness_solve_many_dev": (c_int, [u64, u64, u64, u32, u64, u64, u64p]),
     "zkp_fr_poly_mul": (c_int, [vp, u64, vp, u64, vp]),
     "zkp_fr_poly_divmod": (c_int, [vp, u64, vp, u64, vp, vp]),
     "zkp_msm_profile": (c_int, [c_int]),

@@ -1387,3 +1387,4 @@ int zkp_groth16_quotient(const uint8_t* a, const uint8_t* b, const uint8_t* cc, 
 #include "qap.cuh"
 #include "groth16_batch.cuh"
 #include "plonk_batch.cuh"
+#include "witness.cuh"

@@ -265,6 +265,33 @@ static int ap_interpolate(Context& c, const Fr* y, uint64_t k, const Fr* scale_m
   return launches;
 }
 
+// Checks a host CSR matrix and uploads it into r: buf = values (Montgomery), aux[0] = row_ptr, aux[1] = columns.
+static void sparse_upload(Context& c, Resource& r, const uint32_t* row_ptr, const uint32_t* col_idx, const uint8_t* values,
+                          uint64_t rows, uint64_t cols, uint64_t nnz, const char* what) {
+  if (!row_ptr || (nnz && (!col_idx || !values))) throw InvalidArgument(std::string(what) + ": null argument");
+  if (rows >= (uint64_t(1) << 31) || cols >= (uint64_t(1) << 32) || nnz >= (uint64_t(1) << 32))
+    throw InvalidArgument(std::string(what) + ": dimensions exceed 32-bit indices");
+  if (row_ptr[0] != 0 || row_ptr[rows] != nnz) throw InvalidArgument(std::string(what) + ": row_ptr must run from 0 to nnz");
+  for (uint64_t i = 0; i < rows; i++)
+    if (row_ptr[i] > row_ptr[i + 1]) throw InvalidArgument(std::string(what) + ": row_ptr is not monotone");
+  for (uint64_t e = 0; e < nnz; e++)
+    if (col_idx[e] >= cols) throw InvalidArgument(std::string(what) + ": column index out of range");
+  r.n = rows;
+  r.cols = cols;
+  r.nnz = nnz;
+  r.buf.reserve_pooled((nnz ? nnz : 1) * sizeof(Fr));
+  r.aux[0].reserve_pooled((rows + 1) * 4);
+  r.aux[1].reserve_pooled((nnz ? nnz : 1) * 4);
+  CUDA_CHECK(cudaMemcpyAsync(r.aux[0].p, row_ptr, (rows + 1) * 4, cudaMemcpyHostToDevice, c.stream));
+  if (nnz) {
+    CUDA_CHECK(cudaMemcpyAsync(r.aux[1].p, col_idx, nnz * 4, cudaMemcpyHostToDevice, c.stream));
+    CUDA_CHECK(cudaMemcpyAsync(r.buf.p, values, nnz * 32, cudaMemcpyHostToDevice, c.stream));
+    fr_to_mont_kernel<<<GRID_1D(nnz)>>>(r.buf.as<Fr>(), nnz, r.buf.as<Fr>());
+    CUDA_CHECK_LAUNCH();
+    c.launches++;
+  }
+}
+
 }  // namespace zkp
 
 using namespace zkp;
@@ -274,30 +301,10 @@ extern "C" {
 int zkp_sparse_load(const uint32_t* row_ptr, const uint32_t* col_idx, const uint8_t* values, uint64_t rows, uint64_t cols,
                     uint64_t nnz, uint64_t* handle) {
   return guarded([&](Context& c) {
-    if (!handle || !row_ptr || (nnz && (!col_idx || !values))) throw InvalidArgument("zkp_sparse_load: null argument");
-    if (rows >= (uint64_t(1) << 31) || cols >= (uint64_t(1) << 32) || nnz >= (uint64_t(1) << 32))
-      throw InvalidArgument("zkp_sparse_load: dimensions exceed 32-bit indices");
-    if (row_ptr[0] != 0 || row_ptr[rows] != nnz) throw InvalidArgument("zkp_sparse_load: row_ptr must run from 0 to nnz");
-    for (uint64_t r = 0; r < rows; r++)
-      if (row_ptr[r] > row_ptr[r + 1]) throw InvalidArgument("zkp_sparse_load: row_ptr is not monotone");
-    for (uint64_t e = 0; e < nnz; e++)
-      if (col_idx[e] >= cols) throw InvalidArgument("zkp_sparse_load: column index out of range");
+    if (!handle) throw InvalidArgument("zkp_sparse_load: null argument");
     auto r = std::make_unique<Resource>();
     r->kind = HandleKind::Sparse;
-    r->n = rows;
-    r->cols = cols;
-    r->nnz = nnz;
-    r->buf.reserve_pooled((nnz ? nnz : 1) * sizeof(Fr));
-    r->aux[0].reserve_pooled((rows + 1) * 4);
-    r->aux[1].reserve_pooled((nnz ? nnz : 1) * 4);
-    CUDA_CHECK(cudaMemcpyAsync(r->aux[0].p, row_ptr, (rows + 1) * 4, cudaMemcpyHostToDevice, c.stream));
-    if (nnz) {
-      CUDA_CHECK(cudaMemcpyAsync(r->aux[1].p, col_idx, nnz * 4, cudaMemcpyHostToDevice, c.stream));
-      CUDA_CHECK(cudaMemcpyAsync(r->buf.p, values, nnz * 32, cudaMemcpyHostToDevice, c.stream));
-      fr_to_mont_kernel<<<GRID_1D(nnz)>>>(r->buf.as<Fr>(), nnz, r->buf.as<Fr>());
-      CUDA_CHECK_LAUNCH();
-      c.launches++;
-    }
+    sparse_upload(c, *r, row_ptr, col_idx, values, rows, cols, nnz, "zkp_sparse_load");
     CUDA_CHECK(cudaStreamSynchronize(c.stream));
     *handle = registry().put(std::move(r));
   });

@@ -9,7 +9,7 @@
 
 namespace zkp {
 
-enum class HandleKind : int { G1Table = 1, G2Table = 2, Scalars = 3, Sparse = 4 };
+enum class HandleKind : int { G1Table = 1, G2Table = 2, Scalars = 3, Sparse = 4, WitnessProgram = 5 };
 
 struct Resource {
   HandleKind kind;
@@ -18,7 +18,10 @@ struct Resource {
   DevBuf buf;
   // sparse matrices (CSR): n rows; buf = values (Montgomery), aux[0] = row_ptr, aux[1] = column indices
   uint64_t cols = 0, nnz = 0;
-  DevBuf aux[2];
+  DevBuf aux[3];
+  // witness programs (csrc/witness.cuh): the four forms of every step as one CSR of 4 * steps rows over `cols`
+  // variables in buf / aux[0] / aux[1]; aux[2] = out_var[steps] | level_ptr[levels + 1] | in_var[inputs]
+  uint64_t steps = 0, levels = 0, inputs = 0;
   Resource() = default;
   Resource(const Resource&) = delete;
   Resource& operator=(const Resource&) = delete;
@@ -26,8 +29,7 @@ struct Resource {
   // buffers back to the pool (recycle() is a no-op on an empty buffer)
   ~Resource() {
     buf.recycle();
-    aux[0].recycle();
-    aux[1].recycle();
+    for (DevBuf& b : aux) b.recycle();
   }
 };
 

@@ -871,3 +871,34 @@ def fr_ap_lagrange_dev(k, x):
     out = scalars_alloc(k)
     check(_lib.lib().zkp_fr_ap_lagrange_dev(k, buf(fe_bytes(x)), out.handle, 0))
     return out
+
+
+# ------------------------------------------------------------------ witness solving (zkp/witness.py)
+def witness_program_load(row_ptr, col_idx, values, out_var, level_ptr, in_var, nvars):
+    """Step program (include/zkp_b200.h zkp_witness_program_load) -> device handle.  row_ptr: 4 * steps + 1 offsets;
+    col_idx / values: the entries of the four forms of every step; out_var: steps entries (0xFFFFFFFF = check)."""
+    import numpy as np
+    arr = lambda a: np.ascontiguousarray(a, dtype=np.uint32)
+    rp, ci, ov, lp, iv = arr(row_ptr), arr(col_idx), arr(out_var), arr(level_ptr), arr(in_var)
+    steps, nnz = len(ov), len(ci)
+    if len(rp) != 4 * steps + 1 or len(lp) < 1:
+        raise ValueError("witness_program_load: row_ptr needs 4 * steps + 1 entries and level_ptr at least one")
+    vb = values if isinstance(values, (bytes, bytearray)) else fr_vec_bytes(values)
+    if len(vb) != 32 * nnz:
+        raise ValueError("witness_program_load: one value per column index")
+    ptr = lambda a: a.ctypes.data if len(a) else None
+    h = ctypes.c_uint64()
+    check(_lib.lib().zkp_witness_program_load(rp.ctypes.data, ptr(ci), buf(vb) if nnz else None, nnz, ptr(ov), steps,
+                                              lp.ctypes.data, len(lp) - 1, ptr(iv), len(iv), nvars, ctypes.byref(h)))
+    out = DeviceHandle(h.value, nvars, "witness_program")
+    out.steps, out.inputs = steps, len(iv)
+    return out
+
+
+def witness_solve_many_dev(program, inputs, count, out, in_off=0, out_off=0):
+    """Solve count witnesses: inputs j at in_off + j * n_in, values j at out_off + j * nvars.  Returns the lowest
+    j * steps + s whose step failed, or None."""
+    bad = ctypes.c_uint64()
+    check(_lib.lib().zkp_witness_solve_many_dev(program.handle, inputs.handle, in_off, count, out.handle, out_off,
+                                                ctypes.byref(bad)))
+    return _first_bad(bad.value)
