@@ -323,7 +323,18 @@ int zkp_plonk_quotient_dev(const uint64_t evals[12], uint64_t n, uint32_t ext, u
  * zkp_fr_lincomb_many_dev: dst_j[i] = sum_k coeffs[j][k] src_k,j[i] + (i == 0 ? coeffs[j][K] : 0), i < n, sources
  *   shared or per proof as above, coeffs count x (K + 1) (round5.py:90-160); dst must not overlap a source.
  * zkp_fr_div_linear_many_dev: zkp_fr_div_linear_dev per proof (round5.py:165-171, kzg.py:95-104), p_j at
- *   src_off + j * src_stride (len coefficients), quotient j at dst_off + j * dst_stride; zeta_j = 0 is a shift. */
+ *   src_off + j * src_stride (len coefficients), quotient j at dst_off + j * dst_stride; zeta_j = 0 is a shift.
+ * Public inputs: proof j has ell <= n public inputs x_j,0..ell-1 at off + j * stride of the scalar handle pub, and
+ * PI_j(X) = sum_i x_j,i L_i(X) (utils.py:84-116 public_input_polynomial) enters the gate identity with a plus sign
+ * (round3.py:33).  ell = 0 leaves every result as without public inputs.
+ * zkp_plonk_pi_scatter_many_dev: count blocks of n evaluations at dst_off: x_j,i at row i < ell, zero elsewhere.
+ * zkp_plonk_coset_inputs_pi_many_dev: zkp_plonk_coset_inputs_many_dev plus a fifth group of count blocks: the PI_j
+ *   coefficients (count blocks of n at pi_off), zero-padded to 2^log_N, Montgomery; 5 * count * 2^log_N < 2^32.
+ * zkp_plonk_quotient_pi_many_dev: zkp_plonk_quotient_many_dev on 5 count blocks, the fifth PI_j on the coset, added
+ *   to q_c in the gate term (round3.py:33, 114-147).
+ * zkp_plonk_pi_eval_many_dev: out_j = PI_j(zeta_j) = sum_{i < ell} x_j,i w^i (zeta_j^n - 1) / (n (zeta_j - w^i))
+ *   (utils.py:25-81 lagrange_basis_eval, public_input_poly_eval; round5.py:20,30; verifier.py:99), x_j,i when
+ *   zeta_j = w^i with i < ell, 0 when i >= ell; the inversions are one batch in which a zero gap stays zero. */
 int zkp_fr_ntt_many_dev(uint64_t scalars, uint64_t offset, uint32_t log_n, const uint8_t omega[32], int inverse,
                         const uint8_t* coset_shift, uint32_t count);
 int zkp_plonk_blind_many_dev(uint64_t src, uint64_t src_off, uint64_t src_stride, uint64_t n, uint32_t nvec,
@@ -347,6 +358,15 @@ int zkp_fr_lincomb_many_dev(uint64_t dst, uint64_t dst_off, uint64_t dst_stride,
                             const uint8_t* coeffs);
 int zkp_fr_div_linear_many_dev(uint64_t src, uint64_t src_off, uint64_t src_stride, uint64_t len, uint32_t count,
                                const uint8_t* zetas, uint64_t dst, uint64_t dst_off, uint64_t dst_stride);
+int zkp_plonk_pi_scatter_many_dev(uint64_t pub, uint64_t off, uint64_t stride, uint64_t ell, uint64_t n, uint32_t count,
+                                  uint64_t dst, uint64_t dst_off);
+int zkp_plonk_coset_inputs_pi_many_dev(uint64_t wires, uint64_t z, uint64_t pi, uint64_t pi_off, uint64_t n, uint32_t count,
+                                       uint32_t log_N, uint64_t out);
+int zkp_plonk_quotient_pi_many_dev(uint64_t evals, const uint64_t circuit[8], uint64_t n, uint32_t ext, uint32_t count,
+                                   uint64_t x, uint64_t l1f, uint64_t zh8, const uint8_t* betas, const uint8_t* gammas,
+                                   const uint8_t* alphas, uint64_t t_out);
+int zkp_plonk_pi_eval_many_dev(uint64_t pub, uint64_t off, uint64_t stride, uint64_t ell, uint64_t n, uint32_t count,
+                               const uint8_t omega[32], const uint8_t* zetas, uint8_t* out);
 /* General product and exact/long division over Fr in coefficient form
  * (Polynomial.__mul__ polynomial.py:144-159; poly_div polynomial.py:385-435). */
 int zkp_fr_poly_mul(const uint8_t* a, uint64_t a_len, const uint8_t* b, uint64_t b_len, uint8_t* out);

@@ -25,20 +25,76 @@ __global__ void plonk_blind_many_kernel(const Fr* __restrict__ in, uint64_t in_s
 }
 
 // The round-3 transform inputs of every proof: vector v < 3 count is wire v (n + 2 coefficients at stride n + 2),
-// vector 3 count + j is z_j (n + 3 at stride n + 3); each lands zero-padded and in Montgomery form in its own block
-// of 2^log_N elements.
-__global__ void plonk_coset_inputs_many_kernel(const Fr* __restrict__ wires, const Fr* __restrict__ z, uint64_t n,
-                                               uint64_t count, uint32_t log_N, uint64_t total, Fr* __restrict__ out) {
+// vector 3 count + j is z_j (n + 3 at stride n + 3), vector 4 count + j (when total covers it) is PI_j (n at stride
+// n); each lands zero-padded and in Montgomery form in its own block of 2^log_N elements.
+__global__ void plonk_coset_inputs_many_kernel(const Fr* __restrict__ wires, const Fr* __restrict__ z,
+                                               const Fr* __restrict__ pi, uint64_t n, uint64_t count, uint32_t log_N,
+                                               uint64_t total, Fr* __restrict__ out) {
   uint64_t idx = IDX64;
   if (idx >= total) return;
   const uint64_t v = idx >> log_N, i = idx & ((uint64_t(1) << log_N) - 1);
   Fr x = Fr::zero();
   if (v < 3 * count) {
     if (i < n + 2) x = wires[v * (n + 2) + i].to_mont();
-  } else if (i < n + 3) {
-    x = z[(v - 3 * count) * (n + 3) + i].to_mont();
+  } else if (v < 4 * count) {
+    if (i < n + 3) x = z[(v - 3 * count) * (n + 3) + i].to_mont();
+  } else if (i < n) {
+    x = pi[(v - 4 * count) * n + i].to_mont();
   }
   out[idx] = x;
+}
+
+// ------------------------------------------------------------------ public inputs
+// out[j * n + i] = i < ell ? pub[j * stride + i] : 0: the evaluations of PI_j on H (utils.py:84-116), canonical
+__global__ void plonk_pi_scatter_many_kernel(const Fr* __restrict__ pub, uint64_t stride, uint64_t ell, uint32_t log_n,
+                                             uint64_t total, Fr* __restrict__ out) {
+  uint64_t idx = IDX64;
+  if (idx >= total) return;
+  const uint64_t j = idx >> log_n, i = idx & ((uint64_t(1) << log_n) - 1);
+  out[idx] = i < ell ? pub[j * stride + i] : Fr::zero();
+}
+
+// gap[j * ell + i] = n (zeta_j - w^i), Montgomery: the denominator of L_i(zeta_j), zero when zeta_j = w^i
+__global__ void plonk_pi_gap_many_kernel(const Fr* __restrict__ zetas, const Fr* __restrict__ omega_tab, uint64_t ell,
+                                         uint64_t n, uint64_t total, Fr* __restrict__ gap) {
+  uint64_t idx = IDX64;
+  if (idx >= total) return;
+  const uint64_t j = idx / ell, i = idx % ell;
+  Fr nc = Fr::zero();
+  nc.v[0] = (uint32_t)n;  // n <= 2^28
+  gap[idx] = (zetas[j].to_mont() - power_at(omega_tab, (uint32_t)i)) * nc.to_mont();
+}
+
+// one block per proof: out_j = sum_{i < ell} x_j,i w^i (zeta_j^n - 1) / (n (zeta_j - w^i)) from the inverted gaps;
+// a zero inverse marks zeta_j = w^i (at most one i per proof), and then out_j = x_j,i (utils.py lagrange_basis_eval)
+__global__ void __launch_bounds__(DOT_THREADS) plonk_pi_eval_many_kernel(const Fr* __restrict__ pub, uint64_t stride,
+                                                                          uint64_t ell, uint32_t log_n,
+                                                                          const Fr* __restrict__ zetas,
+                                                                          const Fr* __restrict__ omega_tab,
+                                                                          const Fr* __restrict__ inv, Fr* __restrict__ out) {
+  __shared__ Fr sm[DOT_THREADS];
+  __shared__ uint64_t hit;
+  const uint64_t j = blockIdx.x;
+  if (threadIdx.x == 0) hit = ~uint64_t(0);
+  __syncthreads();
+  const Fr* x = pub + j * stride;
+  const Fr* iv = inv + j * ell;
+  Fr acc = Fr::zero();
+  for (uint64_t i = threadIdx.x; i < ell; i += DOT_THREADS) {
+    const Fr d = iv[i];
+    if (d.is_zero()) hit = i;
+    else acc = acc + x[i] * (power_at(omega_tab, (uint32_t)i) * d);  // canonical * Montgomery -> canonical
+  }
+  const Fr tot = dot_block_reduce(acc, sm);  // ends with a barrier: `hit` is visible
+  if (threadIdx.x == 0) {
+    if (hit != ~uint64_t(0)) {
+      out[j] = x[hit];
+    } else {
+      Fr zn = zetas[j].to_mont();
+      for (uint32_t k = 0; k < log_n; k++) zn = zn.sqr();
+      out[j] = tot * (zn - Fr::one());
+    }
+  }
 }
 
 // plonk_perm_terms_kernel for proof j = idx >> log_n with its own beta_j, gamma_j (canonical arrays); the witness of
@@ -209,11 +265,14 @@ struct PlonkQuotManyArgs {
   const Fr *ql, *qr, *qo, *qm, *qc, *s1, *s2, *s3;  // shared circuit coset evaluations, Montgomery
   const Fr *x, *l1f, *zh_inv;                       // static coset data of the device key
   const Fr *betas, *gammas, *alphas;                // count canonical challenges each
+  const Fr* pi;  // with public inputs: count blocks of N, the Montgomery coset evaluations of PI_j (round3.py:33)
   uint64_t count;
   uint32_t log_N, ext;
   Fr* t;  // out: count blocks of N quotient evaluations, Montgomery
 };
-// plonk_quotient_kernel for proof j = idx >> log_N with its own challenges; z(w x) wraps inside proof j's block
+// plonk_quotient_kernel for proof j = idx >> log_N with its own challenges; z(w x) wraps inside proof j's block.
+// PI: q_c + PI_j in the gate term (a separate instantiation, so the kernel without public inputs is unchanged)
+template <bool PI>
 __global__ void __launch_bounds__(128) plonk_quotient_many_kernel(PlonkQuotManyArgs q) {
   uint64_t idx = IDX64;
   const uint64_t N = uint64_t(1) << q.log_N;
@@ -225,7 +284,9 @@ __global__ void __launch_bounds__(128) plonk_quotient_many_kernel(PlonkQuotManyA
   const Fr* zj = q.ev + 3 * blk + (j << q.log_N);
   Fr z = zj[i];
   Fr zw = zj[(i + q.ext) & (N - 1)];
-  Fr gate = q.ql[i] * a + q.qr[i] * b + q.qo[i] * c + q.qm[i] * (a * b) + q.qc[i];
+  Fr qc = q.qc[i];
+  if (PI) qc = qc + q.pi[idx];
+  Fr gate = q.ql[i] * a + q.qr[i] * b + q.qo[i] * c + q.qm[i] * (a * b) + qc;
   Fr bx = beta * q.x[i];
   Fr ag = a + gamma, bg = b + gamma, cg = c + gamma;
   Fr num = (ag + bx) * (bg + bx.dbl()) * (cg + bx.dbl() + bx) * z;
@@ -365,6 +426,68 @@ static Fr* upload_canon(Context& c, const uint8_t* host, uint64_t n) {
   return d;
 }
 
+static void pi_check_shape(const char* what, uint64_t n, uint64_t ell, uint64_t stride, uint32_t count) {
+  if (!n || (n & (n - 1)) || n > (uint64_t(1) << 28)) throw InvalidArgument(std::string(what) + ": n must be a power of two <= 2^28");
+  if (ell > n) throw InvalidArgument(std::string(what) + ": more public inputs than gates");
+  if (count > 1 && stride < ell) throw InvalidArgument(std::string(what) + ": stride shorter than the public inputs");
+}
+
+// nblk = 4: a_*, b_*, c_*, z_*; nblk = 5: PI_* too, from pi (count blocks of n coefficients at pi_off)
+static void coset_inputs_many(Context& c, const char* what, uint64_t wires, uint64_t z, uint64_t pi, uint64_t pi_off,
+                              uint64_t n, uint32_t count, uint32_t log_N, uint64_t out, uint32_t nblk) {
+  if (log_N > 28 || (uint64_t(1) << log_N) < n + 3) throw InvalidArgument(std::string(what) + ": 2^log_N must hold n + 3 coefficients");
+  if (((uint64_t)nblk * count << log_N) >= (uint64_t(1) << 32))
+    throw InvalidArgument(std::string(what) + ": blocks * count * 2^log_N must be < 2^32");
+  Fr* pw = hptr(wires, 0, 3 * (uint64_t)count * (n + 2), what);
+  Fr* pz = hptr(z, 0, (uint64_t)count * (n + 3), what);
+  Fr* pp = nblk == 5 ? hptr(pi, pi_off, (uint64_t)count * n, what) : nullptr;
+  const uint64_t total = (uint64_t)nblk * count << log_N;
+  Fr* po = hptr(out, 0, total, what);
+  if (!count) return;
+  plonk_coset_inputs_many_kernel<<<GRID_1D(total)>>>(pw, pz, pp, n, count, log_N, total, po);
+  CUDA_CHECK_LAUNCH();
+  c.launches++;
+}
+
+// evals: 4 count blocks of N (a_*, b_*, c_*, z_*), or 5 with PI_* (with_pi)
+static void quotient_many(Context& c, const char* w, uint64_t evals, const uint64_t circuit[8], uint64_t n, uint32_t ext,
+                          uint32_t count, uint64_t x, uint64_t l1f, uint64_t zh8, const uint8_t* betas,
+                          const uint8_t* gammas, const uint8_t* alphas, uint64_t t_out, bool with_pi) {
+  if (!circuit || (count && (!betas || !gammas || !alphas))) throw InvalidArgument(std::string(w) + ": null argument");
+  if (ext != 4 && ext != 8 && ext != 16) throw InvalidArgument(std::string(w) + ": ext must be 4, 8 or 16");
+  const uint64_t N = (uint64_t)ext * n;
+  if (!n || (N & (N - 1)) || N > (uint64_t(1) << 28)) throw InvalidArgument(std::string(w) + ": n must be a power of two");
+  if (N < 3 * n + 6) throw InvalidArgument(std::string(w) + ": coset too small for the quotient degree");
+  const uint64_t nblk = with_pi ? 5 : 4;
+  if (nblk * count * N >= (uint64_t(1) << 32)) throw InvalidArgument(std::string(w) + ": blocks * count * N must be < 2^32");
+  PlonkQuotManyArgs q;
+  q.ev = hptr(evals, 0, nblk * count * N, w);
+  q.pi = q.ev + 4 * (uint64_t)count * N;
+  const Fr** slots[8] = {&q.ql, &q.qr, &q.qo, &q.qm, &q.qc, &q.s1, &q.s2, &q.s3};
+  for (int k = 0; k < 8; k++) *slots[k] = hptr(circuit[k], 0, N, w);
+  q.x = hptr(x, 0, N, w);
+  q.l1f = hptr(l1f, 0, N, w);
+  q.zh_inv = hptr(zh8, 0, ext, w);
+  q.t = hptr(t_out, 0, (uint64_t)count * N, w);
+  q.count = count;
+  q.log_N = log2_ceil(N);
+  q.ext = ext;
+  if (!count) return;
+  ArenaScope scope;
+  Fr* ch = g_arena.alloc(3 * (uint64_t)count);
+  CUDA_CHECK(cudaMemcpyAsync(ch, betas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
+  CUDA_CHECK(cudaMemcpyAsync(ch + count, gammas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
+  CUDA_CHECK(cudaMemcpyAsync(ch + 2 * count, alphas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
+  q.betas = ch;
+  q.gammas = ch + count;
+  q.alphas = ch + 2 * count;
+  if (with_pi) plonk_quotient_many_kernel<true><<<ceil_div((uint64_t)count * N, 128), 128, 0, c.stream>>>(q);
+  else plonk_quotient_many_kernel<false><<<ceil_div((uint64_t)count * N, 128), 128, 0, c.stream>>>(q);
+  CUDA_CHECK_LAUNCH();
+  c.launches++;
+  CUDA_CHECK(cudaStreamSynchronize(c.stream));
+}
+
 }  // namespace zkp
 
 using namespace zkp;
@@ -458,17 +581,14 @@ int zkp_fr_scan_many_dev(int op, uint64_t dst, uint64_t dst_off, uint64_t src, u
 
 int zkp_plonk_coset_inputs_many_dev(uint64_t wires, uint64_t z, uint64_t n, uint32_t count, uint32_t log_N, uint64_t out) {
   return guarded([&](Context& c) {
-    const char* what = "zkp_plonk_coset_inputs_many_dev";
-    if (log_N > 28 || (uint64_t(1) << log_N) < n + 3) throw InvalidArgument(std::string(what) + ": 2^log_N must hold n + 3 coefficients");
-    if ((4 * (uint64_t)count << log_N) >= (uint64_t(1) << 32)) throw InvalidArgument(std::string(what) + ": 4 * count * 2^log_N must be < 2^32");
-    Fr* pw = hptr(wires, 0, 3 * (uint64_t)count * (n + 2), what);
-    Fr* pz = hptr(z, 0, (uint64_t)count * (n + 3), what);
-    const uint64_t total = 4 * (uint64_t)count << log_N;
-    Fr* po = hptr(out, 0, total, what);
-    if (!count) return;
-    plonk_coset_inputs_many_kernel<<<GRID_1D(total)>>>(pw, pz, n, count, log_N, total, po);
-    CUDA_CHECK_LAUNCH();
-    c.launches++;
+    coset_inputs_many(c, "zkp_plonk_coset_inputs_many_dev", wires, z, 0, 0, n, count, log_N, out, 4);
+  });
+}
+
+int zkp_plonk_coset_inputs_pi_many_dev(uint64_t wires, uint64_t z, uint64_t pi, uint64_t pi_off, uint64_t n, uint32_t count,
+                                       uint32_t log_N, uint64_t out) {
+  return guarded([&](Context& c) {
+    coset_inputs_many(c, "zkp_plonk_coset_inputs_pi_many_dev", wires, z, pi, pi_off, n, count, log_N, out, 5);
   });
 }
 
@@ -476,37 +596,73 @@ int zkp_plonk_quotient_many_dev(uint64_t evals, const uint64_t circuit[8], uint6
                                 uint64_t x, uint64_t l1f, uint64_t zh8, const uint8_t* betas, const uint8_t* gammas,
                                 const uint8_t* alphas, uint64_t t_out) {
   return guarded([&](Context& c) {
-    const char* w = "zkp_plonk_quotient_many_dev";
-    if (!circuit || (count && (!betas || !gammas || !alphas))) throw InvalidArgument(std::string(w) + ": null argument");
-    if (ext != 4 && ext != 8 && ext != 16) throw InvalidArgument(std::string(w) + ": ext must be 4, 8 or 16");
-    const uint64_t N = (uint64_t)ext * n;
-    if (!n || (N & (N - 1)) || N > (uint64_t(1) << 28)) throw InvalidArgument(std::string(w) + ": n must be a power of two");
-    if (N < 3 * n + 6) throw InvalidArgument(std::string(w) + ": coset too small for the quotient degree");
-    if (4 * (uint64_t)count * N >= (uint64_t(1) << 32)) throw InvalidArgument(std::string(w) + ": 4 * count * N must be < 2^32");
-    PlonkQuotManyArgs q;
-    q.ev = hptr(evals, 0, 4 * (uint64_t)count * N, w);
-    const Fr** slots[8] = {&q.ql, &q.qr, &q.qo, &q.qm, &q.qc, &q.s1, &q.s2, &q.s3};
-    for (int k = 0; k < 8; k++) *slots[k] = hptr(circuit[k], 0, N, w);
-    q.x = hptr(x, 0, N, w);
-    q.l1f = hptr(l1f, 0, N, w);
-    q.zh_inv = hptr(zh8, 0, ext, w);
-    q.t = hptr(t_out, 0, (uint64_t)count * N, w);
-    q.count = count;
-    q.log_N = log2_ceil(N);
-    q.ext = ext;
+    quotient_many(c, "zkp_plonk_quotient_many_dev", evals, circuit, n, ext, count, x, l1f, zh8, betas, gammas, alphas,
+                  t_out, false);
+  });
+}
+
+int zkp_plonk_quotient_pi_many_dev(uint64_t evals, const uint64_t circuit[8], uint64_t n, uint32_t ext, uint32_t count,
+                                   uint64_t x, uint64_t l1f, uint64_t zh8, const uint8_t* betas, const uint8_t* gammas,
+                                   const uint8_t* alphas, uint64_t t_out) {
+  return guarded([&](Context& c) {
+    quotient_many(c, "zkp_plonk_quotient_pi_many_dev", evals, circuit, n, ext, count, x, l1f, zh8, betas, gammas, alphas,
+                  t_out, true);
+  });
+}
+
+int zkp_plonk_pi_scatter_many_dev(uint64_t pub, uint64_t off, uint64_t stride, uint64_t ell, uint64_t n, uint32_t count,
+                                  uint64_t dst, uint64_t dst_off) {
+  return guarded([&](Context& c) {
+    const char* what = "zkp_plonk_pi_scatter_many_dev";
+    pi_check_shape(what, n, ell, stride, count);
+    const uint64_t total = (uint64_t)count * n;
+    Fr* d = hptr(dst, dst_off, total, what);
     if (!count) return;
-    ArenaScope scope;
-    Fr* ch = g_arena.alloc(3 * (uint64_t)count);
-    CUDA_CHECK(cudaMemcpyAsync(ch, betas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
-    CUDA_CHECK(cudaMemcpyAsync(ch + count, gammas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
-    CUDA_CHECK(cudaMemcpyAsync(ch + 2 * count, alphas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
-    q.betas = ch;
-    q.gammas = ch + count;
-    q.alphas = ch + 2 * count;
-    plonk_quotient_many_kernel<<<ceil_div((uint64_t)count * N, 128), 128, 0, c.stream>>>(q);
+    Fr* px = nullptr;
+    if (ell) {
+      const uint64_t span = (uint64_t)(count - 1) * stride + ell;
+      px = hptr(pub, off, span, what);
+      if (px < d + total && d < px + span) throw InvalidArgument(std::string(what) + ": destination overlaps the source");
+    }
+    plonk_pi_scatter_many_kernel<<<GRID_1D(total)>>>(px, stride, ell, log2_ceil(n), total, d);
     CUDA_CHECK_LAUNCH();
     c.launches++;
+  });
+}
+
+int zkp_plonk_pi_eval_many_dev(uint64_t pub, uint64_t off, uint64_t stride, uint64_t ell, uint64_t n, uint32_t count,
+                               const uint8_t omega[32], const uint8_t* zetas, uint8_t* out) {
+  return guarded([&](Context& c) {
+    const char* what = "zkp_plonk_pi_eval_many_dev";
+    if (!omega || (count && (!zetas || !out))) throw InvalidArgument(std::string(what) + ": null argument");
+    pi_check_shape(what, n, ell, stride, count);
+    if (!count) return;
+    if (!ell) {
+      memset(out, 0, (size_t)count * 32);
+      return;
+    }
+    Fr* px = hptr(pub, off, (uint64_t)(count - 1) * stride + ell, what);
+    ArenaScope scope;
+    FrBytes ob;
+    memcpy(ob.b, omega, 32);
+    int launches = 0;
+    const uint32_t log_n = log2_ceil(n);
+    const Fr* tab = power_table(c, ob, false, log_n, &launches);
+    Fr* zs = upload_canon(c, zetas, count);
+    const uint64_t m = (uint64_t)count * ell;
+    Fr* gap = g_arena.alloc(m);
+    Fr* inv = g_arena.alloc(m);
+    Fr* res = g_arena.alloc(count);
+    plonk_pi_gap_many_kernel<<<GRID_1D(m)>>>(zs, tab, ell, n, m, gap);
+    CUDA_CHECK_LAUNCH();
+    const uint64_t T = (m + BATCH_INV_CHUNK - 1) / BATCH_INV_CHUNK;
+    fr_batch_inverse_kernel<<<ceil_div(T, 128), 128, 0, c.stream>>>(gap, m, T, 1, inv);  // zeros stay zero
+    CUDA_CHECK_LAUNCH();
+    plonk_pi_eval_many_kernel<<<count, DOT_THREADS, 0, c.stream>>>(px, stride, ell, log_n, zs, tab, inv, res);
+    CUDA_CHECK_LAUNCH();
+    CUDA_CHECK(cudaMemcpyAsync(out, res, (size_t)count * 32, cudaMemcpyDeviceToHost, c.stream));
     CUDA_CHECK(cudaStreamSynchronize(c.stream));
+    c.launches += launches + 3;
   });
 }
 

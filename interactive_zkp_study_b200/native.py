@@ -816,6 +816,41 @@ def div_linear_many_dev(src, src_off, src_stride, length, zetas, dst, dst_off, d
                                                 buf(zs) if zetas else None, dst.handle, dst_off, dst_stride))
 
 
+def plonk_pi_scatter_many_dev(pub, off, stride, ell, n, count, dst, dst_off=0):
+    """count blocks of n values at dst_off: proof j's ell public inputs (pub[off + j * stride ..]) at rows i < ell,
+    zeros elsewhere.  pub may be None when ell = 0."""
+    check(_lib.lib().zkp_plonk_pi_scatter_many_dev(pub.handle if pub is not None else 0, off, stride, ell, n, count,
+                                                   dst.handle, dst_off))
+
+
+def plonk_coset_inputs_pi_many_dev(wires, z, pi, pi_off, n, count, log_N, out):
+    """plonk_coset_inputs_many_dev plus a fifth group: count blocks of n PI coefficients at pi_off."""
+    check(_lib.lib().zkp_plonk_coset_inputs_pi_many_dev(wires.handle, z.handle, pi.handle, pi_off, n, count, log_N,
+                                                        out.handle))
+
+
+def plonk_quotient_pi_many_dev(evals, circuit8, n, ext, x, l1f, zh8, betas, gammas, alphas, t_out):
+    """plonk_quotient_many_dev on 5 groups of blocks: a_*, b_*, c_*, z_*, PI_* (PI_j added to q_c)."""
+    count = len(betas)
+    if len(circuit8) != 8:
+        raise ValueError("plonk_quotient_pi_many_dev: 8 circuit coset evaluations, got %d" % len(circuit8))
+    ch = _fr_rows("plonk_quotient_pi_many_dev: betas, gammas, alphas", [betas, gammas, alphas], 3, count)
+    check(_lib.lib().zkp_plonk_quotient_pi_many_dev(evals.handle, _u64s([h.handle for h in circuit8]), n, ext, count,
+                                                    x.handle, l1f.handle, zh8.handle, buf(ch[:32 * count]),
+                                                    buf(ch[32 * count:64 * count]), buf(ch[64 * count:]), t_out.handle))
+
+
+def plonk_pi_eval_many_dev(pub, off, stride, ell, n, omega, zetas):
+    """[PI_j(zeta_j) for j < len(zetas)]: PI_j = sum_{i < ell} x_j,i L_i over the n-th roots of unity of omega, proof j's
+    inputs at pub[off + j * stride ..].  pub may be None when ell = 0."""
+    count = len(zetas)
+    out = bytearray(32 * max(count, 1))
+    zs = fr_vec_bytes([int(z) % R_MOD for z in zetas])
+    check(_lib.lib().zkp_plonk_pi_eval_many_dev(pub.handle if pub is not None else 0, off, stride, ell, n, count,
+                                                buf(fe_bytes(omega)), buf(zs) if count else None, buf(out)))
+    return fr_vec_from_bytes(bytes(out), count)
+
+
 # ------------------------------------------------------------------ QAP over {1..k} at scale (SURVEY 8 f2)
 def sparse_load(row_ptr, col_idx, values, rows, cols):
     """CSR matrix with Fr values -> device handle.  row_ptr: rows+1 offsets, col_idx: column of each

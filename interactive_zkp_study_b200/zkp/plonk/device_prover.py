@@ -14,8 +14,17 @@ proof elements (bit-identical to the reference-minted golden proofs for equal bl
            "coefficients above 3n+5 vanish", 3 MSMs                                   (round3.py:56-184)
   round 4  6 two-level Horner evaluations                     (round4.py:39-81)
   round 5  linearisation r(x) by axpy, the two openings as (P(x)-P(z))/(x-z) = powers + sum scan, 2 MSMs (round5.py:42-175)
+
+Public inputs (beyond the reference, whose PI is always 0): a key preprocessed with num_public_inputs = l > 0 binds
+each proof to l field elements x_0..x_{l-1}.  Row i < l is public input i's gate, PI(X) = sum_i x_i L_i(X) (the
+reference's utils.public_input_polynomial) enters the gate identity as q_L a + q_R b + q_O c + q_M ab + q_C + PI = 0
+on H, the transcript absorbs append_scalar(b"public_input", x_i) for i = 0..l-1 before the round-1 commitments, the
+quotient's gate term gains PI on the coset and the linearisation constant gains PI(zeta).  l = 0 is exactly the
+protocol above: nothing extra is hashed and every proof is unchanged.
 """
 import secrets
+
+import numpy as np
 
 from ... import native
 from ...compat import curve_order, g1_from_ints
@@ -36,6 +45,7 @@ class DeviceKey:
     def __init__(self):
         self.coeffs, self.coset, self.comm = {}, {}, {}
         self.ranks, self.srs_range = None, None     # sharded SRS: the communicator and this rank's row range
+        self.num_public_inputs = 0
 
 
 def _alloc_from(src, n, total):
@@ -78,14 +88,22 @@ def _commit_many(key, items):
     return native.g1_msm_dev_batch(key.srs_table, [(h, off, 0, length) for h, off, length in items])
 
 
-def preprocess(n, selector_evals, sigma_evals, srs_table, srs_size, comm=None, srs_range=None):
+def preprocess(n, selector_evals, sigma_evals, srs_table, srs_size, comm=None, srs_range=None, num_public_inputs=0):
     """selector_evals: 5 handles (q_l, q_r, q_o, q_m, q_c evaluations on H, n each); sigma_evals: 3
     handles with the evaluations of S_sigma1..3 (permutation.py:44-86).  Mirrors
     preprocessor.py:59-130: 8 iNTTs + 8 commitments, plus the static round-3 data.
     comm / srs_range: a sharded.Communicator and the (start, count) row range of the SRS that `srs_table`
     holds on this rank; every commitment of preprocess() and prove() is then a collective over the ranks,
-    while the NTT / quotient work is done by every rank for itself (it stays single-GPU work, SURVEY 8e)."""
+    while the NTT / quotient work is done by every rank for itself (it stays single-GPU work, SURVEY 8e).
+    num_public_inputs: l, 0 <= l <= n; the proofs of the key are bound to l public inputs (gates 0..l-1).
+    ValueError for l outside that range or l > 0 with a sharded SRS."""
+    num_public_inputs = int(num_public_inputs)
+    if not 0 <= num_public_inputs <= n:
+        raise ValueError("preprocess: num_public_inputs must be in [0, n = %d], got %d" % (n, num_public_inputs))
+    if num_public_inputs and comm is not None:
+        raise ValueError("preprocess: public inputs are not supported on a sharded key")
     key = DeviceKey()
+    key.num_public_inputs = num_public_inputs
     key.ranks, key.srs_range = comm, srs_range
     key.n, key.log_n = n, n.bit_length() - 1
     key.omega = int(get_root_of_unity(n))
@@ -114,6 +132,50 @@ def preprocess(n, selector_evals, sigma_evals, srs_table, srs_size, comm=None, s
     return key
 
 
+def public_input_values(values, ell, what):
+    """The l public inputs as ints: ValueError unless there are exactly l of them, each an integer in [0, r) (not
+    reduced: x and x + r would be one statement).  Decimal strings, as the reference's fixtures hold them, are read."""
+    values = list(values) if values is not None else []
+    if len(values) != ell:
+        raise ValueError("%s: %d public inputs given, the circuit has %d" % (what, len(values), ell))
+    out = []
+    for x in values:
+        if isinstance(x, (bool, float)):
+            raise ValueError("%s: public input %r is not an integer" % (what, x))
+        try:
+            v = int(x)
+        except (TypeError, ValueError):
+            raise ValueError("%s: public input %r is not an integer" % (what, x)) from None
+        if not 0 <= v < R:
+            raise ValueError("%s: public input %d is outside [0, r)" % (what, v))
+        out.append(v)
+    return out
+
+
+_R_WORDS = np.array([(R >> (64 * (3 - k))) & (2 ** 64 - 1) for k in range(4)], dtype=np.uint64)
+
+
+def _absorb_public_inputs(trs, raw, ell, j0):
+    """tr.append_scalar(b"public_input", x_j,i) for i < ell into trs[j], from raw = the inputs of every proof back to
+    back as 32-byte little-endian values, checked to be below r (a device handle is not reduced on load).  j0: the
+    batch index of trs[0], for the error."""
+    be = np.frombuffer(raw, dtype=np.uint8).reshape(len(trs), ell, 32)[:, :, ::-1]
+    words = np.ascontiguousarray(be).view(">u8").reshape(-1, 4).astype(np.uint64)
+    lt, eq = np.zeros(len(words), dtype=bool), np.ones(len(words), dtype=bool)
+    for k in range(4):
+        lt |= eq & (words[:, k] < _R_WORDS[k])
+        eq &= words[:, k] == _R_WORDS[k]
+    if not lt.all():
+        j, i = divmod(int(np.argmin(lt)), ell)
+        raise ValueError("prove_batch: public input %d of proof %d is outside [0, r)" % (i, j0 + j))
+    label = np.frombuffer(b"public_input", dtype=np.uint8)
+    rec = np.empty((len(trs), ell, len(label) + 32), dtype=np.uint8)
+    rec[:, :, :len(label)] = label
+    rec[:, :, len(label):] = be
+    for j, tr in enumerate(trs):
+        tr.state += rec[j].tobytes()
+
+
 def _blind(h, n, blinds):
     """p(x) += (b0 + b1 x + ...)(x^n - 1): subtract the b's at the bottom, add them at x^n."""
     k = len(blinds)
@@ -123,16 +185,21 @@ def _blind(h, n, blinds):
     up.free()
 
 
-def prove(key, a_vals, b_vals, c_vals, blinds=None, keep=False):
+def prove(key, a_vals, b_vals, c_vals, blinds=None, keep=False, public_inputs=None):
     """a_vals, b_vals, c_vals: device handles with the n wire values.  blinds: optional 9 scalars
     (round 1: 2 per wire polynomial, round 2: 3) to reproduce a golden proof; random otherwise.
+    public_inputs: the key's num_public_inputs ints (ValueError otherwise).
     Returns a Proof whose fields are the reference's types."""
     n, log_n, w = key.n, key.log_n, key.omega
     N8 = key.N8
+    ell = key.num_public_inputs
+    pubs = public_input_values(public_inputs, ell, "prove")
     if blinds is None:
         blinds = [secrets.randbelow(R) for _ in range(9)]
     tr = Transcript()
     proof = Proof()
+    for x in pubs:
+        tr.append_scalar(b"public_input", x)
     # ---- round 1
     wires = {}
     for i, (name, vals) in enumerate((("a", a_vals), ("b", b_vals), ("c", c_vals))):
@@ -172,11 +239,26 @@ def prove(key, a_vals, b_vals, c_vals, blinds=None, keep=False):
     tr.append_point(b"z_comm", proof.z_comm)
     # ---- round 3
     alpha = int(tr.challenge_scalar(b"alpha"))
+    circuit = {k: key.coset[k] for k in CIRCUIT_POLYS}
+    pub = None
+    if ell:
+        # PI on the coset, added into a copy of q_c's coset evaluations (Montgomery form is linear)
+        pub = native.scalars_load(native.fr_vec_bytes(pubs), ell)
+        pi = native.scalars_alloc(N8)
+        native.plonk_pi_scatter_many_dev(pub, 0, ell, ell, n, 1, pi)
+        native.ntt_dev(pi, 0, log_n, w, inverse=True)
+        native.scalars_convert(pi, 0, n, True)
+        native.ntt_dev(pi, 0, log_n + key.log_ext, key.omega8, coset_shift=COSET_SHIFT)
+        circuit["q_c"] = _alloc_from(key.coset["q_c"], N8, N8)
+        native.vec_op_dev(0, circuit["q_c"], 0, circuit["q_c"], 0, pi, 0, N8)
+        pi.free()
     t = native.scalars_alloc(N8)
-    native.plonk_quotient_dev(ext + [key.coset[k] for k in CIRCUIT_POLYS], n, key.ext, key.x, key.l1f, key.zh8, beta,
+    native.plonk_quotient_dev(ext + [circuit[k] for k in CIRCUIT_POLYS], n, key.ext, key.x, key.l1f, key.zh8, beta,
                               gamma, alpha, t)
     for e in ext:
         e.free()
+    if ell:
+        circuit["q_c"].free()
     native.ntt_dev(t, 0, log_n + key.log_ext, key.omega8, inverse=True, coset_shift=COSET_SHIFT)
     native.scalars_convert(t, 0, N8, False)
     if not native.scalars_is_zero(t, 3 * n + 6, N8 - (3 * n + 6)):
@@ -207,6 +289,9 @@ def prove(key, a_vals, b_vals, c_vals, blinds=None, keep=False):
     ab = (a_e + beta * s1_e + gamma) * (b_e + beta * s2_e + gamma) % R
     perm_s3 = alpha * ab % R * beta % R * zw_e % R
     const = (-alpha * ab % R * zw_e % R * (c_e + gamma) - alpha * alpha % R * l1_zeta) % R   # pi(zeta) = 0
+    if ell:
+        const = (const + native.plonk_pi_eval_many_dev(pub, 0, ell, ell, n, w, [zeta])[0]) % R
+        pub.free()
     # linearisation polynomial: seven scalar-times-polynomial terms in one pass
     r = native.scalars_alloc(n + 3)
     native.lincomb_dev(r, 0, n + 3,
@@ -250,33 +335,42 @@ _PASS_MSMS = ((3, 2), (1, 3), (3, 6), (2, 5))
 def plan_chunk(key, count, free_bytes):
     """Largest number of proofs per pass of prove_batch: within the 32-bit entry and 31-bit bucket numbering of the
     many-MSM (vectors * W * L < 2^32, vectors * buckets < 2^31 at the padded length L of each round's vectors), the
-    32-bit batched coset transforms (4 * count * N8 < 2^32), and half of `free_bytes` of device memory at the working
-    set estimated below.  At least 1, at most count."""
+    32-bit batched coset transforms (4 * count * N8 < 2^32, 5 with public inputs), and half of `free_bytes` of device
+    memory at the working set estimated below.  At least 1, at most count."""
     from ..groth16.device_prover import _many_msm_shape
     n, N = key.n, key.N8
-    limit = ((1 << 32) - 1) // (4 * N)
+    pi = 1 if key.num_public_inputs else 0             # one more coset block and one more n-block per proof
+    limit = ((1 << 32) - 1) // ((4 + pi) * N)
     msm_ws = 0
     for vecs, pad in _PASS_MSMS:
         W, per = _many_msm_shape(key.srs_table, n + pad)
         limit = min(limit, ((1 << 32) - 1) // (vecs * W * (n + pad)), ((1 << 31) - 1) // (vecs * per))
         msm_ws = max(msm_ws, vecs * (8 * W * (n + pad) + per * (3 * 128 + 12)))   # entries; buckets and levels
-    per_proof = msm_ws + 32 * (9 * N + 20 * n + 64)     # coset blocks, transform scratch and the per-round vectors
+    per_proof = msm_ws + 32 * ((9 + pi) * N + (20 + pi) * n + 64)  # coset blocks, transform scratch, per-round vectors
     limit = min(limit, (free_bytes // 2) // per_proof)
     return int(max(1, min(limit, count)))
 
 
-def prove_batch(key, a_vals, b_vals, c_vals, count, blinds=None, chunk=None):
+def prove_batch(key, a_vals, b_vals, c_vals, count, blinds=None, chunk=None, public_inputs=None):
     """count proofs of the circuit of `key`, proof j from the wire values at offset j * n of a_vals, b_vals, c_vals
     and blinds[j] (9 scalars in the order of prove; fresh ones from `secrets` when blinds is None).  Proof j is
     bit-identical to prove(key, a_j, b_j, c_j, blinds=blinds[j]).  Per chunk of proofs every round is a fixed number of
     launches whatever the chunk size: batched transforms, per-proof challenge arrays, segmented scans and one many-MSM
     per commitment group.  The transcripts stay on the host, one per proof.  chunk=None picks the largest chunk
     plan_chunk allows; the result does not depend on it.  An unsatisfied witness raises the ValueError of prove,
-    naming the first failing proof, before any round-3 commitment of its chunk."""
+    naming the first failing proof, before any round-3 commitment of its chunk.
+    public_inputs: for a key with l = num_public_inputs > 0, a scalar handle of count * l values, proof j's at j * l
+    (as witness.solve_batch returns them); proof j then equals prove(..., public_inputs=those l values)."""
     n = key.n
     count = int(count)
+    ell = key.num_public_inputs
     if key.ranks is not None:
         raise ValueError("prove_batch: a sharded key is not supported (batch over one GPU's SRS)")
+    if ell and (public_inputs is None or public_inputs.n < count * ell):
+        raise ValueError("prove_batch: public_inputs holds %s values, needs %d"
+                         % (None if public_inputs is None else public_inputs.n, count * ell))
+    if not ell and public_inputs is not None:
+        raise ValueError("prove_batch: the key has no public inputs (preprocess with num_public_inputs)")
     if chunk is not None and int(chunk) <= 0:
         raise ValueError("prove_batch: chunk must be positive")
     if count < 0:
@@ -296,14 +390,18 @@ def prove_batch(key, a_vals, b_vals, c_vals, count, blinds=None, chunk=None):
     step = min(int(chunk), count) if chunk is not None else plan_chunk(key, count, native.device_mem_info()[0])
     proofs = []
     for j0 in range(0, count, step):
-        proofs.extend(_prove_chunk(key, a_vals, b_vals, c_vals, j0, min(step, count - j0), blinds))
+        proofs.extend(_prove_chunk(key, a_vals, b_vals, c_vals, j0, min(step, count - j0), blinds, public_inputs))
     return proofs
 
 
-def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds):
+def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds, pub):
     n, log_n, w, N = key.n, key.log_n, key.omega, key.N8
+    ell = key.num_public_inputs
+    nb = 4 if ell else 3                                    # transform blocks per proof in round 1; + 1 in round 3
     bl = blinds[j0:j0 + cnt]
     trs = [Transcript() for _ in range(cnt)]
+    if ell:
+        _absorb_public_inputs(trs, native.scalars_download(pub, j0 * ell, cnt * ell), ell, j0)
     proofs = [Proof() for _ in range(cnt)]
     tmp = []
 
@@ -313,11 +411,14 @@ def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds):
         return h
 
     try:
-        # ---- round 1: 3 cnt inverse transforms, blinding at stride n + 2 (vector i * cnt + j: wire i of proof j)
-        ev = alloc(3 * cnt * n)
+        # ---- round 1: 3 cnt inverse transforms, blinding at stride n + 2 (vector i * cnt + j: wire i of proof j);
+        # with public inputs cnt more for PI_j, from their evaluations on H at 3 cnt n
+        ev = alloc(nb * cnt * n)
         for i, vals in enumerate((a_vals, b_vals, c_vals)):
             native.scalars_copy(ev, i * cnt * n, vals, j0 * n, cnt * n)
-        native.ntt_many_dev(ev, 0, log_n, 3 * cnt, w, inverse=True)
+        if ell:
+            native.plonk_pi_scatter_many_dev(pub, j0 * ell, ell, ell, n, cnt, ev, 3 * cnt * n)
+        native.ntt_many_dev(ev, 0, log_n, nb * cnt, w, inverse=True)
         wires = alloc(3 * cnt * (n + 2))
         native.plonk_blind_many_dev(ev, 0, n, n, 3 * cnt, [b[2 * i:2 * i + 2] for i in range(3) for b in bl], wires, 0, n + 2)
         pts = native.msm_dev_many(key.srs_table, 0, n + 2, 3 * cnt, wires)
@@ -345,12 +446,15 @@ def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds):
             tr.append_point(b"z_comm", prf.z_comm)
         # ---- round 3: 4 cnt coset transforms, the quotient with per-proof challenges, cnt inverse transforms
         alphas = [int(tr.challenge_scalar(b"alpha")) for tr in trs]
-        ext = alloc(4 * cnt * N)
-        native.plonk_coset_inputs_many_dev(wires, z, n, cnt, key.log_n + key.log_ext, ext)
-        native.ntt_many_dev(ext, 0, log_n + key.log_ext, 4 * cnt, key.omega8, coset_shift=COSET_SHIFT)
+        ext = alloc((nb + 1) * cnt * N)
+        if ell:
+            native.plonk_coset_inputs_pi_many_dev(wires, z, ev, 3 * cnt * n, n, cnt, key.log_n + key.log_ext, ext)
+        else:
+            native.plonk_coset_inputs_many_dev(wires, z, n, cnt, key.log_n + key.log_ext, ext)
+        native.ntt_many_dev(ext, 0, log_n + key.log_ext, (nb + 1) * cnt, key.omega8, coset_shift=COSET_SHIFT)
         t = alloc(cnt * N)
-        native.plonk_quotient_many_dev(ext, [key.coset[k] for k in CIRCUIT_POLYS], n, key.ext, key.x, key.l1f, key.zh8,
-                                       betas, gammas, alphas, t)
+        quotient = native.plonk_quotient_pi_many_dev if ell else native.plonk_quotient_many_dev
+        quotient(ext, [key.coset[k] for k in CIRCUIT_POLYS], n, key.ext, key.x, key.l1f, key.zh8, betas, gammas, alphas, t)
         native.ntt_many_dev(t, 0, log_n + key.log_ext, cnt, key.omega8, inverse=True, coset_shift=COSET_SHIFT)
         bad = native.plonk_divisible_many_dev(t, n, key.ext, cnt)
         if bad is not None:
@@ -377,6 +481,7 @@ def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds):
                 tr.append_scalar(name.encode(), evals[g][j])
         # ---- round 5: linearisation and opening polynomials as batched lincombs, segmented divisions by (x - zeta)
         vs = [int(tr.challenge_scalar(b"v")) for tr in trs]
+        pis = native.plonk_pi_eval_many_dev(pub, j0 * ell, ell, ell, n, w, zetas) if ell else [0] * cnt
         r_rows, p_rows = [], []
         for j in range(cnt):
             beta, gamma, alpha, zeta, v = betas[j], gammas[j], alphas[j], zetas[j], vs[j]
@@ -386,7 +491,7 @@ def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds):
             perm_z = alpha * (a_e + beta * zeta + gamma) % R * (b_e + beta * K1 * zeta + gamma) % R * (c_e + beta * K2 * zeta + gamma) % R
             ab = (a_e + beta * s1_e + gamma) * (b_e + beta * s2_e + gamma) % R
             perm_s3 = alpha * ab % R * beta % R * zw_e % R
-            const = (-alpha * ab % R * zw_e % R * (c_e + gamma) - alpha * alpha % R * l1_zeta) % R
+            const = (-alpha * ab % R * zw_e % R * (c_e + gamma) - alpha * alpha % R * l1_zeta + pis[j]) % R
             r_rows.append([a_e * b_e % R, a_e, b_e, c_e, 1, (-perm_s3) % R, (perm_z + alpha * alpha % R * l1_zeta) % R, const])
             zeta_n = pow(zeta, n, R)
             p_rows.append([1, zeta_n, zeta_n * zeta_n % R, v] + [pow(v, e, R) for e in range(2, 7)] + [0])

@@ -14,6 +14,11 @@ zkp.pairing.pairing runs them on the GPU).
 
 `verify_batch` checks k proofs against one SRS with e(sum rho_j A_j, [tau]_2) e(-sum rho_j B_j, [1]_2) == 1:
 the same two MSMs (over all proofs' terms at once) and two pairings for any k.
+
+By default both keep the reference's semantics: `public_inputs` is not read and PI(zeta) = 0.  With
+bind_public_inputs=True they check the protocol of device_prover's public inputs: the transcript absorbs
+append_scalar(b"public_input", x_i) for every input before the first challenge, and r0 gains PI(zeta), evaluated on
+the GPU (one zkp_plonk_pi_eval_many_dev call for a whole batch).
 """
 from ... import native
 from ..pairing import batch_weights, pairing_check
@@ -30,11 +35,37 @@ def _msm(terms):
     return g1_from_ints(native.g1_msm(native.g1_vec_bytes(pts), native.fr_vec_bytes(sc), len(pts)))
 
 
-def _pairing_terms(proof, public_inputs, preprocessed):
-    """(point, scalar) terms of the two G1 points A and B of the final check e(A, [tau]_2) == e(B, [1]_2)."""
-    pp = preprocessed
-    n, omega = pp.n, pp.omega
+def _public_inputs(public_inputs, pp, bind):
+    """The inputs to bind as ints ([] when not binding); ValueError before any device call for a wrong count or a
+    value that is not an integer in [0, r)."""
+    if not bind:
+        return []
+    from .device_prover import public_input_values
+    return public_input_values(public_inputs, int(getattr(pp, "num_public_inputs", 0)), "verify")
+
+
+def _pi_evals(rows):
+    """[PI_j(zeta_j)] for rows = [(inputs, pp, zeta)], one device call per (n, omega, count of inputs) group."""
+    out = [FR(0)] * len(rows)
+    groups = {}
+    for j, (pubs, pp, zeta) in enumerate(rows):
+        if pubs:
+            groups.setdefault((int(pp.n), int(pp.omega), len(pubs)), []).append(j)
+    for (n, omega, ell), idx in groups.items():
+        h = native.scalars_load(native.fr_vec_bytes([x for j in idx for x in rows[j][0]]), len(idx) * ell)
+        try:
+            vals = native.plonk_pi_eval_many_dev(h, 0, ell, ell, n, omega, [int(rows[j][2]) for j in idx])
+        finally:
+            h.free()
+        for j, v in zip(idx, vals):
+            out[j] = FR(v)
+    return out
+
+
+def _challenges(proof, pubs):
     t = Transcript()
+    for x in pubs:
+        t.append_scalar(b"public_input", x)
     for name in ("a_comm", "b_comm", "c_comm"):
         t.append_point(name.encode(), getattr(proof, name))
     beta = t.challenge_scalar(b"beta")
@@ -48,7 +79,14 @@ def _pairing_terms(proof, public_inputs, preprocessed):
         t.append_scalar(name.encode(), getattr(proof, name))
     v = t.challenge_scalar(b"v")
     u = t.challenge_scalar(b"u")
+    return beta, gamma, alpha, zeta, v, u
 
+
+def _pairing_terms(proof, preprocessed, challenges, pi_zeta):
+    """(point, scalar) terms of the two G1 points A and B of the final check e(A, [tau]_2) == e(B, [1]_2)."""
+    pp = preprocessed
+    n, omega = pp.n, pp.omega
+    beta, gamma, alpha, zeta, v, u = challenges
     a, b, c = proof.a_eval, proof.b_eval, proof.c_eval
     s1, s2, zw = proof.s_sigma1_eval, proof.s_sigma2_eval, proof.z_omega_eval
     zh = vanishing_poly_eval(n, zeta)
@@ -56,7 +94,7 @@ def _pairing_terms(proof, public_inputs, preprocessed):
     perm_z = alpha * (a + beta * zeta + gamma) * (b + beta * K1 * zeta + gamma) * (c + beta * K2 * zeta + gamma)
     ab = (a + beta * s1 + gamma) * (b + beta * s2 + gamma)
     perm_s3 = alpha * ab * beta * zw
-    r0 = FR(0) - alpha * ab * zw * (c + gamma) - alpha * alpha * l1     # PI(zeta) = 0 in the reference (:99)
+    r0 = pi_zeta - alpha * ab * zw * (c + gamma) - alpha * alpha * l1   # PI(zeta) = 0 in the reference (:99)
     zeta_n = zeta ** n
     e_scalar = proof.r_eval / zh + v * proof.r_eval
     vp = v
@@ -80,8 +118,13 @@ def _pairing_terms(proof, public_inputs, preprocessed):
     return A, B
 
 
-def verify(proof, public_inputs, preprocessed, srs, pairing=None):
-    a_terms, b_terms = _pairing_terms(proof, public_inputs, preprocessed)
+def verify(proof, public_inputs, preprocessed, srs, pairing=None, *, bind_public_inputs=False):
+    """True iff the proof passes the reference's check; with bind_public_inputs=True, also bound to public_inputs
+    (exactly preprocessed.num_public_inputs integers in [0, r), ValueError otherwise)."""
+    pubs = _public_inputs(public_inputs, preprocessed, bind_public_inputs)
+    ch = _challenges(proof, pubs)
+    pi_zeta = _pi_evals([(pubs, preprocessed, ch[3])])[0]
+    a_terms, b_terms = _pairing_terms(proof, preprocessed, ch, pi_zeta)
     A = _msm(a_terms)
     B = _msm(b_terms)
     if pairing is None:
@@ -92,17 +135,21 @@ def verify(proof, public_inputs, preprocessed, srs, pairing=None):
     return pairing(srs.g2_powers[1], A) == pairing(srs.g2_powers[0], B)
 
 
-def verify_batch(items, srs, rng=None):
+def verify_batch(items, srs, rng=None, *, bind_public_inputs=False):
     """True iff every (proof, public_inputs, preprocessed) in `items` passes `verify` against the one `srs`, up
     to a 2^-128 chance of accepting a bad batch: with random non-zero 128-bit weights rho_j (from `secrets`, or
     from rng.getrandbits for reproducible runs) it checks e(sum rho_j A_j, [tau]_2) e(-sum rho_j B_j, [1]_2) == 1,
-    i.e. two GPU MSMs over the terms of all proofs and one pairing check with two pairs."""
+    i.e. two GPU MSMs over the terms of all proofs and one pairing check with two pairs.  bind_public_inputs: as in
+    verify; every input list is checked before any device call, and all PI_j(zeta_j) come from one device call."""
     items = list(items)
     if not items:
         return True
+    pubs = [_public_inputs(public_inputs, pp, bind_public_inputs) for _, public_inputs, pp in items]
+    chs = [_challenges(proof, p) for (proof, _, _), p in zip(items, pubs)]
+    pis = _pi_evals([(p, pp, ch[3]) for p, (_, _, pp), ch in zip(pubs, items, chs)])
     a_all, b_all = [], []
-    for rho, (proof, public_inputs, pp) in zip(batch_weights(len(items), rng), items):
-        a_terms, b_terms = _pairing_terms(proof, public_inputs, pp)
+    for rho, (proof, _, pp), ch, pi_zeta in zip(batch_weights(len(items), rng), items, chs, pis):
+        a_terms, b_terms = _pairing_terms(proof, pp, ch, pi_zeta)
         a_all += [(p, int(s) * rho) for p, s in a_terms]
         b_all += [(p, int(s) * rho) for p, s in b_terms]
     return pairing_check([(srs.g2_powers[1], _msm(a_all)), (srs.g2_powers[0], _msm(b_all))], [1, CURVE_ORDER - 1])

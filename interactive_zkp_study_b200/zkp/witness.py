@@ -18,6 +18,10 @@ otherwise solve_batch raises, naming the proof and the constraint.  There is no 
     prog = compile_plonk(n, selectors, sigma, inputs=[0])
     a, b, c = solve_batch(prog, X, count)            # count * n values each
     proofs = plonk.device_prover.prove_batch(key, a, b, c, count)
+
+    prog = compile_plonk(n, selectors, sigma, inputs=[0], num_public_inputs=l)
+    a, b, c, pub = solve_batch(prog, X, count)       # X rows: l public inputs, then the inputs; pub: count * l values
+    proofs = plonk.device_prover.prove_batch(key, a, b, c, count, public_inputs=pub)
 """
 import heapq
 
@@ -46,10 +50,12 @@ def _scaled(form, k):
 class WitnessProgram:
     """A compiled circuit: the step program (host arrays, uploaded to the device on first use) and how its variables
     map to the outputs.  kind "r1cs": variable i is wire i.  kind "plonk": variables are the copy classes of sigma that
-    some gate uses (v_0 = 1 is not a class); pos_var[p] is the variable of wire position p, -1 for a class fixed at 0."""
+    some gate uses (v_0 = 1 is not a class); pos_var[p] is the variable of wire position p, -1 for a class fixed at 0;
+    pub_var: the variables of the public inputs (the first entries of each input row)."""
 
-    def __init__(self, kind, nvars, in_var, steps, size, pos_var=None):
+    def __init__(self, kind, nvars, in_var, steps, size, pos_var=None, pub_var=()):
         self.kind, self.nvars, self.size, self.pos_var = kind, nvars, size, pos_var
+        self.pub_var = list(pub_var)
         self.in_var = np.asarray(in_var, dtype=np.uint32)
         steps = sorted(steps, key=lambda st: (st[0], st[1]))   # (level, source index, out_var, forms)
         self.step_src = [st[1] for st in steps]
@@ -95,16 +101,17 @@ class WitnessProgram:
         return self._dev
 
     def selections(self):
-        """PLONK: the n x nvars 0/1 matrices that gather a, b, c from the variables (an empty row gives 0)."""
+        """PLONK: the n x nvars 0/1 matrices that gather a, b, c from the variables (an empty row gives 0), and with
+        public inputs the l x nvars one that gathers them."""
         if self._sel is None:
             n = self.size
             self._sel = []
-            for part in range(3):
-                pv = self.pos_var[part * n:(part + 1) * n]
+            parts = [self.pos_var[part * n:(part + 1) * n] for part in range(3)]
+            for pv in parts + ([self.pub_var] if self.pub_var else []):
                 rows = [[v] if v >= 0 else [] for v in pv]
                 rp = np.cumsum([0] + [len(r) for r in rows]).astype(np.uint32)
                 ci = [v for r in rows for v in r]
-                self._sel.append(native.sparse_load(rp, ci, [1] * len(ci), n, self.nvars))
+                self._sel.append(native.sparse_load(rp, ci, [1] * len(ci), len(pv), self.nvars))
         return self._sel
 
     def free(self):
@@ -209,14 +216,19 @@ def compile_r1cs(r1cs, inputs):
     return WitnessProgram("r1cs", m, inputs, steps, m)
 
 
-def compile_plonk(n, selectors, sigma, inputs):
+def compile_plonk(n, selectors, sigma, inputs, num_public_inputs=0):
     """Step program of a PLONK circuit in the reference's layout: selectors = (q_l, q_r, q_o, q_m, q_c), n values each;
     sigma a permutation of the 3n wire positions (a_g at g, b_g at n + g, c_g at 2n + g); inputs: the positions the
     caller supplies.  Variables are the copy classes (cycles of sigma).  A gate q_l a + q_r b + q_o c + q_m a b + q_c = 0
     solves its single unknown class when the equation is of degree 1 in it; the coefficient may be a linear form
     (q_l + q_m b when the unknown is a).  A class no gate uses with a non-zero coefficient, and not an input, is 0.
-    ValueError for two inputs in one class or an undetermined class."""
+    num_public_inputs: l public inputs x_0..x_{l-1}, fresh variables that come first in every input row; gate i < l
+    gains + x_i (q_l a + q_r b + q_o c + q_m a b + q_c + x_i = 0, the PI term of device_prover's public inputs).
+    ValueError for two inputs in one class, an undetermined class or l outside [0, n]."""
     n = int(n)
+    ell = int(num_public_inputs)
+    if not 0 <= ell <= n:
+        raise ValueError("compile_plonk: num_public_inputs must be in [0, %d], got %d" % (n, ell))
     q = [[int(x) % R for x in s] for s in selectors]
     sigma = [int(s) for s in sigma]
     if len(q) != 5 or any(len(s) != n for s in q):
@@ -245,12 +257,16 @@ def compile_plonk(n, selectors, sigma, inputs):
         raise ValueError("compile_plonk: two inputs lie in one copy class (positions %s)" % inputs)
     used = set(in_cls) | {c for s in slots for c in s if c is not None}
     var_of = {c: i + 1 for i, c in enumerate(sorted(used))}
-    nvars = len(used) + 1
+    pub_var = [len(used) + 1 + i for i in range(ell)]
+    pub_of = lambda g: pub_var[g] if g < ell else None     # the public-input variable in gate g's equation
+    nvars = len(used) + 1 + ell
     pos_var = [var_of.get(c, -1) for c in cls]
     gv = [tuple(var_of[c] if c is not None else None for c in s) for s in slots]
     cons_vars = [sorted({v for v in s if v is not None}) for s in gv]
     known = [False] * nvars
     known[0] = True
+    for v in pub_var:
+        known[v] = True
     for c in in_cls:
         known[var_of[c]] = True
 
@@ -272,6 +288,8 @@ def compile_plonk(n, selectors, sigma, inputs):
             if x is not None and not s and sel:
                 _add(gamma, x, R - sel)
         _add(gamma, 0, R - q_c[g])
+        if pub_of(g) is not None:
+            _add(gamma, pub_of(g), R - 1)
         if set(coeff) <= {0}:
             if not coeff:
                 return None
@@ -286,6 +304,8 @@ def compile_plonk(n, selectors, sigma, inputs):
             if x is not None and sel:
                 _add(gamma, x, sel)
         _add(gamma, 0, q_c[g])
+        if pub_of(g) is not None:
+            _add(gamma, pub_of(g), 1)
         return ({xa: q_m[g]} if q_m[g] else {}, {xb: 1} if q_m[g] else {}, gamma, ONE)
 
     steps, left = _schedule(n, cons_vars, nvars, known, solve, check)
@@ -293,14 +313,15 @@ def compile_plonk(n, selectors, sigma, inputs):
         p = pos_var.index(left[0])
         raise ValueError("compile_plonk: the copy class of %s_%d (position %d) is not determined by the gates "
                          "(%d classes undetermined)" % ("abc"[p // n], p % n, p, len(left)))
-    return WitnessProgram("plonk", nvars, [var_of[c] for c in in_cls], steps, n, pos_var)
+    return WitnessProgram("plonk", nvars, pub_var + [var_of[c] for c in in_cls], steps, n, pos_var, pub_var)
 
 
 def solve_batch(program, X, count):
     """Solve `count` witnesses of `program` on the device from the scalar handle X (witness j's inputs at
     X[j * n_in], in the order of the compiler's `inputs`).  R1CS: returns W, count * m values (witness j at j * m),
     as qap_device.prove_batch takes it.  PLONK: returns the (a_vals, b_vals, c_vals) handles of count * n values each,
-    as plonk.device_prover.prove_batch takes them.  One solving launch whatever count and the circuit depth are.
+    as plonk.device_prover.prove_batch takes them, and for a program with l public inputs a fourth handle of count * l
+    values (proof j's at j * l), its public_inputs.  One solving launch whatever count and the circuit depth are.
     ValueError naming the first failing proof and its constraint (gate) when a division by zero occurs or a
     constraint is not satisfied."""
     count = int(count)
@@ -318,10 +339,9 @@ def solve_batch(program, X, count):
         raise ValueError("solve_batch: proof %d, %s %d: %s" % (j, what, program.step_src[s], reason))
     if program.kind == "r1cs":
         return W
-    n = program.size
     out = []
     for sel in program.selections():
-        h = native.scalars_alloc(count * n)
+        h = native.scalars_alloc(count * sel.n)
         if count:
             native.sparse_matvec_many_dev(sel, W, h, count)
         out.append(h)

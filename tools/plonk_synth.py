@@ -36,6 +36,44 @@ def chain_circuit(n, seed=1, break_witness=False):
     return {"n": n, "a": a, "b": b, "c": c, "sel": [q_l, q_r, q_o, q_m, q_c], "sigma": sigma}
 
 
+def prepend_public_gates(circ, tied, n=None, public_inputs=None):
+    """The circuit `circ` (keys n, a, b, c, sel, sigma) behind len(tied) public-input gates, padded with zero gates to n
+    gates (default: the smallest power of two that fits).  Gate i has q_l = -1, so with the PI term it reads
+    x_i - a_i = 0, and a_i is copy-constrained to wire position tied[i] of circ; x_i defaults to that wire's value.
+    Adds "num_public_inputs", "public_inputs" and "pos", the map from circ's wire positions to the new ones."""
+    ell, m = len(tied), circ["n"]
+    n = n or 1 << max(0, (m + ell - 1).bit_length())
+    if n < m + ell:
+        raise ValueError("prepend_public_gates: %d gates do not fit in %d" % (m + ell, n))
+    pos = lambda p: (p // m) * n + ell + p % m
+    sigma = list(range(3 * n))
+    for p in range(3 * m):
+        sigma[pos(p)] = pos(circ["sigma"][p])
+    for i, p in enumerate(tied):                          # splice a_i into the copy cycle of the tied wire
+        q = pos(p)
+        sigma[i], sigma[q] = sigma[q], sigma[i]
+    wires = circ["a"] + circ["b"] + circ["c"]
+    x = [wires[p] for p in tied] if public_inputs is None else list(public_inputs)
+    pad, zeros = [0] * (n - ell - m), [0] * ell
+    a, b, c = (x + circ["a"] + pad, zeros + circ["b"] + pad, zeros + circ["c"] + pad)
+    sel = [zeros + list(q) + pad for q in circ["sel"]]
+    sel[0][:ell] = [R - 1] * ell
+    return {"n": n, "a": a, "b": b, "c": c, "sel": sel, "sigma": sigma, "num_public_inputs": ell,
+            "public_inputs": x, "pos": [pos(p) for p in range(3 * m)]}
+
+
+def public_chain_circuit(n, ell, seed=1):
+    """chain_circuit of n - ell gates behind ell public-input gates, public input i tied to b of chain gate i
+    (2 ell <= n): the public inputs are the first ell free inputs of the chain.  "inputs": the wire positions a witness
+    solver takes after the public inputs (a of the first chain gate, then the untied b's)."""
+    if not 0 <= 2 * ell <= n:
+        raise ValueError("public_chain_circuit: needs 2 * ell <= n")
+    m = n - ell
+    circ = prepend_public_gates(chain_circuit(m, seed), [m + i for i in range(ell)], n)
+    circ["inputs"] = [ell] + [n + g for g in range(2 * ell, n)]
+    return circ
+
+
 def sigma_evals_bytes(sigma, n, omega):
     """Evaluations of S_sigma1..3 (permutation.py:44-86): position -> K * w^i, as three byte strings."""
     dom = nat.scalars_alloc(n)
@@ -56,7 +94,8 @@ def sigma_evals_bytes(sigma, n, omega):
 def device_setup(circ, srs_tau=None, precompute=True, comm=None):
     """SRS on the device (tau^i G from a prefix-product + fixed-base kernel), the circuit uploaded, the
     device key preprocessed.  Returns (key, witness handles, tau).  comm: a sharded.Communicator -> every rank
-    keeps only its row range of the SRS and all commitments are collective (same arguments on every rank)."""
+    keeps only its row range of the SRS and all commitments are collective (same arguments on every rank).  A circuit
+    with "num_public_inputs" (public_chain_circuit) gets a key bound to that many public inputs."""
     from interactive_zkp_study_b200.zkp.plonk import device_prover as dp
     from interactive_zkp_study_b200.zkp.plonk.field import get_root_of_unity
     n = circ["n"]
@@ -76,6 +115,7 @@ def device_setup(circ, srs_tau=None, precompute=True, comm=None):
     enc = nat.fr_vec_bytes
     sel_h = [nat.scalars_load(enc(v), n) for v in circ["sel"]]
     sig_h = [nat.scalars_load(bts, n) for bts in sigma_evals_bytes(circ["sigma"], n, omega)]
-    key = dp.preprocess(n, sel_h, sig_h, srs, size, comm=comm, srs_range=srs_range)
+    key = dp.preprocess(n, sel_h, sig_h, srs, size, comm=comm, srs_range=srs_range,
+                        num_public_inputs=circ.get("num_public_inputs", 0))
     wit = [nat.scalars_load(enc(circ[k]), n) for k in "abc"]
     return key, wit, tau
