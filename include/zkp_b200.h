@@ -188,6 +188,19 @@ int zkp_g2_table_scale(uint64_t table, uint64_t offset, uint64_t scalars, uint64
 int zkp_g1_table_validate(uint64_t table, uint64_t offset, uint64_t n, uint64_t* first_bad);
 int zkp_g2_table_validate(uint64_t table, uint64_t offset, uint64_t n, int subgroup_check, uint64_t* first_bad);
 int zkp_table_download(uint64_t table, uint64_t offset, uint64_t n, uint8_t* out_pts);
+/* Compressed points (csrc/point_codec.cuh): the storage form of SRSs, keys and proofs, half the size of the affine
+ * encoding above (the wire format of plonk_serializers.py:23-250 writes x and y).  G1: 32 B, x little-endian; G2:
+ * 64 B, x.c0 | x.c1.  The top two bits of the last byte are flags: bit 7 y-sign (G1: y > (p-1)/2; G2: y1 > (p-1)/2,
+ * or y0 > (p-1)/2 when y1 = 0), bit 6 infinity (every other bit zero).  Decoding takes the square root of x^3 + b,
+ * so it also checks the point: a field >= p, both flags, an infinity encoding with another bit set, or an x with no
+ * point is invalid, and G2 with subgroup_check also a twist point outside the order-r subgroup.
+ * load: n encodings -> a new plain table, usable by every table entry point.  *first_bad = lowest invalid index, or
+ *   UINT64_MAX.  On an invalid encoding *handle = 0 and nothing stays allocated (the call itself returns ZKP_OK).
+ * download: table rows [offset, offset + n) -> compressed encodings on the host (G1 or G2 by handle kind); plain
+ *   or window-precomputed tables (the points are the first row). */
+int zkp_g1_table_load_compressed(const uint8_t* enc, uint64_t n, uint64_t* handle, uint64_t* first_bad);
+int zkp_g2_table_load_compressed(const uint8_t* enc, uint64_t n, int subgroup_check, uint64_t* handle, uint64_t* first_bad);
+int zkp_table_download_compressed(uint64_t table, uint64_t offset, uint64_t n, uint8_t* out);
 int zkp_scalars_download(uint64_t scalars, uint64_t offset, uint64_t n, uint8_t* out);
 
 /* ---- synthetic inputs (bench / large parity tests; SURVEY 8d) --------------------------------

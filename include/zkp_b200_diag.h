@@ -30,9 +30,11 @@ int zkp_imad_peak(int variant, double* gmacs_per_s, double* sm_clock_mhz_effecti
  * The MSM's reduction tail is bounded by these, not by throughput. */
 int zkp_latency_probe(int mode, double* ns_per_op);
 /* Field-op self-test hooks used by tests/ (field: 0 = Fp, 1 = Fr, 2 = Fp2 with 64-byte elements c0 || c1 and
- * ops 2 / 3 / 4 only; op: 0 add, 1 sub, 2 mul, 3 inv, 4 sqr,
+ * ops 2 / 3 / 4 / 9 only; op: 0 add, 1 sub, 2 mul, 3 inv, 4 sqr,
  * 5 Fermat inverse, 6 mul as 512-bit product + separate Montgomery reduction, 7 inverse by binary extended Euclid,
- * 8 a b - (a + b)(a - b) through the lazily reduced product pair of the group formulas' Y coordinate) */
+ * 8 a b - (a + b)(a - b) through the lazily reduced product pair of the group formulas' Y coordinate,
+ * 9 the square root of the point decoder (csrc/point_codec.cuh; Fp and Fp2 only), all-ones bytes when a is not a
+ * square) */
 int zkp_dbg_field_op(int field, int op, const uint8_t* a, const uint8_t* b, uint64_t n, uint8_t* out);
 /* out[i] = a[i] + b[i] (group: 0 = G1, 1 = G2; 2 / 3 = the same through the quad-lane operations of
  * csrc/ec_quad.cuh) via XYZZ, result affine; exercises all edge cases */

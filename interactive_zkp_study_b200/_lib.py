@@ -87,6 +87,9 @@ PROTOTYPES = {
     "zkp_g1_table_validate": (c_int, [u64, u64, u64, u64p]),
     "zkp_g2_table_validate": (c_int, [u64, u64, u64, c_int, u64p]),
     "zkp_table_download": (c_int, [u64, u64, u64, vp]),
+    "zkp_g1_table_load_compressed": (c_int, [vp, u64, u64p, u64p]),
+    "zkp_g2_table_load_compressed": (c_int, [vp, u64, c_int, u64p, u64p]),
+    "zkp_table_download_compressed": (c_int, [u64, u64, u64, vp]),
     "zkp_scalars_download": (c_int, [u64, u64, u64, vp]),
     "zkp_scalars_generate": (c_int, [u64, u64, u64p]),
     "zkp_fr_ntt": (c_int, [vp, u32, vp, c_int, vp]),

@@ -6,6 +6,7 @@
 #include "../../include/zkp_b200_diag.h"
 #include "ec.cuh"
 #include "ec_quad.cuh"
+#include "point_codec.cuh"
 #include "registry.cuh"
 
 namespace zkp {
@@ -281,6 +282,14 @@ __global__ void dbg_field_op_kernel(int op, const FE* a, const FE* b, uint64_t n
   uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   FE x = a[i].to_mont(), y = b ? b[i].to_mont() : FE::zero(), r;
+  if constexpr (FE::Params::MOD_(0) == FpParams::MOD_(0)) {
+    if (op == 9) {
+      if (!fp_sqrt(x, r)) r.v[0] = r.v[1] = r.v[2] = r.v[3] = r.v[4] = r.v[5] = r.v[6] = r.v[7] = ~0u;
+      else r = r.from_mont();
+      out[i] = r;
+      return;
+    }
+  }
   switch (op) {
     case 0: r = x + y; break;
     case 1: r = x - y; break;
@@ -313,6 +322,13 @@ __global__ void dbg_fp2_op_kernel(int op, const Fp2* a, const Fp2* b, uint64_t n
   switch (op) {
     case 2: r = x * y; break;
     case 3: r = x.inv(); break;
+    case 9:
+      if (!fp2_sqrt(x, r)) {
+        for (int k = 0; k < 8; k++) r.c0.v[k] = r.c1.v[k] = ~0u;
+        out[i] = r;
+        return;
+      }
+      break;
     default: r = x.sqr(); break;
   }
   out[i] = r.from_mont();
@@ -424,9 +440,10 @@ int zkp_imad_peak(int variant, double* gmacs_per_s, double* sm_clock_mhz_effecti
 
 int zkp_dbg_field_op(int field, int op, const uint8_t* a, const uint8_t* b, uint64_t n, uint8_t* out) {
   return guarded([&](Context& c) {
-    if (!a || !out || op < 0 || op > 8) throw InvalidArgument("zkp_dbg_field_op: bad argument");
+    if (!a || !out || op < 0 || op > 9) throw InvalidArgument("zkp_dbg_field_op: bad argument");
     if (n == 0) return;
     if (field < 0 || field > 2) throw InvalidArgument("zkp_dbg_field_op: field must be 0 (Fp), 1 (Fr) or 2 (Fp2)");
+    if (op == 9 && field == 1) throw InvalidArgument("zkp_dbg_field_op: the square root is for Fp and Fp2 (p = 3 mod 4)");
     const size_t sz = field == 2 ? 64 : 32;
     ScopedDevBuf da, db, dout;
     da.reserve(n * sz);

@@ -5,6 +5,7 @@
 #include "comm.cuh"
 #include "curve_check.cuh"
 #include "msm.cuh"
+#include "point_codec.cuh"
 #include "registry.cuh"
 
 namespace zkp {
@@ -573,6 +574,49 @@ struct GroupApi {
       }
       *first_bad = bad;
     });
+  }
+
+  // n compressed encodings (PT / 2 bytes each, point_codec.cuh) -> a new plain table, decoded and checked in one
+  // launch.  *first_bad = lowest rejected index or UINT64_MAX; on a rejection no handle is made (*handle = 0).
+  static int table_load_compressed(const uint8_t* enc, uint64_t n, bool subgroup, uint64_t* handle, uint64_t* first_bad) {
+    return guarded([&](Context& c) {
+      if (!handle || !first_bad || (n && !enc)) throw InvalidArgument("table_load_compressed: null argument");
+      *handle = 0;
+      auto r = std::make_unique<Resource>();
+      r->kind = KIND;
+      r->n = n;
+      r->buf.reserve_pooled(n ? n * PT : PT);
+      unsigned long long bad = ~0ull;
+      if (n) {
+        DevBuf& de = scratch_pts();
+        de.reserve(n * PT / 2);
+        ScopedDevBuf flag;
+        flag.reserve(sizeof bad);
+        CUDA_CHECK(cudaMemcpyAsync(de.p, enc, n * PT / 2, cudaMemcpyHostToDevice, c.stream));
+        CUDA_CHECK(cudaMemsetAsync(flag.p, 0xff, sizeof bad, c.stream));
+        constexpr unsigned BLK = std::is_same<F, Fp2>::value ? 64 : 128;
+        decompress_kernel<F><<<ceil_div(n, BLK), BLK, 0, c.stream>>>(de.as<uint4>(), n, subgroup, r->buf.as<Affine<F>>(),
+                                                                     flag.as<unsigned long long>());
+        CUDA_CHECK_LAUNCH();
+        c.launches++;
+        CUDA_CHECK(cudaMemcpyAsync(&bad, flag.p, sizeof bad, cudaMemcpyDeviceToHost, c.stream));
+      }
+      CUDA_CHECK(cudaStreamSynchronize(c.stream));
+      *first_bad = bad;
+      if (bad == ~0ull) *handle = registry().put(std::move(r));
+    });
+  }
+
+  static void download_compressed(Context& c, Resource* t, uint64_t offset, uint64_t n, uint8_t* out) {
+    if (!range_ok(offset, n, t->n)) throw InvalidArgument("table_download_compressed: range out of bounds");
+    if (!n) return;
+    DevBuf& dp = scratch_pts();
+    dp.reserve(n * PT / 2);
+    compress_kernel<F><<<ceil_div(n, 128), 128, 0, c.stream>>>(table_points(t, offset), n, dp.as<uint4>());
+    CUDA_CHECK_LAUNCH();
+    c.launches++;
+    CUDA_CHECK(cudaMemcpyAsync(out, dp.p, n * PT / 2, cudaMemcpyDeviceToHost, c.stream));
+    CUDA_CHECK(cudaStreamSynchronize(c.stream));
   }
 
   static void download(Context& c, Resource* t, uint64_t offset, uint64_t n, uint8_t* out_pts) {

@@ -132,6 +132,24 @@ int zkp_table_download(uint64_t table, uint64_t offset, uint64_t n, uint8_t* out
   });
 }
 
+int zkp_g1_table_load_compressed(const uint8_t* enc, uint64_t n, uint64_t* handle, uint64_t* first_bad) {
+  return Api::table_load_compressed(enc, n, false, handle, first_bad);
+}
+
+// G1 or G2 table -> compressed encodings on the host (32 / 64 B per point)
+int zkp_table_download_compressed(uint64_t table, uint64_t offset, uint64_t n, uint8_t* out) {
+  return guarded([&](Context& c) {
+    if (n && !out) throw InvalidArgument("zkp_table_download_compressed: null output");
+    if (Resource* t = registry().get(table, HandleKind::G1Table)) {
+      GroupApi<Fp>::download_compressed(c, t, offset, n, out);
+    } else if (Resource* t2 = registry().get(table, HandleKind::G2Table)) {
+      GroupApi<Fp2>::download_compressed(c, t2, offset, n, out);
+    } else {
+      throw BadHandle("zkp_table_download_compressed: not a point table");
+    }
+  });
+}
+
 // The three multi-scalar multiplications of one Groth16 proof (proving.py:23-75 reduced to one MSM per
 // element, device_prover.py): B (G2) runs on the second stream beside A and C (G1) on the first.  The G2
 // accumulation keeps only 8 warps per SM busy (228 registers per thread), so blocks of the G1 kernels

@@ -60,6 +60,10 @@ int zkp_g2_table_scale(uint64_t table, uint64_t offset, uint64_t scalars, uint64
 int zkp_g2_table_validate(uint64_t table, uint64_t offset, uint64_t n, int subgroup_check, uint64_t* first_bad) {
   return Api::table_validate(table, offset, n, subgroup_check, first_bad);
 }
+int zkp_g2_table_load_compressed(const uint8_t* enc, uint64_t n, int subgroup_check, uint64_t* handle,
+                                 uint64_t* first_bad) {
+  return Api::table_load_compressed(enc, n, subgroup_check != 0, handle, first_bad);
+}
 int zkp_g2_table_precompute(uint64_t table, int window_bits) { return Api::table_precompute(table, window_bits); }
 int zkp_g2_msm_dev_many(uint64_t table, uint64_t offset, uint64_t n, uint32_t count, uint64_t scalars, uint64_t sc_offset,
                         uint8_t* out_xy, int* out_is_inf) {

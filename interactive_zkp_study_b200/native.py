@@ -52,6 +52,39 @@ def g2_vec_bytes(pts):
     return b"".join([g2_bytes(p) for p in pts])
 
 
+# Compressed points (csrc/point_codec.cuh): x plus a y-sign flag (bit 255) and an infinity flag (bit 254) in the last
+# 32-byte field element.  Encoding a point the caller holds is one comparison; decoding needs a square root and is
+# done on the device (g1_table_load_compressed / g2_table_load_compressed).
+_HALF_P = (P_MOD - 1) // 2
+_FLAG_SIGN, _FLAG_INF = 1 << 255, 1 << 254
+
+
+def g1_compressed_bytes(pt):
+    if pt is None:
+        return _FLAG_INF.to_bytes(32, "little")
+    x, y = int(pt[0]), int(pt[1])
+    return (x | (_FLAG_SIGN if y > _HALF_P else 0)).to_bytes(32, "little")
+
+
+def g1_vec_compressed_bytes(pts):
+    return b"".join([g1_compressed_bytes(p) for p in pts])
+
+
+def g2_compressed_bytes(pt):
+    if pt is None:
+        return bytes(32) + _FLAG_INF.to_bytes(32, "little")
+    (x, y) = pt
+    xc = x.coeffs if hasattr(x, "coeffs") else x
+    yc = y.coeffs if hasattr(y, "coeffs") else y
+    y0, y1 = int(yc[0]), int(yc[1])
+    sign = y1 > _HALF_P if y1 else y0 > _HALF_P
+    return int(xc[0]).to_bytes(32, "little") + (int(xc[1]) | (_FLAG_SIGN if sign else 0)).to_bytes(32, "little")
+
+
+def g2_vec_compressed_bytes(pts):
+    return b"".join([g2_compressed_bytes(p) for p in pts])
+
+
 def g1_from_bytes(b, is_inf=False):
     if is_inf or b == bytes(64):
         return None
@@ -232,6 +265,43 @@ def table_download(handle, offset, n):
     sz = 64 if handle.kind == "g1" else 128
     out = bytearray(sz * n)
     check(_lib.lib().zkp_table_download(handle.handle, offset, n, buf(out)))
+    return bytes(out)
+
+
+class InvalidPointError(ValueError):
+    """A compressed encoding the device decoder rejected; `index` is the lowest such index of the call."""
+
+    def __init__(self, msg, index):
+        super().__init__(msg)
+        self.index = index
+
+
+def _load_compressed(what, enc, n, size, *extra):
+    enc = bytes(enc)
+    if len(enc) != size * n:
+        raise ValueError("%s: %d compressed points need %d bytes, got %d" % (what, n, size * n, len(enc)))
+    h, bad = ctypes.c_uint64(), ctypes.c_uint64()
+    check(getattr(_lib.lib(), "zkp_" + what)(buf(enc) if n else None, n, *extra, ctypes.byref(h), ctypes.byref(bad)))
+    if _first_bad(bad.value) is not None:
+        raise InvalidPointError("%s: invalid compressed point at index %d" % (what, bad.value), bad.value)
+    return DeviceHandle(h.value, n, "g1" if size == 32 else "g2")
+
+
+def g1_table_load_compressed(enc, n):
+    """n compressed G1 points (32 B each) -> a plain table, decoded on the device.  Raises ValueError naming the lowest
+    index whose encoding is invalid (bad flags, x >= p, or no point with that x)."""
+    return _load_compressed("g1_table_load_compressed", enc, n, 32)
+
+
+def g2_table_load_compressed(enc, n, subgroup_check=True):
+    """n compressed G2 points (64 B each) -> a plain table; with subgroup_check a point outside G2 is invalid too."""
+    return _load_compressed("g2_table_load_compressed", enc, n, 64, 1 if subgroup_check else 0)
+
+
+def table_download_compressed(handle, offset, n):
+    """Points [offset, offset + n) of a G1 / G2 table as compressed encodings (32 / 64 B each)."""
+    out = bytearray((32 if handle.kind == "g1" else 64) * n)
+    check(_lib.lib().zkp_table_download_compressed(handle.handle, offset, n, buf(out)))
     return bytes(out)
 
 

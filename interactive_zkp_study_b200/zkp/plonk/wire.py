@@ -15,11 +15,16 @@ written and read without ever becoming Python integers:
 Composite objects (SRS, PreprocessedData, Proof, ceremony Contribution) are a flat container: magic, then (name, tag, length,
 payload) records.  `to_text` / `from_text` wrap any payload as base64 for stores that only take strings
 (TinyDB, JSON responses).
+
+With `compressed=True` the serializers write points compressed (native.g1_compressed_bytes / g2_compressed_bytes:
+x plus a y-sign and an infinity flag, 32 / 64 bytes) under their own record tags; uncompressed stays the default.
+Every deserializer reads both.  Compressed points are decoded on the device, all G1 points of an object in one call
+and all G2 points in another, which also checks them: a G1 point lies on the curve, a G2 point in G2.
 """
 import base64
 import struct
 
-from ... import native
+from ... import native, tables
 from ...compat import FQ, FQ2, curve_order
 from .ceremony import Contribution
 from .field import FR
@@ -31,6 +36,7 @@ from .transcript import Transcript
 
 MAGIC = b"ZKPB\x01"
 T_NONE, T_FR, T_G1, T_G2, T_FRVEC, T_INT, T_U32VEC, T_G1VEC, T_G2VEC, T_BYTES = range(10)
+T_G1C, T_G2C, T_G1CVEC, T_G2CVEC = range(10, 14)  # compressed points
 
 
 # ------------------------------------------------------------------ scalars and points
@@ -130,17 +136,70 @@ def loads(blob):
     return out
 
 
-def _g1f(name, p):
-    return (name, T_NONE, None) if p is None else (name, T_G1, serialize_g1(p))
+def _g1f(name, p, compressed=False):
+    if p is None:
+        return (name, T_NONE, None)
+    return (name, T_G1C, native.g1_compressed_bytes(p)) if compressed else (name, T_G1, serialize_g1(p))
 
 
 def _frf(name, v):
     return (name, T_NONE, None) if v is None else (name, T_FR, serialize_fr(v))
 
 
-def _get_g1(rec, name):
-    tag, payload = rec.get(name, (T_NONE, b""))
-    return None if tag == T_NONE else deserialize_g1(payload)
+def _split(what, payload, size):
+    if len(payload) % size:
+        raise ValueError("%s: %d bytes is not a whole number of %d-byte points" % (what, len(payload), size))
+    return len(payload) // size
+
+
+def _decode_compressed(what, payload, g2):
+    """Compressed G1 / G2 points, back to back -> points as deserialize_g1 / g2 give them: one device decode (G2 with
+    the subgroup check).  A rejected encoding raises native.InvalidPointError (a ValueError) with its index."""
+    size = 64 if g2 else 32
+    n = _split(what, payload, size)
+    if not n:
+        return []
+    if g2:
+        h = native.g2_table_load_compressed(payload, n, subgroup_check=True)
+    else:
+        h = native.g1_table_load_compressed(payload, n)
+    raw = native.table_download(h, 0, n)
+    h.free()
+    dec, sz = (deserialize_g2, 128) if g2 else (deserialize_g1, 64)
+    return [dec(raw[sz * i:sz * i + sz]) for i in range(n)]
+
+
+def _get_g1s(rec, names, what):
+    """{name: point} for the single-G1 records `names`; the compressed ones are decoded together."""
+    out, comp = {}, []
+    for name in names:
+        tag, payload = rec.get(name, (T_NONE, b""))
+        if tag == T_G1C:
+            if len(payload) != 32:
+                raise ValueError("%s: record %s holds %d bytes, a compressed G1 point is 32" % (what, name, len(payload)))
+            comp.append((name, payload))
+        else:
+            out[name] = None if tag == T_NONE else deserialize_g1(payload)
+    try:
+        pts = _decode_compressed(what, b"".join(p for _, p in comp), False)
+    except native.InvalidPointError as e:
+        raise ValueError("%s: record %s is not a valid compressed G1 point" % (what, comp[e.index][0])) from e
+    out.update(zip([name for name, _ in comp], pts))
+    return out
+
+
+def _g1_vec(rec, name, what):
+    tag, payload = rec[name]
+    if tag == T_G1CVEC:
+        return _decode_compressed(what, payload, False)
+    return [deserialize_g1(payload[i:i + 64]) for i in range(0, len(payload), 64)]
+
+
+def _g2_vec(rec, name, what):
+    tag, payload = rec[name]
+    if tag == T_G2CVEC:
+        return _decode_compressed(what, payload, True)
+    return [deserialize_g2(payload[i:i + 128]) for i in range(0, len(payload), 128)]
 
 
 def _get_fr(rec, name):
@@ -157,41 +216,86 @@ def from_text(text):
 
 
 # ------------------------------------------------------------------ SRS
-def serialize_srs(srs):
-    return dumps([("g1_powers", T_G1VEC, native.g1_vec_bytes(srs.g1_powers)),
-                  ("g2_powers", T_G2VEC, native.g2_vec_bytes(srs.g2_powers)),
-                  ("max_degree", T_INT, struct.pack("<q", srs.max_degree))])
+def _srs_fields(g1_payload, g2_powers, max_degree, compressed):
+    g2 = native.g2_vec_compressed_bytes(g2_powers) if compressed else native.g2_vec_bytes(g2_powers)
+    return dumps([("g1_powers", T_G1CVEC if compressed else T_G1VEC, g1_payload),
+                  ("g2_powers", T_G2CVEC if compressed else T_G2VEC, g2),
+                  ("max_degree", T_INT, struct.pack("<q", max_degree))])
+
+
+def serialize_srs(srs, compressed=False):
+    """compressed=True: 32 bytes per G1 power and 64 per G2 power instead of 64 / 128."""
+    g1 = native.g1_vec_compressed_bytes(srs.g1_powers) if compressed else native.g1_vec_bytes(srs.g1_powers)
+    return _srs_fields(g1, srs.g2_powers, srs.max_degree, compressed)
 
 
 def deserialize_srs(blob):
     rec = loads(blob)
-    g1b, g2b = rec["g1_powers"][1], rec["g2_powers"][1]
-    g1 = [deserialize_g1(g1b[i:i + 64]) for i in range(0, len(g1b), 64)]
-    g2 = [deserialize_g2(g2b[i:i + 128]) for i in range(0, len(g2b), 128)]
+    g1 = _g1_vec(rec, "g1_powers", "deserialize_srs")
+    g2 = _g2_vec(rec, "g2_powers", "deserialize_srs")
     return SRS(g1, g2, struct.unpack("<q", rec["max_degree"][1])[0])
 
 
+def deserialize_srs_to_table(blob, precompute=True):
+    """SRS blob -> (G1 table handle, g2_powers, max_degree) without making the G1 powers Python integers.  A
+    compressed G1 vector is decoded on the device (g1_table_load_compressed); an uncompressed one is uploaded and put
+    through g1_table_validate, so either encoding is checked.  ValueError names the first G1 power that is not a
+    point of the curve.  precompute=True gives the window-precomputed layout tables.g1_table gives a cached SRS; the
+    handle goes straight to plonk.device_prover.preprocess(..., srs_table, srs_size)."""
+    rec = loads(blob)
+    tag, g1b = rec["g1_powers"]
+    what = "deserialize_srs_to_table"
+    if tag == T_G1CVEC:
+        n = _split(what, g1b, 32)
+        try:
+            table = native.g1_table_load_compressed(g1b, n)
+        except native.InvalidPointError as e:
+            raise ValueError("%s: G1 power %d is not a valid compressed point" % (what, e.index)) from e
+    elif tag == T_G1VEC:
+        n = _split(what, g1b, 64)
+        table = native.g1_table_load(g1b, n)
+        bad = native.g1_table_validate(table, 0, n)
+        if bad is not None:
+            table.free()
+            raise ValueError("%s: G1 power %d is not on the curve" % (what, bad))
+    else:
+        raise ValueError("%s: g1_powers is not a G1 vector record (tag %d)" % (what, tag))
+    g2 = _g2_vec(rec, "g2_powers", what)
+    if precompute:
+        tables._maybe_precompute(table, n)
+    return table, g2, struct.unpack("<q", rec["max_degree"][1])[0]
+
+
+def serialize_srs_table(table, g2_powers, max_degree, compressed=False):
+    """The inverse of deserialize_srs_to_table: a device-resident G1 table (SRS.generate's, a ceremony's) written as
+    serialize_srs would write the same SRS, straight from the device (zkp_table_download[_compressed])."""
+    dl = native.table_download_compressed if compressed else native.table_download
+    return _srs_fields(dl(table, 0, table.n), g2_powers, max_degree, compressed)
+
+
 # ------------------------------------------------------------------ powers-of-tau Contribution (ceremony.py)
-def serialize_contribution(contribution):
-    return dumps([_g1f("s_g1", contribution.s_g1), _g1f("R", contribution.R), _frf("z", contribution.z)])
+def serialize_contribution(contribution, compressed=False):
+    return dumps([_g1f("s_g1", contribution.s_g1, compressed), _g1f("R", contribution.R, compressed),
+                  _frf("z", contribution.z)])
 
 
 def deserialize_contribution(blob):
     rec = loads(blob)
     z = _get_fr(rec, "z")
-    return Contribution(_get_g1(rec, "s_g1"), _get_g1(rec, "R"), 0 if z is None else int(z))
+    g1 = _get_g1s(rec, ("s_g1", "R"), "deserialize_contribution")
+    return Contribution(g1["s_g1"], g1["R"], 0 if z is None else int(z))
 
 
 # ------------------------------------------------------------------ PreprocessedData
 _PP_POLYS = ("q_l", "q_r", "q_o", "q_m", "q_c", "s_sigma1", "s_sigma2", "s_sigma3")
 
 
-def serialize_preprocessed(pp):
+def serialize_preprocessed(pp, compressed=False):
     fields = [("n", T_INT, struct.pack("<q", pp.n)), ("omega", T_FR, serialize_fr(pp.omega)),
               ("domain", T_FRVEC, serialize_fr_list(pp.domain))]
     for name in _PP_POLYS:
         fields.append((name + "_poly", T_FRVEC, serialize_poly(getattr(pp, name + "_poly"))))
-        fields.append(_g1f(name + "_comm", getattr(pp, name + "_comm")))
+        fields.append(_g1f(name + "_comm", getattr(pp, name + "_comm"), compressed))
     fields.append(("sigma", T_U32VEC, struct.pack("<%dI" % len(pp.sigma), *pp.sigma)))
     fields.append(("num_public_inputs", T_INT, struct.pack("<q", pp.num_public_inputs)))
     return dumps(fields)
@@ -203,9 +307,10 @@ def deserialize_preprocessed(blob):
     pp.n = struct.unpack("<q", rec["n"][1])[0]
     pp.omega = deserialize_fr(rec["omega"][1])
     pp.domain = deserialize_fr_list(rec["domain"][1])
+    comms = _get_g1s(rec, [name + "_comm" for name in _PP_POLYS], "deserialize_preprocessed")
     for name in _PP_POLYS:
         setattr(pp, name + "_poly", deserialize_poly(rec[name + "_poly"][1]))
-        setattr(pp, name + "_comm", _get_g1(rec, name + "_comm"))
+        setattr(pp, name + "_comm", comms[name + "_comm"])
     sb = rec["sigma"][1]
     pp.sigma = list(struct.unpack("<%dI" % (len(sb) // 4), sb))
     pp.num_public_inputs = struct.unpack("<q", rec["num_public_inputs"][1])[0]
@@ -218,16 +323,18 @@ _PROOF_G1 = ("a_comm", "b_comm", "c_comm", "z_comm", "t_lo_comm", "t_mid_comm", 
 _PROOF_FR = ("a_eval", "b_eval", "c_eval", "s_sigma1_eval", "s_sigma2_eval", "z_omega_eval", "r_eval")
 
 
-def serialize_proof(proof):
-    """9 G1 points + 7 field elements: 800 bytes of payload for a complete proof."""
-    return dumps([_g1f(n, getattr(proof, n)) for n in _PROOF_G1] + [_frf(n, getattr(proof, n)) for n in _PROOF_FR])
+def serialize_proof(proof, compressed=False):
+    """9 G1 points + 7 field elements: 800 bytes of payload for a complete proof, 512 compressed."""
+    return dumps([_g1f(n, getattr(proof, n), compressed) for n in _PROOF_G1] +
+                 [_frf(n, getattr(proof, n)) for n in _PROOF_FR])
 
 
 def deserialize_proof(blob):
     rec = loads(blob)
     proof = Proof()
+    g1 = _get_g1s(rec, _PROOF_G1, "deserialize_proof")
     for n in _PROOF_G1:
-        setattr(proof, n, _get_g1(rec, n))
+        setattr(proof, n, g1[n])
     for n in _PROOF_FR:
         setattr(proof, n, _get_fr(rec, n))
     return proof
