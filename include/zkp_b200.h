@@ -380,6 +380,32 @@ int zkp_plonk_quotient_pi_many_dev(uint64_t evals, const uint64_t circuit[8], ui
                                    const uint8_t* alphas, uint64_t t_out);
 int zkp_plonk_pi_eval_many_dev(uint64_t pub, uint64_t off, uint64_t stride, uint64_t ell, uint64_t n, uint32_t count,
                                const uint8_t omega[32], const uint8_t* zetas, uint8_t* out);
+/* ---- batch PLONK proving over many circuits of one size (zkp/plonk/device_prover.py prove_batch_circuits) --------
+ * PLONK's SRS is universal: circuits of one size n commit against one table, so one pass can prove for several
+ * circuits.  Proof j proves circuit circuit_of[j] < ncirc (count x uint32, each checked before any launch).  The
+ * circuits' device vectors are addressed through a table of pointers resolved from their handles (circuit-major rows,
+ * every handle checked for its length); key data is never copied.  Per proof, each entry gives exactly what its
+ * one-circuit form above gives with that circuit's vectors.
+ * zkp_plonk_perm_terms_multi_dev: zkp_plonk_perm_terms_many_dev (permutation.py:120-135) with sigmas = ncirc rows of
+ *   3 handles (S_sigma1..3 on H, n each).
+ * zkp_plonk_quotient_multi_dev, zkp_plonk_quotient_pi_multi_dev: zkp_plonk_quotient_many_dev and its _pi_ form
+ *   (round3.py:33, 114-147) with circuits = ncirc rows of the 8 coset evaluations q_l, q_r, q_o, q_m, q_c,
+ *   s_sigma1..3 (N = ext * n each); x, l1f, zh8 depend on n only and are shared.
+ * zkp_fr_gather_many_dev: dst[dst_off + (k * count + j) * len + i] = handles[circuit_of[j] * K + k][i], i < len,
+ *   k < K <= 16: the circuit coefficient vectors each proof reads in rounds 4 and 5 (s_sigma1, s_sigma2 for
+ *   round4.py:39-81; q_m, q_l, q_r, q_o, q_c, s_sigma3 for the linearisation of round5.py:90-160) as per-proof
+ *   blocks at stride len, one launch whatever count and ncirc are; dst must not overlap a source. */
+int zkp_plonk_perm_terms_multi_dev(uint64_t a, uint64_t b, uint64_t c, uint64_t off, uint32_t ncirc, const uint64_t* sigmas,
+                                   const uint32_t* circuit_of, uint64_t n, uint32_t count, const uint8_t omega[32],
+                                   const uint8_t* betas, const uint8_t* gammas, uint64_t num, uint64_t den);
+int zkp_plonk_quotient_multi_dev(uint64_t evals, uint32_t ncirc, const uint64_t* circuits, const uint32_t* circuit_of,
+                                 uint64_t n, uint32_t ext, uint32_t count, uint64_t x, uint64_t l1f, uint64_t zh8,
+                                 const uint8_t* betas, const uint8_t* gammas, const uint8_t* alphas, uint64_t t_out);
+int zkp_plonk_quotient_pi_multi_dev(uint64_t evals, uint32_t ncirc, const uint64_t* circuits, const uint32_t* circuit_of,
+                                    uint64_t n, uint32_t ext, uint32_t count, uint64_t x, uint64_t l1f, uint64_t zh8,
+                                    const uint8_t* betas, const uint8_t* gammas, const uint8_t* alphas, uint64_t t_out);
+int zkp_fr_gather_many_dev(uint32_t ncirc, uint32_t K, const uint64_t* handles, const uint32_t* circuit_of, uint64_t len,
+                           uint32_t count, uint64_t dst, uint64_t dst_off);
 /* General product and exact/long division over Fr in coefficient form
  * (Polynomial.__mul__ polynomial.py:144-159; poly_div polynomial.py:385-435). */
 int zkp_fr_poly_mul(const uint8_t* a, uint64_t a_len, const uint8_t* b, uint64_t b_len, uint8_t* out);

@@ -139,6 +139,13 @@ PROTOTYPES = {
     "zkp_plonk_coset_inputs_pi_many_dev": (c_int, [u64, u64, u64, u64, u64, u32, u32, u64]),
     "zkp_plonk_quotient_pi_many_dev": (c_int, [u64, u64p, u64, u32, u32, u64, u64, u64, vp, vp, vp, u64]),
     "zkp_plonk_pi_eval_many_dev": (c_int, [u64, u64, u64, u64, u64, u32, vp, vp, vp]),
+    "zkp_plonk_perm_terms_multi_dev": (c_int, [u64, u64, u64, u64, u32, u64p, ctypes.POINTER(u32), u64, u32, vp, vp, vp,
+                                               u64, u64]),
+    "zkp_plonk_quotient_multi_dev": (c_int, [u64, u32, u64p, ctypes.POINTER(u32), u64, u32, u32, u64, u64, u64, vp, vp, vp,
+                                             u64]),
+    "zkp_plonk_quotient_pi_multi_dev": (c_int, [u64, u32, u64p, ctypes.POINTER(u32), u64, u32, u32, u64, u64, u64, vp, vp,
+                                                vp, u64]),
+    "zkp_fr_gather_many_dev": (c_int, [u32, u32, u64p, ctypes.POINTER(u32), u64, u32, u64, u64]),
     "zkp_sparse_load": (c_int, [vp, vp, vp, u64, u64, u64, u64p]),
     "zkp_sparse_matvec_dev": (c_int, [u64, u64, u64, u64, u64]),
     "zkp_fr_ap_interpolate_dev": (c_int, [u64, u64, u64, vp, u64, u64]),

@@ -98,15 +98,24 @@ __global__ void __launch_bounds__(DOT_THREADS) plonk_pi_eval_many_kernel(const F
 }
 
 // plonk_perm_terms_kernel for proof j = idx >> log_n with its own beta_j, gamma_j (canonical arrays); the witness of
-// proof j at a/b/c[j * n], sigma shared
+// proof j at a/b/c[j * n].  MULTI = false: sigma shared (s1, s2, s3).  MULTI = true: proof j reads the sigma
+// evaluations of circuit circ[j], sig[3 circ[j] + 0..2] (a separate instantiation, so the one-circuit kernel is unchanged)
+template <bool MULTI>
 __global__ void plonk_perm_terms_many_kernel(const Fr* __restrict__ a, const Fr* __restrict__ b, const Fr* __restrict__ c,
                                              const Fr* __restrict__ s1, const Fr* __restrict__ s2, const Fr* __restrict__ s3,
+                                             const Fr* const* __restrict__ sig, const uint32_t* __restrict__ circ,
                                              uint32_t log_n, const Fr* __restrict__ omega_tab, const Fr* __restrict__ betas,
                                              const Fr* __restrict__ gammas, uint64_t total, Fr* __restrict__ num,
                                              Fr* __restrict__ den) {
   uint64_t idx = IDX64;
   if (idx >= total) return;
   const uint64_t j = idx >> log_n, i = idx & ((uint64_t(1) << log_n) - 1);
+  if (MULTI) {
+    const Fr* const* t = sig + 3 * (uint64_t)circ[j];
+    s1 = t[0];
+    s2 = t[1];
+    s3 = t[2];
+  }
   Fr beta = betas[j].to_mont(), gamma = gammas[j].to_mont();
   Fr w = power_at(omega_tab, (uint32_t)i);
   Fr bw = beta * w;
@@ -115,6 +124,18 @@ __global__ void plonk_perm_terms_many_kernel(const Fr* __restrict__ a, const Fr*
   Fr de = (am + beta * s1[i].to_mont()) * (bm + beta * s2[i].to_mont()) * (cm + beta * s3[i].to_mont());
   num[idx] = nu.from_mont();
   den[idx] = de.from_mont();
+}
+
+// ------------------------------------------------------------------ many circuits of one size per pass
+// dst[(k * count + j) * len + i] = src[circ[j] * K + k][i], i < len: the K circuit vectors proof j needs, gathered
+// from its circuit's data into per-proof blocks, so the strided batch kernels read them like per-proof vectors
+__global__ void fr_gather_many_kernel(const Fr* const* __restrict__ src, const uint32_t* __restrict__ circ, uint32_t K,
+                                      uint64_t count, uint64_t len, uint64_t total, Fr* __restrict__ dst) {
+  uint64_t idx = IDX64;
+  if (idx >= total) return;
+  const uint64_t v = idx / len, i = idx % len;
+  const uint64_t k = v / count, j = v % count;
+  dst[idx] = src[(uint64_t)circ[j] * K + k][i];
 }
 
 // ------------------------------------------------------------------ segmented exclusive scan
@@ -266,31 +287,46 @@ struct PlonkQuotManyArgs {
   const Fr *x, *l1f, *zh_inv;                       // static coset data of the device key
   const Fr *betas, *gammas, *alphas;                // count canonical challenges each
   const Fr* pi;  // with public inputs: count blocks of N, the Montgomery coset evaluations of PI_j (round3.py:33)
+  const Fr* const* circ_tab;  // many circuits: 8 pointers per circuit, in the order of ql .. s3
+  const uint32_t* circ;       // many circuits: the circuit of each proof
   uint64_t count;
   uint32_t log_N, ext;
   Fr* t;  // out: count blocks of N quotient evaluations, Montgomery
 };
 // plonk_quotient_kernel for proof j = idx >> log_N with its own challenges; z(w x) wraps inside proof j's block.
-// PI: q_c + PI_j in the gate term (a separate instantiation, so the kernel without public inputs is unchanged)
-template <bool PI>
+// PI: q_c + PI_j in the gate term.  MULTI: proof j reads the 8 coset evaluations of circuit circ[j] through circ_tab
+// instead of the shared ones.  (Separate instantiations, so the kernel of one circuit without public inputs is unchanged.)
+template <bool PI, bool MULTI>
 __global__ void __launch_bounds__(128) plonk_quotient_many_kernel(PlonkQuotManyArgs q) {
   uint64_t idx = IDX64;
   const uint64_t N = uint64_t(1) << q.log_N;
   if (idx >= q.count * N) return;
   const uint64_t j = idx >> q.log_N, i = idx & (N - 1);
   const uint64_t blk = q.count * N;
+  const Fr *ql = q.ql, *qr = q.qr, *qo = q.qo, *qm = q.qm, *qcp = q.qc, *s1 = q.s1, *s2 = q.s2, *s3 = q.s3;
+  if (MULTI) {
+    const Fr* const* t = q.circ_tab + 8 * (uint64_t)q.circ[j];
+    ql = t[0];
+    qr = t[1];
+    qo = t[2];
+    qm = t[3];
+    qcp = t[4];
+    s1 = t[5];
+    s2 = t[6];
+    s3 = t[7];
+  }
   Fr beta = q.betas[j].to_mont(), gamma = q.gammas[j].to_mont(), alpha = q.alphas[j].to_mont();
   Fr a = q.ev[idx], b = q.ev[blk + idx], c = q.ev[2 * blk + idx];
   const Fr* zj = q.ev + 3 * blk + (j << q.log_N);
   Fr z = zj[i];
   Fr zw = zj[(i + q.ext) & (N - 1)];
-  Fr qc = q.qc[i];
+  Fr qc = qcp[i];
   if (PI) qc = qc + q.pi[idx];
-  Fr gate = q.ql[i] * a + q.qr[i] * b + q.qo[i] * c + q.qm[i] * (a * b) + qc;
+  Fr gate = ql[i] * a + qr[i] * b + qo[i] * c + qm[i] * (a * b) + qc;
   Fr bx = beta * q.x[i];
   Fr ag = a + gamma, bg = b + gamma, cg = c + gamma;
   Fr num = (ag + bx) * (bg + bx.dbl()) * (cg + bx.dbl() + bx) * z;
-  Fr den = (ag + beta * q.s1[i]) * (bg + beta * q.s2[i]) * (cg + beta * q.s3[i]) * zw;
+  Fr den = (ag + beta * s1[i]) * (bg + beta * s2[i]) * (cg + beta * s3[i]) * zw;
   Fr main = (gate + alpha * (num - den)) * q.zh_inv[i & (q.ext - 1)];
   Fr l1 = alpha * alpha * ((z - Fr::one()) * q.l1f[i]);
   q.t[idx] = main + l1;
@@ -426,6 +462,26 @@ static Fr* upload_canon(Context& c, const uint8_t* host, uint64_t n) {
   return d;
 }
 
+// The device side of a many-circuit call: a table of ncirc x per pointers (circuit-major) resolved from the handles,
+// each checked to hold len elements, and the count circuit indices, each checked to be < ncirc.  Both go to the arena
+// (key data is addressed where it is, never copied).
+static void circuit_table(Context& c, const char* what, uint32_t ncirc, uint32_t per, const uint64_t* handles, uint64_t len,
+                          const uint32_t* circuit_of, uint32_t count, const Fr* const** tab, const uint32_t** circ) {
+  if (!ncirc || !handles || (count && !circuit_of)) throw InvalidArgument(std::string(what) + ": null argument or no circuits");
+  std::vector<const Fr*> ptrs((size_t)ncirc * per);
+  for (size_t k = 0; k < ptrs.size(); k++) ptrs[k] = hptr(handles[k], 0, len, what);
+  for (uint32_t j = 0; j < count; j++)
+    if (circuit_of[j] >= ncirc) throw InvalidArgument(std::string(what) + ": circuit index out of range");
+  if (!count) return;
+  Fr* dt = g_arena.alloc((ptrs.size() * sizeof(Fr*) + sizeof(Fr) - 1) / sizeof(Fr));
+  Fr* dc = g_arena.alloc(((uint64_t)count * 4 + sizeof(Fr) - 1) / sizeof(Fr));
+  CUDA_CHECK(cudaMemcpyAsync(dt, ptrs.data(), ptrs.size() * sizeof(Fr*), cudaMemcpyHostToDevice, c.stream));
+  CUDA_CHECK(cudaMemcpyAsync(dc, circuit_of, (size_t)count * 4, cudaMemcpyHostToDevice, c.stream));
+  CUDA_CHECK(cudaStreamSynchronize(c.stream));  // ptrs is freed on return
+  *tab = reinterpret_cast<const Fr* const*>(dt);
+  *circ = reinterpret_cast<const uint32_t*>(dc);
+}
+
 static void pi_check_shape(const char* what, uint64_t n, uint64_t ell, uint64_t stride, uint32_t count) {
   if (!n || (n & (n - 1)) || n > (uint64_t(1) << 28)) throw InvalidArgument(std::string(what) + ": n must be a power of two <= 2^28");
   if (ell > n) throw InvalidArgument(std::string(what) + ": more public inputs than gates");
@@ -449,10 +505,12 @@ static void coset_inputs_many(Context& c, const char* what, uint64_t wires, uint
   c.launches++;
 }
 
-// evals: 4 count blocks of N (a_*, b_*, c_*, z_*), or 5 with PI_* (with_pi)
-static void quotient_many(Context& c, const char* w, uint64_t evals, const uint64_t circuit[8], uint64_t n, uint32_t ext,
+// evals: 4 count blocks of N (a_*, b_*, c_*, z_*), or 5 with PI_* (with_pi).  circuit: the 8 shared coset evaluations,
+// or with multi ncirc x 8 handles, of which proof j uses row circuit_of[j]
+static void quotient_many(Context& c, const char* w, uint64_t evals, const uint64_t* circuit, uint64_t n, uint32_t ext,
                           uint32_t count, uint64_t x, uint64_t l1f, uint64_t zh8, const uint8_t* betas,
-                          const uint8_t* gammas, const uint8_t* alphas, uint64_t t_out, bool with_pi) {
+                          const uint8_t* gammas, const uint8_t* alphas, uint64_t t_out, bool with_pi, bool multi = false,
+                          uint32_t ncirc = 1, const uint32_t* circuit_of = nullptr) {
   if (!circuit || (count && (!betas || !gammas || !alphas))) throw InvalidArgument(std::string(w) + ": null argument");
   if (ext != 4 && ext != 8 && ext != 16) throw InvalidArgument(std::string(w) + ": ext must be 4, 8 or 16");
   const uint64_t N = (uint64_t)ext * n;
@@ -464,7 +522,9 @@ static void quotient_many(Context& c, const char* w, uint64_t evals, const uint6
   q.ev = hptr(evals, 0, nblk * count * N, w);
   q.pi = q.ev + 4 * (uint64_t)count * N;
   const Fr** slots[8] = {&q.ql, &q.qr, &q.qo, &q.qm, &q.qc, &q.s1, &q.s2, &q.s3};
-  for (int k = 0; k < 8; k++) *slots[k] = hptr(circuit[k], 0, N, w);
+  for (int k = 0; k < 8; k++) *slots[k] = multi ? nullptr : hptr(circuit[k], 0, N, w);
+  q.circ_tab = nullptr;
+  q.circ = nullptr;
   q.x = hptr(x, 0, N, w);
   q.l1f = hptr(l1f, 0, N, w);
   q.zh_inv = hptr(zh8, 0, ext, w);
@@ -472,8 +532,9 @@ static void quotient_many(Context& c, const char* w, uint64_t evals, const uint6
   q.count = count;
   q.log_N = log2_ceil(N);
   q.ext = ext;
-  if (!count) return;
   ArenaScope scope;
+  if (multi) circuit_table(c, w, ncirc, 8, circuit, N, circuit_of, count, &q.circ_tab, &q.circ);
+  if (!count) return;
   Fr* ch = g_arena.alloc(3 * (uint64_t)count);
   CUDA_CHECK(cudaMemcpyAsync(ch, betas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
   CUDA_CHECK(cudaMemcpyAsync(ch + count, gammas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
@@ -481,10 +542,55 @@ static void quotient_many(Context& c, const char* w, uint64_t evals, const uint6
   q.betas = ch;
   q.gammas = ch + count;
   q.alphas = ch + 2 * count;
-  if (with_pi) plonk_quotient_many_kernel<true><<<ceil_div((uint64_t)count * N, 128), 128, 0, c.stream>>>(q);
-  else plonk_quotient_many_kernel<false><<<ceil_div((uint64_t)count * N, 128), 128, 0, c.stream>>>(q);
+  const unsigned grid = ceil_div((uint64_t)count * N, 128);
+  if (multi) {
+    if (with_pi) plonk_quotient_many_kernel<true, true><<<grid, 128, 0, c.stream>>>(q);
+    else plonk_quotient_many_kernel<false, true><<<grid, 128, 0, c.stream>>>(q);
+  } else {
+    if (with_pi) plonk_quotient_many_kernel<true, false><<<grid, 128, 0, c.stream>>>(q);
+    else plonk_quotient_many_kernel<false, false><<<grid, 128, 0, c.stream>>>(q);
+  }
   CUDA_CHECK_LAUNCH();
   c.launches++;
+  CUDA_CHECK(cudaStreamSynchronize(c.stream));
+}
+
+// sigma: the 3 shared handles of S_sigma1..3 on H (n each), or with multi ncirc x 3 of them, row circuit_of[j] for proof j
+static void perm_terms_many(Context& c, const char* w, uint64_t a, uint64_t b, uint64_t cc, uint64_t off, bool multi,
+                            uint32_t ncirc, const uint64_t* sigma, const uint32_t* circuit_of, uint64_t n, uint32_t count,
+                            const uint8_t omega[32], const uint8_t* betas, const uint8_t* gammas, uint64_t num,
+                            uint64_t den) {
+  if (!omega || !sigma || (count && (!betas || !gammas))) throw InvalidArgument(std::string(w) + ": null argument");
+  if (!n || (n & (n - 1)) || n > (uint64_t(1) << 28)) throw InvalidArgument(std::string(w) + ": n must be a power of two <= 2^28");
+  const uint64_t total = (uint64_t)count * n;
+  Fr *pa = hptr(a, off, total, w), *pb = hptr(b, off, total, w), *pc = hptr(cc, off, total, w);
+  Fr *p1 = nullptr, *p2 = nullptr, *p3 = nullptr;
+  if (!multi) {
+    p1 = hptr(sigma[0], 0, n, w);
+    p2 = hptr(sigma[1], 0, n, w);
+    p3 = hptr(sigma[2], 0, n, w);
+  }
+  Fr *pn = hptr(num, 0, total, w), *pd = hptr(den, 0, total, w);
+  ArenaScope scope;
+  const Fr* const* tab_s = nullptr;
+  const uint32_t* circ = nullptr;
+  if (multi) circuit_table(c, w, ncirc, 3, sigma, n, circuit_of, count, &tab_s, &circ);
+  if (!count) return;
+  FrBytes ob;
+  memcpy(ob.b, omega, 32);
+  int launches = 0;
+  const Fr* tab = power_table(c, ob, false, log2_ceil(n), &launches);
+  Fr* ch = g_arena.alloc(2 * (uint64_t)count);
+  CUDA_CHECK(cudaMemcpyAsync(ch, betas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
+  CUDA_CHECK(cudaMemcpyAsync(ch + count, gammas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
+  if (multi)
+    plonk_perm_terms_many_kernel<true><<<GRID_1D(total)>>>(pa, pb, pc, p1, p2, p3, tab_s, circ, log2_ceil(n), tab, ch,
+                                                           ch + count, total, pn, pd);
+  else
+    plonk_perm_terms_many_kernel<false><<<GRID_1D(total)>>>(pa, pb, pc, p1, p2, p3, nullptr, nullptr, log2_ceil(n), tab,
+                                                            ch, ch + count, total, pn, pd);
+  CUDA_CHECK_LAUNCH();
+  c.launches += launches + 1;
   CUDA_CHECK(cudaStreamSynchronize(c.stream));
 }
 
@@ -538,25 +644,40 @@ int zkp_plonk_perm_terms_many_dev(uint64_t a, uint64_t b, uint64_t cc, uint64_t 
                                   uint64_t n, uint32_t count, const uint8_t omega[32], const uint8_t* betas,
                                   const uint8_t* gammas, uint64_t num, uint64_t den) {
   return guarded([&](Context& c) {
-    const char* w = "zkp_plonk_perm_terms_many_dev";
-    if (!omega || (count && (!betas || !gammas))) throw InvalidArgument(std::string(w) + ": null argument");
-    if (!n || (n & (n - 1)) || n > (uint64_t(1) << 28)) throw InvalidArgument(std::string(w) + ": n must be a power of two <= 2^28");
-    const uint64_t total = (uint64_t)count * n;
-    Fr *pa = hptr(a, off, total, w), *pb = hptr(b, off, total, w), *pc = hptr(cc, off, total, w);
-    Fr *p1 = hptr(s1, 0, n, w), *p2 = hptr(s2, 0, n, w), *p3 = hptr(s3, 0, n, w);
-    Fr *pn = hptr(num, 0, total, w), *pd = hptr(den, 0, total, w);
-    if (!count) return;
+    const uint64_t sigma[3] = {s1, s2, s3};
+    perm_terms_many(c, "zkp_plonk_perm_terms_many_dev", a, b, cc, off, false, 1, sigma, nullptr, n, count, omega, betas, gammas,
+                    num, den);
+  });
+}
+
+int zkp_plonk_perm_terms_multi_dev(uint64_t a, uint64_t b, uint64_t cc, uint64_t off, uint32_t ncirc, const uint64_t* sigmas,
+                                   const uint32_t* circuit_of, uint64_t n, uint32_t count, const uint8_t omega[32],
+                                   const uint8_t* betas, const uint8_t* gammas, uint64_t num, uint64_t den) {
+  return guarded([&](Context& c) {
+    perm_terms_many(c, "zkp_plonk_perm_terms_multi_dev", a, b, cc, off, true, ncirc, sigmas, circuit_of, n, count, omega, betas, gammas,
+                    num, den);
+  });
+}
+
+int zkp_fr_gather_many_dev(uint32_t ncirc, uint32_t K, const uint64_t* handles, const uint32_t* circuit_of, uint64_t len,
+                           uint32_t count, uint64_t dst, uint64_t dst_off) {
+  return guarded([&](Context& c) {
+    const char* what = "zkp_fr_gather_many_dev";
+    if (!K || K > (uint32_t)MANY_GROUPS || !len) throw InvalidArgument(std::string(what) + ": 1..16 vectors of len > 0");
+    const uint64_t total = (uint64_t)K * count * len;
+    Fr* d = hptr(dst, dst_off, total, what);
     ArenaScope scope;
-    FrBytes ob;
-    memcpy(ob.b, omega, 32);
-    int launches = 0;
-    const Fr* tab = power_table(c, ob, false, log2_ceil(n), &launches);
-    Fr* ch = g_arena.alloc(2 * (uint64_t)count);
-    CUDA_CHECK(cudaMemcpyAsync(ch, betas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
-    CUDA_CHECK(cudaMemcpyAsync(ch + count, gammas, (size_t)count * 32, cudaMemcpyHostToDevice, c.stream));
-    plonk_perm_terms_many_kernel<<<GRID_1D(total)>>>(pa, pb, pc, p1, p2, p3, log2_ceil(n), tab, ch, ch + count, total, pn, pd);
+    const Fr* const* tab = nullptr;
+    const uint32_t* circ = nullptr;
+    circuit_table(c, what, ncirc, K, handles, len, circuit_of, count, &tab, &circ);
+    if (!count) return;
+    for (uint64_t k = 0; k < (uint64_t)ncirc * K; k++) {
+      const Fr* s = hptr(handles[k], 0, len, what);
+      if (s < d + total && d < s + len) throw InvalidArgument(std::string(what) + ": destination overlaps a source");
+    }
+    fr_gather_many_kernel<<<GRID_1D(total)>>>(tab, circ, K, count, len, total, d);
     CUDA_CHECK_LAUNCH();
-    c.launches += launches + 1;
+    c.launches++;
     CUDA_CHECK(cudaStreamSynchronize(c.stream));
   });
 }
@@ -607,6 +728,24 @@ int zkp_plonk_quotient_pi_many_dev(uint64_t evals, const uint64_t circuit[8], ui
   return guarded([&](Context& c) {
     quotient_many(c, "zkp_plonk_quotient_pi_many_dev", evals, circuit, n, ext, count, x, l1f, zh8, betas, gammas, alphas,
                   t_out, true);
+  });
+}
+
+int zkp_plonk_quotient_multi_dev(uint64_t evals, uint32_t ncirc, const uint64_t* circuits, const uint32_t* circuit_of,
+                                 uint64_t n, uint32_t ext, uint32_t count, uint64_t x, uint64_t l1f, uint64_t zh8,
+                                 const uint8_t* betas, const uint8_t* gammas, const uint8_t* alphas, uint64_t t_out) {
+  return guarded([&](Context& c) {
+    quotient_many(c, "zkp_plonk_quotient_multi_dev", evals, circuits, n, ext, count, x, l1f, zh8, betas, gammas, alphas,
+                  t_out, false, true, ncirc, circuit_of);
+  });
+}
+
+int zkp_plonk_quotient_pi_multi_dev(uint64_t evals, uint32_t ncirc, const uint64_t* circuits, const uint32_t* circuit_of,
+                                    uint64_t n, uint32_t ext, uint32_t count, uint64_t x, uint64_t l1f, uint64_t zh8,
+                                    const uint8_t* betas, const uint8_t* gammas, const uint8_t* alphas, uint64_t t_out) {
+  return guarded([&](Context& c) {
+    quotient_many(c, "zkp_plonk_quotient_pi_multi_dev", evals, circuits, n, ext, count, x, l1f, zh8, betas, gammas,
+                  alphas, t_out, true, true, ncirc, circuit_of);
   });
 }
 

@@ -921,6 +921,59 @@ def plonk_pi_eval_many_dev(pub, off, stride, ell, n, omega, zetas):
     return fr_vec_from_bytes(bytes(out), count)
 
 
+# ------------------------------------------------------------------ batch PLONK proving over many circuits of one size
+def _circuit_rows(what, rows, width, circuit_of, count):
+    """rows: per circuit `width` device handles -> (ncirc, flat handle array, circuit index array).  The host lists
+    must have their lengths; the indices are range-checked by the library (one outside [0, 2^32) is passed as
+    2^32 - 1, which no circuit has, instead of wrapping)."""
+    rows = [list(r) for r in rows]
+    if not rows or any(len(r) != width for r in rows):
+        raise ValueError("%s: every circuit needs %d handles" % (what, width))
+    circ = [int(x) for x in circuit_of]
+    if len(circ) != count:
+        raise ValueError("%s: circuit_of has %d entries, needs %d" % (what, len(circ), count))
+    idx = (ctypes.c_uint32 * max(count, 1))(*[x if 0 <= x < 1 << 32 else (1 << 32) - 1 for x in circ])
+    return len(rows), _u64s([h.handle for r in rows for h in r]), idx
+
+
+def plonk_perm_terms_multi_dev(a, b, c, off, sigmas, circuit_of, n, omega, betas, gammas, num, den):
+    """plonk_perm_terms_many_dev where proof j reads the sigma evaluations sigmas[circuit_of[j]] (3 handles each)."""
+    count = len(betas)
+    ch = _fr_rows("plonk_perm_terms_multi_dev: betas, gammas", [betas, gammas], 2, count)
+    nc, tab, idx = _circuit_rows("plonk_perm_terms_multi_dev: sigmas", sigmas, 3, circuit_of, count)
+    check(_lib.lib().zkp_plonk_perm_terms_multi_dev(a.handle, b.handle, c.handle, off, nc, tab, idx, n, count,
+                                                    buf(fe_bytes(omega)), buf(ch[:32 * count]), buf(ch[32 * count:]),
+                                                    num.handle, den.handle))
+
+
+def _quotient_multi(what, evals, circuits8, circuit_of, n, ext, x, l1f, zh8, betas, gammas, alphas, t_out):
+    count = len(betas)
+    ch = _fr_rows(what + ": betas, gammas, alphas", [betas, gammas, alphas], 3, count)
+    nc, tab, idx = _circuit_rows(what + ": circuits", circuits8, 8, circuit_of, count)
+    check(getattr(_lib.lib(), "zkp_" + what)(evals.handle, nc, tab, idx, n, ext, count, x.handle, l1f.handle, zh8.handle, buf(ch[:32 * count]),
+             buf(ch[32 * count:64 * count]), buf(ch[64 * count:]), t_out.handle))
+
+
+def plonk_quotient_multi_dev(evals, circuits8, circuit_of, n, ext, x, l1f, zh8, betas, gammas, alphas, t_out):
+    """plonk_quotient_many_dev where proof j reads the 8 coset evaluations circuits8[circuit_of[j]]."""
+    _quotient_multi("plonk_quotient_multi_dev", evals, circuits8, circuit_of, n, ext, x, l1f, zh8, betas, gammas, alphas,
+                    t_out)
+
+
+def plonk_quotient_pi_multi_dev(evals, circuits8, circuit_of, n, ext, x, l1f, zh8, betas, gammas, alphas, t_out):
+    """plonk_quotient_pi_many_dev where proof j reads the 8 coset evaluations circuits8[circuit_of[j]]."""
+    _quotient_multi("plonk_quotient_pi_multi_dev", evals, circuits8, circuit_of, n, ext, x, l1f, zh8, betas, gammas,
+                    alphas, t_out)
+
+
+def fr_gather_many_dev(rows, circuit_of, length, dst, dst_off=0):
+    """dst[dst_off + (k * count + j) * length ..][:length] = rows[circuit_of[j]][k][:length], count = len(circuit_of),
+    k < K = len(rows[0]) <= 16: per-proof copies of their circuits' vectors, in one launch."""
+    K = len(rows[0]) if rows else 0
+    nc, tab, idx = _circuit_rows("fr_gather_many_dev: rows", rows, K, circuit_of, len(circuit_of))
+    check(_lib.lib().zkp_fr_gather_many_dev(nc, K, tab, idx, length, len(circuit_of), dst.handle, dst_off))
+
+
 # ------------------------------------------------------------------ QAP over {1..k} at scale (SURVEY 8 f2)
 def sparse_load(row_ptr, col_idx, values, rows, cols):
     """CSR matrix with Fr values -> device handle.  row_ptr: rows+1 offsets, col_idx: column of each

@@ -22,6 +22,7 @@ on H, the transcript absorbs append_scalar(b"public_input", x_i) for i = 0..l-1 
 quotient's gate term gains PI on the coset and the linearisation constant gains PI(zeta).  l = 0 is exactly the
 protocol above: nothing extra is hashed and every proof is unchanged.
 """
+import numbers
 import secrets
 
 import numpy as np
@@ -330,13 +331,16 @@ def prove(key, a_vals, b_vals, c_vals, blinds=None, keep=False, public_inputs=No
 _NOT_DIVISIBLE = "제약 다항식이 Z_H(x)로 나누어 떨어지지 않습니다. 회로 또는 witness에 오류가 있습니다."
 # the many-MSMs of one pass: (scalar vectors per proof, padded length - n) -- rounds 1, 2, 3 and 5
 _PASS_MSMS = ((3, 2), (1, 3), (3, 6), (2, 5))
+# the circuit coefficient vectors rounds 4 and 5 read, gathered per proof when a pass holds several circuits
+_GATHERED = ("q_m", "q_l", "q_r", "q_o", "q_c", "s_sigma3", "s_sigma1", "s_sigma2")
 
 
-def plan_chunk(key, count, free_bytes):
+def plan_chunk(key, count, free_bytes, multi=False):
     """Largest number of proofs per pass of prove_batch: within the 32-bit entry and 31-bit bucket numbering of the
     many-MSM (vectors * W * L < 2^32, vectors * buckets < 2^31 at the padded length L of each round's vectors), the
     32-bit batched coset transforms (4 * count * N8 < 2^32, 5 with public inputs), and half of `free_bytes` of device
-    memory at the working set estimated below.  At least 1, at most count."""
+    memory at the working set estimated below.  At least 1, at most count.  multi: a pass of prove_batch_circuits,
+    whose proofs also hold their own copies of the 8 circuit coefficient vectors of rounds 4 and 5 (8n per proof)."""
     from ..groth16.device_prover import _many_msm_shape
     n, N = key.n, key.N8
     pi = 1 if key.num_public_inputs else 0             # one more coset block and one more n-block per proof
@@ -347,6 +351,8 @@ def plan_chunk(key, count, free_bytes):
         limit = min(limit, ((1 << 32) - 1) // (vecs * W * (n + pad)), ((1 << 31) - 1) // (vecs * per))
         msm_ws = max(msm_ws, vecs * (8 * W * (n + pad) + per * (3 * 128 + 12)))   # entries; buckets and levels
     per_proof = msm_ws + 32 * ((9 + pi) * N + (20 + pi) * n + 64)  # coset blocks, transform scratch, per-round vectors
+    if multi:
+        per_proof += 32 * len(_GATHERED) * n
     limit = min(limit, (free_bytes // 2) // per_proof)
     return int(max(1, min(limit, count)))
 
@@ -361,32 +367,12 @@ def prove_batch(key, a_vals, b_vals, c_vals, count, blinds=None, chunk=None, pub
     naming the first failing proof, before any round-3 commitment of its chunk.
     public_inputs: for a key with l = num_public_inputs > 0, a scalar handle of count * l values, proof j's at j * l
     (as witness.solve_batch returns them); proof j then equals prove(..., public_inputs=those l values)."""
-    n = key.n
     count = int(count)
-    ell = key.num_public_inputs
     if key.ranks is not None:
         raise ValueError("prove_batch: a sharded key is not supported (batch over one GPU's SRS)")
-    if ell and (public_inputs is None or public_inputs.n < count * ell):
-        raise ValueError("prove_batch: public_inputs holds %s values, needs %d"
-                         % (None if public_inputs is None else public_inputs.n, count * ell))
-    if not ell and public_inputs is not None:
-        raise ValueError("prove_batch: the key has no public inputs (preprocess with num_public_inputs)")
-    if chunk is not None and int(chunk) <= 0:
-        raise ValueError("prove_batch: chunk must be positive")
-    if count < 0:
-        raise ValueError("prove_batch: count must be >= 0")
-    for name, h in (("a_vals", a_vals), ("b_vals", b_vals), ("c_vals", c_vals)):
-        if h is None or h.n < count * n:
-            raise ValueError("prove_batch: %s holds %s values, needs %d" % (name, None if h is None else h.n, count * n))
-    if blinds is not None:
-        blinds = [list(b) for b in blinds]
-        if len(blinds) != count or any(len(b) != 9 for b in blinds):
-            raise ValueError("prove_batch: blinds must be %d lists of 9 scalars" % count)
+    blinds = _batch_arguments("prove_batch", key, a_vals, b_vals, c_vals, count, blinds, chunk, public_inputs)
     if count == 0:
         return []
-    if blinds is None:
-        blinds = [[secrets.randbelow(R) for _ in range(9)] for _ in range(count)]
-    blinds = [[int(b) % R for b in bl] for bl in blinds]
     step = min(int(chunk), count) if chunk is not None else plan_chunk(key, count, native.device_mem_info()[0])
     proofs = []
     for j0 in range(0, count, step):
@@ -394,7 +380,83 @@ def prove_batch(key, a_vals, b_vals, c_vals, count, blinds=None, chunk=None, pub
     return proofs
 
 
-def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds, pub):
+def _batch_arguments(what, key, a_vals, b_vals, c_vals, count, blinds, chunk, public_inputs):
+    """The checks of prove_batch's arguments before any device call (ValueError); returns the blinds as count rows of 9
+    reduced ints, fresh from `secrets` when blinds is None."""
+    n, ell = key.n, key.num_public_inputs
+    if ell and (public_inputs is None or public_inputs.n < count * ell):
+        raise ValueError("%s: public_inputs holds %s values, needs %d"
+                         % (what, None if public_inputs is None else public_inputs.n, count * ell))
+    if not ell and public_inputs is not None:
+        raise ValueError("%s: the key has no public inputs (preprocess with num_public_inputs)" % what)
+    if chunk is not None and int(chunk) <= 0:
+        raise ValueError("%s: chunk must be positive" % what)
+    if count < 0:
+        raise ValueError("%s: count must be >= 0" % what)
+    for name, h in (("a_vals", a_vals), ("b_vals", b_vals), ("c_vals", c_vals)):
+        if h is None or h.n < count * n:
+            raise ValueError("%s: %s holds %s values, needs %d" % (what, name, None if h is None else h.n, count * n))
+    if blinds is not None:
+        blinds = [list(b) for b in blinds]
+        if len(blinds) != count or any(len(b) != 9 for b in blinds):
+            raise ValueError("%s: blinds must be %d lists of 9 scalars" % (what, count))
+    if blinds is None:
+        blinds = [[secrets.randbelow(R) for _ in range(9)] for _ in range(count)]
+    return [[int(b) % R for b in bl] for bl in blinds]
+
+
+def _same_table(t, u):
+    return t is u or (getattr(t, "handle", None) is not None and getattr(t, "handle", None) == getattr(u, "handle", None))
+
+
+def prove_batch_circuits(keys, circuits, a_vals, b_vals, c_vals, blinds=None, chunk=None, public_inputs=None):
+    """count = len(circuits) proofs of several circuits of one size in the passes of prove_batch: proof j proves the
+    circuit of keys[circuits[j]] from the wire values at offset j * n of a_vals, b_vals, c_vals, with blinds[j] and
+    (for keys with l public inputs) the l values at j * l of public_inputs, as in prove_batch.  Proof j is
+    bit-identical to prove(keys[circuits[j]], a_j, b_j, c_j, blinds=blinds[j], public_inputs=...); a key may serve
+    any number of proofs, none included.  PLONK's SRS is universal, so every commitment group of a pass stays one
+    many-MSM over the one table; the circuit-dependent work reads each proof's circuit through a per-proof index (the
+    permutation terms and the quotient) or per-proof copies of its 8 coefficient vectors (rounds 4 and 5).
+    ValueError before any device call unless the keys are non-empty, of one n, one SRS table, one number of public
+    inputs and none of them sharded, every index is in [0, len(keys)), and the other arguments pass prove_batch's
+    checks.  An unsatisfied witness raises prove_batch's ValueError naming the first failing proof."""
+    what = "prove_batch_circuits"
+    keys = list(keys)
+    if not keys:
+        raise ValueError("%s: no keys" % what)
+    key = keys[0]
+    for k in keys:
+        if k.ranks is not None:
+            raise ValueError("%s: a sharded key is not supported (batch over one GPU's SRS)" % what)
+        if k.n != key.n:
+            raise ValueError("%s: the keys differ in n (%d and %d); group circuits by size" % (what, key.n, k.n))
+        if not _same_table(k.srs_table, key.srs_table):
+            raise ValueError("%s: the keys do not share one SRS table" % what)
+        if k.num_public_inputs != key.num_public_inputs:
+            raise ValueError("%s: the keys differ in num_public_inputs (%d and %d)"
+                             % (what, key.num_public_inputs, k.num_public_inputs))
+    circuits = list(circuits)
+    for j, c in enumerate(circuits):
+        if isinstance(c, bool) or not isinstance(c, numbers.Integral) or not 0 <= c < len(keys):
+            raise ValueError("%s: circuit index %r of proof %d is outside [0, %d)" % (what, c, j, len(keys)))
+    circuits = [int(c) for c in circuits]
+    count = len(circuits)
+    blinds = _batch_arguments(what, key, a_vals, b_vals, c_vals, count, blinds, chunk, public_inputs)
+    if count == 0:
+        return []
+    step = min(int(chunk), count) if chunk is not None else plan_chunk(key, count, native.device_mem_info()[0], multi=True)
+    proofs = []
+    for j0 in range(0, count, step):
+        cnt = min(step, count - j0)
+        proofs.extend(_prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds, public_inputs,
+                                   (keys, circuits[j0:j0 + cnt])))
+    return proofs
+
+
+def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds, pub, multi=None):
+    """Proofs j0 .. j0 + cnt - 1 in one pass.  multi = None: every proof is of `key`'s circuit.  multi = (keys, circ):
+    proof j0 + i is of keys[circ[i]] (all of key's n, SRS table and public-input count); the circuit data is then read
+    through per-proof indices (rounds 2 and 3) and per-proof gathered coefficient blocks (rounds 4 and 5)."""
     n, log_n, w, N = key.n, key.log_n, key.omega, key.N8
     ell = key.num_public_inputs
     nb = 4 if ell else 3                                    # transform blocks per proof in round 1; + 1 in round 3
@@ -432,7 +494,12 @@ def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds, pub):
         zc = alloc(cnt * n)
         if n > 1:
             num, den = alloc(cnt * n), alloc(cnt * n)
-            native.plonk_perm_terms_many_dev(a_vals, b_vals, c_vals, j0 * n, *key.sigma_evals, n, w, betas, gammas, num, den)
+            if multi:
+                native.plonk_perm_terms_multi_dev(a_vals, b_vals, c_vals, j0 * n, [k.sigma_evals for k in multi[0]], multi[1],
+                                                  n, w, betas, gammas, num, den)
+            else:
+                native.plonk_perm_terms_many_dev(a_vals, b_vals, c_vals, j0 * n, *key.sigma_evals, n, w, betas, gammas, num,
+                                                 den)
             native.batch_inverse_dev(den, 0, cnt * n)
             native.vec_op_dev(2, num, 0, num, 0, den, 0, cnt * n)
             native.scan_many_dev(0, zc, 0, num, 0, n, cnt)  # z_j,0 = 1 in every proof
@@ -453,8 +520,13 @@ def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds, pub):
             native.plonk_coset_inputs_many_dev(wires, z, n, cnt, key.log_n + key.log_ext, ext)
         native.ntt_many_dev(ext, 0, log_n + key.log_ext, (nb + 1) * cnt, key.omega8, coset_shift=COSET_SHIFT)
         t = alloc(cnt * N)
-        quotient = native.plonk_quotient_pi_many_dev if ell else native.plonk_quotient_many_dev
-        quotient(ext, [key.coset[k] for k in CIRCUIT_POLYS], n, key.ext, key.x, key.l1f, key.zh8, betas, gammas, alphas, t)
+        if multi:
+            quotient = native.plonk_quotient_pi_multi_dev if ell else native.plonk_quotient_multi_dev
+            quotient(ext, [[k.coset[p] for p in CIRCUIT_POLYS] for k in multi[0]], multi[1], n, key.ext, key.x, key.l1f,
+                     key.zh8, betas, gammas, alphas, t)
+        else:
+            quotient = native.plonk_quotient_pi_many_dev if ell else native.plonk_quotient_many_dev
+            quotient(ext, [key.coset[k] for k in CIRCUIT_POLYS], n, key.ext, key.x, key.l1f, key.zh8, betas, gammas, alphas, t)
         native.ntt_many_dev(t, 0, log_n + key.log_ext, cnt, key.omega8, inverse=True, coset_shift=COSET_SHIFT)
         bad = native.plonk_divisible_many_dev(t, n, key.ext, cnt)
         if bad is not None:
@@ -468,11 +540,17 @@ def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds, pub):
                 tr.append_point(part.encode() + b"_comm", getattr(prf, part + "_comm"))
         # ---- round 4: 6 cnt evaluations in one batched set of Horner launches
         zetas = [int(tr.challenge_scalar(b"zeta")) for tr in trs]
+        if multi:                                           # the circuit coefficients of rounds 4 and 5, per proof
+            gc = alloc(len(_GATHERED) * cnt * n)
+            native.fr_gather_many_dev([[k.coeffs[p] for p in _GATHERED] for k in multi[0]], multi[1], n, gc)
+            coef = lambda name: (gc, _GATHERED.index(name) * cnt * n, n, n)
+        else:
+            coef = lambda name: (key.coeffs[name], 0, 0, n)
         zws = [zeta * w % R for zeta in zetas]
         wl = cnt * (n + 2)
         evals = native.fr_poly_eval_many_dev(
             [(wires, 0, n + 2, n + 2, 0), (wires, wl, n + 2, n + 2, 0), (wires, 2 * wl, n + 2, n + 2, 0),
-             (key.coeffs["s_sigma1"], 0, 0, n, 0), (key.coeffs["s_sigma2"], 0, 0, n, 0), (z, 0, n + 3, n + 3, 1)],
+             coef("s_sigma1") + (0,), coef("s_sigma2") + (0,), (z, 0, n + 3, n + 3, 1)],
             cnt, [zetas, zws])
         names = ("a_eval", "b_eval", "c_eval", "s_sigma1_eval", "s_sigma2_eval", "z_omega_eval")
         for j, (prf, tr) in enumerate(zip(proofs, trs)):
@@ -497,7 +575,7 @@ def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds, pub):
             p_rows.append([1, zeta_n, zeta_n * zeta_n % R, v] + [pow(v, e, R) for e in range(2, 7)] + [0])
         r = alloc(cnt * (n + 3))
         native.lincomb_many_dev(r, 0, n + 3, n + 3, cnt,
-                                [(key.coeffs[k], 0, 0, n) for k in ("q_m", "q_l", "q_r", "q_o", "q_c", "s_sigma3")]
+                                [coef(k) for k in ("q_m", "q_l", "q_r", "q_o", "q_c", "s_sigma3")]
                                 + [(z, 0, n + 3, n + 3)], r_rows)
         r_evals = native.fr_poly_eval_many_dev([(r, 0, n + 3, n + 3, 0)], cnt, [zetas])[0]
         tl = cnt * (n + 6)
@@ -505,7 +583,7 @@ def _prove_chunk(key, a_vals, b_vals, c_vals, j0, cnt, blinds, pub):
         native.lincomb_many_dev(P, 0, n + 6, n + 6, cnt,
                                 [(ts, 0, n + 6, n), (ts, tl, n + 6, n), (ts, 2 * tl, n + 6, n + 6), (r, 0, n + 3, n + 3),
                                  (wires, 0, n + 2, n + 2), (wires, wl, n + 2, n + 2), (wires, 2 * wl, n + 2, n + 2),
-                                 (key.coeffs["s_sigma1"], 0, 0, n), (key.coeffs["s_sigma2"], 0, 0, n)], p_rows)
+                                 coef("s_sigma1"), coef("s_sigma2")], p_rows)
         # W_j (n + 5) and Ww_j (n + 2, zero-padded to n + 5: a zero scalar adds nothing) in one many-MSM
         Wb = alloc(2 * cnt * (n + 5))
         native.div_linear_many_dev(P, 0, n + 6, n + 6, zetas, Wb, 0, n + 5)

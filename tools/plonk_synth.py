@@ -36,6 +36,46 @@ def chain_circuit(n, seed=1, break_witness=False):
     return {"n": n, "a": a, "b": b, "c": c, "sel": [q_l, q_r, q_o, q_m, q_c], "sigma": sigma}
 
 
+def random_circuit(n, seed=1, witness_seed=None, break_witness=False):
+    """A satisfiable circuit of n gates whose structure is drawn from `seed`: every gate is a multiplication
+    (c = a b), an addition (c = a + b) or an addition of a constant (c = a + k, q_c = k), and each of its a and b is,
+    with probability 1/2, a copy of the output of an earlier gate (a copy constraint) or a fresh input.  Two seeds give
+    circuits with different selectors and sigma.  witness_seed (default: seed) draws the fresh inputs, so one circuit
+    has many witnesses; break_witness adds 1 to one output."""
+    rng = random.Random(seed)
+    kinds, const, src_a, src_b = [], [], [], []
+    for g in range(n):
+        kinds.append(rng.randrange(3))
+        const.append(rng.randrange(1, 1 << 60))
+        src_a.append(rng.randrange(g) if g and rng.random() < 0.5 else None)
+        src_b.append(rng.randrange(g) if g and rng.random() < 0.5 else None)
+    vals = random.Random(seed if witness_seed is None else witness_seed)
+    a, b, c = [0] * n, [0] * n, [0] * n
+    q_l, q_r, q_o, q_m, q_c = ([0] * n for _ in range(5))
+    cycles = {}                                          # gate p -> wire positions holding c_p (c_p itself first)
+    for g in range(n):
+        x = c[src_a[g]] if src_a[g] is not None else vals.randrange(1, 1 << 60)
+        y = c[src_b[g]] if src_b[g] is not None else vals.randrange(1, 1 << 60)
+        a[g], b[g] = x, y
+        q_o[g] = R - 1
+        if kinds[g] == 0:
+            q_m[g], c[g] = 1, x * y % R
+        elif kinds[g] == 1:
+            q_l[g], q_r[g], c[g] = 1, 1, (x + y) % R
+        else:
+            q_l[g], q_c[g], c[g] = 1, const[g], (x + const[g]) % R
+        for p, pos in ((src_a[g], g), (src_b[g], n + g)):
+            if p is not None:
+                cycles.setdefault(p, [2 * n + p]).append(pos)
+    sigma = list(range(3 * n))
+    for cyc in cycles.values():                          # each copy class one cycle of the permutation
+        for i, pos in enumerate(cyc):
+            sigma[pos] = cyc[(i + 1) % len(cyc)]
+    if break_witness:
+        c[n // 2] = (c[n // 2] + 1) % R
+    return {"n": n, "a": a, "b": b, "c": c, "sel": [q_l, q_r, q_o, q_m, q_c], "sigma": sigma}
+
+
 def prepend_public_gates(circ, tied, n=None, public_inputs=None):
     """The circuit `circ` (keys n, a, b, c, sel, sigma) behind len(tied) public-input gates, padded with zero gates to n
     gates (default: the smallest power of two that fits).  Gate i has q_l = -1, so with the PI term it reads
@@ -89,6 +129,41 @@ def sigma_evals_bytes(sigma, n, omega):
     for part in range(3):
         out.append(b"".join(table[32 * sigma[part * n + i]:32 * sigma[part * n + i] + 32] for i in range(n)))
     return out
+
+
+def device_srs(size, srs_tau=None, precompute=True):
+    """An SRS table of `size` G1 powers tau^i G on the device (prefix product + fixed-base kernel) -> (table, tau)."""
+    tau = srs_tau or 0x1d0c2e3f4a5b6c7d8e9fa0b1c2d3e4f5061728394a5b6c7d8e9f0011223344 % R
+    powers = nat.fr_prefix_product(nat.fr_vec_bytes([tau] * size), size)
+    srs = nat.g1_fixed_base_mul(nat.g1_bytes((1, 2)), powers, size)
+    if precompute and size >= (1 << 12):
+        nat.table_precompute(srs)
+    return srs, tau
+
+
+def device_key(circ, srs, srs_size):
+    """The circuit uploaded and preprocessed against an existing SRS table -> (key, witness handles).  Keys made this
+    way against one table can share the passes of device_prover.prove_batch_circuits."""
+    from interactive_zkp_study_b200.zkp.plonk import device_prover as dp
+    from interactive_zkp_study_b200.zkp.plonk.field import get_root_of_unity
+    n = circ["n"]
+    omega = int(get_root_of_unity(n))
+    enc = nat.fr_vec_bytes
+    sel_h = [nat.scalars_load(enc(v), n) for v in circ["sel"]]
+    sig_h = [nat.scalars_load(bts, n) for bts in sigma_evals_bytes(circ["sigma"], n, omega)]
+    key = dp.preprocess(n, sel_h, sig_h, srs, srs_size, num_public_inputs=circ.get("num_public_inputs", 0))
+    return key, [nat.scalars_load(enc(circ[k]), n) for k in "abc"]
+
+
+def device_setup_many(circs, srs_tau=None, precompute=True):
+    """Several circuits of one size preprocessed against ONE SRS table (device_setup builds a table per call).
+    Returns (keys, witness handles per circuit, tau)."""
+    n = circs[0]["n"]
+    if any(c["n"] != n for c in circs):
+        raise ValueError("device_setup_many: the circuits differ in size")
+    srs, tau = device_srs(n + 6, srs_tau, precompute)
+    keys, wits = zip(*[device_key(c, srs, n + 6) for c in circs])
+    return list(keys), list(wits), tau
 
 
 def device_setup(circ, srs_tau=None, precompute=True, comm=None):
