@@ -29,15 +29,19 @@ int zkp_imad_peak(int variant, double* gmacs_per_s, double* sm_clock_mhz_effecti
  * on a lone thread / the same with a broadcast after each).
  * The MSM's reduction tail is bounded by these, not by throughput. */
 int zkp_latency_probe(int mode, double* ns_per_op);
-/* Field-op self-test hooks used by tests/ (field: 0 = Fp, 1 = Fr, 2 = Fp2 with 64-byte elements c0 || c1 and
- * ops 2 / 3 / 4 / 9 only; op: 0 add, 1 sub, 2 mul, 3 inv, 4 sqr,
+/* Field-op self-test hooks used by tests/ (field: 0 = Fp, 1 = Fr, 2 = Fp2 with 64-byte elements c0 || c1).
+ * Fp / Fr op: 0 add, 1 sub, 2 mul, 3 inv, 4 sqr,
  * 5 Fermat inverse, 6 mul as 512-bit product + separate Montgomery reduction, 7 inverse by binary extended Euclid,
  * 8 a b - (a + b)(a - b) through the lazily reduced product pair of the group formulas' Y coordinate,
- * 9 the square root of the point decoder (csrc/point_codec.cuh; Fp and Fp2 only), all-ones bytes when a is not a
- * square) */
+ * 9 the square root of the point decoder (csrc/point_codec.cuh; Fp only), all-ones bytes when a is not a square.
+ * Fp2 op: 0 add, 1 sub, 2 mul, 3 inv, 4 sqr, 5 sqr with inlined Fp products (Fp2::sqr_inline_products), 6 mul with
+ * its body inlined (fp2_mul_inline) -- 5 and 6 are the forms of the G2 bucket-accumulation loop -- and 9 the square
+ * root as above; ops 7 and 8 are refused. */
 int zkp_dbg_field_op(int field, int op, const uint8_t* a, const uint8_t* b, uint64_t n, uint8_t* out);
-/* out[i] = a[i] + b[i] (group: 0 = G1, 1 = G2; 2 / 3 = the same through the quad-lane operations of
- * csrc/ec_quad.cuh) via XYZZ, result affine; exercises all edge cases */
+/* out[i] = a[i] + b[i], affine (64-byte G1 / 128-byte G2 points; odd groups are G2).  group 0 / 1: XYZZ mixed then
+ * full addition; 2 / 3: the quad-lane operations of csrc/ec_quad.cuh; 4 / 5: the mixed addition of the MSM's
+ * bucket-accumulation loop (csrc/msm_acc.cuh acc_madd) of b onto a held with ZZ != 1; 6 / 7: XYZZ full addition of
+ * a and b held with different ZZ != 1 (the bucket fold).  Every edge case: infinity operands, P + P, P + (-P). */
 int zkp_dbg_point_add(int group, const uint8_t* a, const uint8_t* b, uint64_t n, uint8_t* out);
 /* Fp12 self-test hook (csrc/pairing.cu): n elements of 384 B each in py_ecc's FQ12 basis (12 canonical
  * coefficients of w^0..w^11); op: 0 a * b, 1 a^2, 2 cyclotomic squaring (valid for a in the cyclotomic subgroup),

@@ -6,6 +6,7 @@
 #include "../../include/zkp_b200_diag.h"
 #include "ec.cuh"
 #include "ec_quad.cuh"
+#include "msm_acc.cuh"
 #include "point_codec.cuh"
 #include "registry.cuh"
 
@@ -314,14 +315,19 @@ __global__ void dbg_field_op_kernel(int op, const FE* a, const FE* b, uint64_t n
   out[i] = r.from_mont();
 }
 
-// Fp2 products / squarings / inverses of n pairs (64-byte elements c0 || c1, canonical)
+// Fp2 ops of n pairs (64-byte elements c0 || c1, canonical); the host refuses ops not listed here (7, 8)
 __global__ void dbg_fp2_op_kernel(int op, const Fp2* a, const Fp2* b, uint64_t n, Fp2* out) {
   uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   Fp2 x = a[i].to_mont(), y = b ? b[i].to_mont() : Fp2::zero(), r;
   switch (op) {
+    case 0: r = x + y; break;
+    case 1: r = x - y; break;
     case 2: r = x * y; break;
     case 3: r = x.inv(); break;
+    case 4: r = x.sqr(); break;
+    case 5: r = x.sqr_inline_products(); break;  // the squaring of the G2 accumulation loop (msm_acc.cuh AccMul2)
+    case 6: r = fp2_mul_inline(x, y); break;     // the product of its P + P path, body inlined
     case 9:
       if (!fp2_sqrt(x, r)) {
         for (int k = 0; k < 8; k++) r.c0.v[k] = r.c1.v[k] = ~0u;
@@ -329,7 +335,7 @@ __global__ void dbg_fp2_op_kernel(int op, const Fp2* a, const Fp2* b, uint64_t n
         return;
       }
       break;
-    default: r = x.sqr(); break;
+    default: return;
   }
   out[i] = r.from_mont();
 }
@@ -346,6 +352,40 @@ __global__ void dbg_point_add_kernel(const Affine<F>* a, const Affine<F>* b, uin
   XYZZ<F> z = XYZZ<F>::inf();
   z.add(acc);
   Affine<F> r = z.to_affine();
+  out[i] = {r.x.from_mont(), r.y.from_mont()};
+}
+
+// A fixed non-zero field element (Montgomery form) that differs with `salt`: the Z scale of the operands below
+template <class F>
+ZKP_DEVINL F dbg_scale(uint32_t salt) {
+  F r;
+  uint32_t* w = reinterpret_cast<uint32_t*>(&r);
+  for (int k = 0; k < (int)(sizeof(F) / 4); k++) w[k] = (0x9e3779b9u * (k + salt)) & ((k & 7) == 7 ? 0x0fffffffu : ~0u);
+  return r;
+}
+// p in XYZZ coordinates with ZZ = l^2, ZZZ = l^3 (l = dbg_scale(salt)): the same point as from_affine(p), so an equal
+// or opposite operand arrives with a different Z, as partial sums of a bucket do
+template <class F>
+ZKP_DEVINL XYZZ<F> dbg_rescaled(const Affine<F>& p, uint32_t salt) {
+  if (p.is_inf()) return XYZZ<F>::inf();
+  const F l = dbg_scale<F>(salt), l2 = l * l, l3 = l2 * l;
+  return {p.x * l2, p.y * l3, l2, l3};
+}
+
+// The group-law steps of the MSM's bucket pipeline with operands whose ZZ != 1 (zkp_dbg_point_add groups 4 - 7).
+// acc: the accumulation loop's mixed addition (acc_madd<F, MSM_ACC_OUTLINE>: AccMul / AccMul2, what
+// msm_accumulate_kernel runs) of b onto a rescaled a.  Otherwise XYZZ::add of rescaled a and b with different scales
+// (what the bucket fold and the continuation of a part-streamed MSM run; F is the fold's field flavour).
+template <class F, bool ACC>
+__global__ void dbg_point_acc_kernel(const Affine<F>* a, const Affine<F>* b, uint64_t n, Affine<F>* out) {
+  uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  Affine<F> p = {a[i].x.to_mont(), a[i].y.to_mont()};
+  Affine<F> q = {b[i].x.to_mont(), b[i].y.to_mont()};
+  XYZZ<F> acc = dbg_rescaled(p, 1);
+  if constexpr (ACC) acc_madd<F, MSM_ACC_OUTLINE>(acc, q);
+  else acc.add(dbg_rescaled(q, 5));
+  Affine<F> r = acc.to_affine();
   out[i] = {r.x.from_mont(), r.y.from_mont()};
 }
 
@@ -443,6 +483,7 @@ int zkp_dbg_field_op(int field, int op, const uint8_t* a, const uint8_t* b, uint
     if (!a || !out || op < 0 || op > 9) throw InvalidArgument("zkp_dbg_field_op: bad argument");
     if (n == 0) return;
     if (field < 0 || field > 2) throw InvalidArgument("zkp_dbg_field_op: field must be 0 (Fp), 1 (Fr) or 2 (Fp2)");
+    if (field == 2 && (op == 7 || op == 8)) throw InvalidArgument("zkp_dbg_field_op: Fp2 has ops 0 - 6 and 9 only");
     if (op == 9 && field == 1) throw InvalidArgument("zkp_dbg_field_op: the square root is for Fp and Fp2 (p = 3 mod 4)");
     const size_t sz = field == 2 ? 64 : 32;
     ScopedDevBuf da, db, dout;
@@ -472,7 +513,9 @@ int zkp_dbg_point_add(int group, const uint8_t* a, const uint8_t* b, uint64_t n,
   return guarded([&](Context& c) {
     if (!a || !b || !out) throw InvalidArgument("zkp_dbg_point_add: null argument");
     if (n == 0) return;
-    if (group < 0 || group > 3) throw InvalidArgument("zkp_dbg_point_add: group must be 0 (G1), 1 (G2), 2 / 3 (the same on quads of lanes)");
+    if (group < 0 || group > 7)
+      throw InvalidArgument("zkp_dbg_point_add: group must be 0 (G1) / 1 (G2), 2 / 3 (quads of lanes), 4 / 5 (accumulation "
+                            "step), 6 / 7 (XYZZ full addition)");
     size_t sz = (group & 1) == 0 ? 64 : 128;
     ScopedDevBuf da, db, dout;
     da.reserve(n * sz);
@@ -480,7 +523,19 @@ int zkp_dbg_point_add(int group, const uint8_t* a, const uint8_t* b, uint64_t n,
     dout.reserve(n * sz);
     CUDA_CHECK(cudaMemcpyAsync(da.p, a, n * sz, cudaMemcpyHostToDevice, c.stream));
     CUDA_CHECK(cudaMemcpyAsync(db.p, b, n * sz, cudaMemcpyHostToDevice, c.stream));
-    if (group == 2)
+    if (group == 4)
+      dbg_point_acc_kernel<Fp, true><<<ceil_div(n, 64), 64, 0, c.stream>>>(da.as<G1Affine>(), db.as<G1Affine>(), n,
+                                                                          dout.as<G1Affine>());
+    else if (group == 5)
+      dbg_point_acc_kernel<Fp2, true><<<ceil_div(n, 64), 64, 0, c.stream>>>(da.as<G2Affine>(), db.as<G2Affine>(), n,
+                                                                           dout.as<G2Affine>());
+    else if (group == 6)  // the G1 fold adds in the compact flavour (same layout)
+      dbg_point_acc_kernel<FpC, false><<<ceil_div(n, 64), 64, 0, c.stream>>>(
+          da.as<Affine<FpC>>(), db.as<Affine<FpC>>(), n, dout.as<Affine<FpC>>());
+    else if (group == 7)
+      dbg_point_acc_kernel<Fp2, false><<<ceil_div(n, 64), 64, 0, c.stream>>>(da.as<G2Affine>(), db.as<G2Affine>(), n,
+                                                                            dout.as<G2Affine>());
+    else if (group == 2)
       dbg_point_add_quad_kernel<Fp><<<ceil_div(4 * n, 64), 64, 0, c.stream>>>(da.as<G1Affine>(), db.as<G1Affine>(), n,
                                                                              dout.as<G1Affine>());
     else if (group == 3)

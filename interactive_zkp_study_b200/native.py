@@ -687,7 +687,8 @@ def dbg_field_op(field, op, a_bytes, b_bytes, n):
 
 
 def dbg_point_add(group, a_bytes, b_bytes, n):
-    sz = 64 if group == 0 else 128
+    """include/zkp_b200_diag.h zkp_dbg_point_add: even groups are G1 (64-byte points), odd ones G2 (128 bytes)."""
+    sz = 128 if group & 1 else 64
     out = bytearray(sz * n)
     check(_lib.lib().zkp_dbg_point_add(group, buf(a_bytes), buf(b_bytes), n, buf(out)))
     return bytes(out)

@@ -7,6 +7,7 @@ import random
 import pytest
 
 from oracle import bn254, synthetic
+from tests.msm_groups import Group, auto_c, edge_cases
 
 pytestmark = pytest.mark.gpu
 R = bn254.R
@@ -39,19 +40,50 @@ def test_g1_msm_empty_is_infinity(native):
     assert native.g1_msm(b"", b"", 0) is None
 
 
-@pytest.mark.parametrize("c", [2, 5, 9, 13, 14, 16, 18, 20])
-def test_g1_msm_every_window_width(native, c):
+@pytest.mark.parametrize("c,group", [pytest.param(c, "g1", id=str(c)) for c in (2, 3, 5, 9, 13, 14, 16, 18, 20)]
+                         + [pytest.param(c, "g2", id="g2-%d" % c) for c in (2, 3, 5, 9, 13, 16, 18, 20)])
+def test_g1_msm_every_window_width(native, c, group):
+    """Every window width on G1 and G2, plain and window-precomputed tables, with a repeated point and a P / -P pair
+    under equal scalars in the data (P + P and P + (-P) inside a bucket at every width)."""
     rng = random.Random(200 + c)
-    pts = _points_g1(rng, 300)
-    scalars = [rng.randrange(R) for _ in range(300)]
-    native.set_window_bits(c)
+    grp = Group(native, group)
+    n = 300 if group == "g1" else 200
+    # a plain table's MSM holds ceil(255 / c) windows of 2^(c-1) XYZZ buckets (twice the affine size: 256 B on G2),
+    # 1.7 GB for G2 at c = 20
+    free, _ = native.device_mem_info()
+    assert free > 4 * ((255 + c - 1) // c) * (1 << (c - 1)) * 2 * grp.size
     try:
-        _check_g1(native, pts, scalars)
+        native.set_window_bits(c)
+        if group == "g1":
+            pts = _points_g1(rng, 300)
+            scalars = [rng.randrange(R) for _ in range(300)]
+            _check_g1(native, pts, scalars)
+        dlogs = [rng.randrange(1, R) for _ in range(n)]
+        dlogs[7] = dlogs[3]
+        dlogs[11] = R - dlogs[10]
+        dlogs[n - 1] = dlogs[0]
+        k = [rng.randrange(R) for _ in range(n)]
+        k[7] = k[3]
+        k[11] = k[10]
+        k[n - 1] = k[0] = R - 1
+        want = grp.want(dlogs, k)
+        table = grp.table(dlogs)
+        assert grp.msm_points(table, n, k) == want
+        assert grp.msm_table(table, 0, native.fr_vec_bytes(k), n) == want
+        native.set_window_bits(0)
+        assert native.table_precompute(table, c) == c
+        assert grp.msm_table(table, 0, native.fr_vec_bytes(k), n) == want
+        sc = native.scalars_load(native.fr_vec_bytes(k), n)
+        assert grp.msm_dev(table, 0, sc, 0, n) == want
     finally:
         native.set_window_bits(0)
 
 
 def test_g1_msm_edge_distributions(native):
+    """The edge distributions on G1 against the oracle's MSM, then at the window width the engine picks over
+    known-discrete-log tables (tests/msm_groups.py edge_cases, shared with the G2 test below): P + P in the
+    accumulation loop and in the fold, P + (-P), infinity entries, unreduced scalars, digits that carry in every
+    window."""
     rng = random.Random(5)
     n = 200
     pts = _points_g1(rng, n)
@@ -72,6 +104,22 @@ def test_g1_msm_edge_distributions(native):
     _check_g1(native, with_inf, [rng.randrange(R) for _ in range(n)])  # infinity points in the table
     _check_g1(native, pts, [(1 << 16) - 1] * n)                        # digit carries
     _check_g1(native, pts, [1 << 15] * n)                              # digit == B exactly
+    _check_edge_cases(native, Group(native, "g1"), rng, 256)
+
+
+def test_g2_msm_edge_distributions(native):
+    """The edge distributions of the G1 test above on G2, whose accumulation loop (AccMul2) and fold have their own
+    copies of the group law."""
+    _check_edge_cases(native, Group(native, "g2"), random.Random(5), 256)
+
+
+def _check_edge_cases(native, grp, rng, n):
+    tables = {}
+    for name, dlogs, k in edge_cases(rng, n, auto_c(n)):
+        key = id(dlogs)
+        if key not in tables:
+            tables[key] = grp.table(dlogs)
+        assert grp.msm_points(tables[key], n, k) == grp.want(dlogs, k), name
 
 
 def test_g1_msm_table_and_dev_paths_agree(native):

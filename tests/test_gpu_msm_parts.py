@@ -8,6 +8,7 @@ import random
 import pytest
 
 from oracle import bn254
+from tests.msm_groups import Group, plus_minus
 
 pytestmark = pytest.mark.gpu
 R = bn254.R
@@ -54,12 +55,17 @@ def test_parts_match_oracle(parts, k, pre):
     assert parts.g1_combine_partials(p0 + p1, 2) == want
 
 
-@pytest.mark.parametrize("c", [3, 9])
-def test_parts_edge_distributions(parts, c):
+@pytest.mark.parametrize("c,group", [pytest.param(c, "g1", id=str(c)) for c in (3, 9)]
+                         + [pytest.param(c, "g2", id="g2-%d" % c) for c in (3, 9)])
+def test_parts_edge_distributions(parts, c, group):
     """One scalar for everything: every window has one bucket that each part cuts into several tasks (fold onto the
-    earlier parts' sum); P / -P pairs that cancel across and inside parts; empty later parts (zero scalars)."""
+    earlier parts' sum); P / -P pairs that cancel across and inside parts; empty later parts (zero scalars).  G1
+    against the oracle's MSM, G2 on known-discrete-log tables."""
     rng = random.Random(2200 + c)
     n = 600
+    if group == "g2":
+        _edge_distributions_dlog(parts, Group(parts, group), rng, c, n)
+        return
     pts = _points_g1(rng, n)
     table = parts.g1_table_load(parts.g1_vec_bytes(pts), n)
     parts.set_window_bits(c)
@@ -84,6 +90,27 @@ def test_parts_edge_distributions(parts, c):
     same = [pts[0]] * n                                                        # P + P when a later part continues a bucket
     t4 = parts.g1_table_load(parts.g1_vec_bytes(same), n)
     check(t4, same, [99] * n)
+
+
+def _edge_distributions_dlog(native, grp, rng, c, n):
+    native.set_window_bits(c)
+    native.msm_set_option("parts", 4)
+    base = [rng.randrange(1, R) for _ in range(n)]
+    cases = [
+        (base, [0x1234567] * n),
+        (base, [1] * n),
+        (base, [rng.randrange(R) for _ in range(150)] + [0] * 450),     # parts 1..3 add nothing
+        (base, [0] * 450 + [rng.randrange(R) for _ in range(150)]),     # only the last part adds
+        (base, [0] * n),
+        (plus_minus(base[:n // 2]), [777] * n),
+        (base[:300] + [R - s for s in base[:300]], [424242] * n),     # cancels across parts: buckets return to infinity
+        ([base[0]] * n, [99] * n),                                     # P + P when a later part continues a bucket
+    ]
+    tables = {}
+    for i, (dlogs, k) in enumerate(cases):
+        if id(dlogs) not in tables:
+            tables[id(dlogs)] = grp.table(dlogs)
+        assert grp.msm_table(tables[id(dlogs)], 0, native.fr_vec_bytes(k), n) == grp.want(dlogs, k), i
 
 
 def test_parts_g2(parts):

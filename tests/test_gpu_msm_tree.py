@@ -8,6 +8,7 @@ import random
 import pytest
 
 from oracle import bn254, synthetic
+from tests.msm_groups import Group, auto_c, edge_cases
 
 pytestmark = pytest.mark.gpu
 R = bn254.R
@@ -60,6 +61,8 @@ def test_tree_every_window_width_and_batch(tree, c, items, rounds):
 
 
 def test_tree_edge_distributions(tree):
+    """G1 against the oracle's MSM, then over known-discrete-log tables (tests/msm_groups.py edge_cases, shared with
+    the G2 test below) in the default and in the late tree rounds."""
     rng = random.Random(15)
     n = 200
     pts = _points_g1(rng, n)
@@ -87,6 +90,23 @@ def test_tree_edge_distributions(tree):
     _check_g1(tree, [pts[0]] * n, [12345] * n)
     _check_g1(tree, pm, [777] * n)
     _check_g1(tree, with_inf, [5] * n)
+    tree.msm_set_option("tree_rounds", 0)
+    _edge_cases_dlog(tree, Group(tree, "g1"), rng)
+
+
+def test_tree_g2_edge_distributions(tree):
+    _edge_cases_dlog(tree, Group(tree, "g2"), random.Random(15))
+
+
+def _edge_cases_dlog(native, grp, rng, n=256):
+    cases = edge_cases(rng, n, auto_c(n))
+    tables = {}
+    for rounds in (0, 9):
+        native.msm_set_option("tree_rounds", rounds)
+        for name, dlogs, k in cases:
+            if id(dlogs) not in tables:
+                tables[id(dlogs)] = grp.table(dlogs)
+            assert grp.msm_points(tables[id(dlogs)], n, k) == grp.want(dlogs, k), (name, rounds)
 
 
 def test_tree_and_heavy_buckets_side_by_side(tree):

@@ -14,6 +14,7 @@ import sys
 import pytest
 
 from oracle import bn254, synthetic
+from tests.msm_groups import Group
 
 pytestmark = pytest.mark.gpu
 R = bn254.R
@@ -146,11 +147,23 @@ def test_large_msm_device_verified(native, log_n, pre_c):
 
 
 def test_skewed_scalars_at_2p17(native):
+    _skewed_scalars_at_2p17(native, "g1")
+
+
+def test_g2_skewed_scalars_at_2p17(native):
+    _skewed_scalars_at_2p17(native, "g2")
+
+
+def _skewed_scalars_at_2p17(native, group):
     """Skewed digit distributions at a size where buckets are cut into many tasks: all scalars equal (every
-    window's digits land in one bucket), half of them zero, tiny scalars (only the lowest window used), r - 1."""
+    window's digits land in one bucket), half of them zero, tiny scalars (only the lowest window used), r - 1; on a
+    plain and on a window-precomputed table.  Then all points equal under all scalars equal: every task's partial sum
+    is 64 P, so the block-per-bucket fold adds equal sums (P + P) at every level of its tree."""
     n = 1 << 17
-    table, s_h, _ = _known_dlog_table(native, n, 0x5EED0102)
-    native.table_precompute(table, 17)
+    grp = Group(native, group)
+    s_h = native.scalars_generate(0x5EED0102, n)
+    spot = {i: native.fr_vec_from_bytes(native.scalars_download(s_h, i, 1))[0] for i in (0, n - 1)}
+    table = grp.table_dev(s_h, n, spot)
     rng = random.Random(4)
     k0 = rng.randrange(R)
     cases = {
@@ -159,11 +172,19 @@ def test_skewed_scalars_at_2p17(native):
         "tiny": [rng.randrange(1, 1000) for _ in range(n)],
         "r - 1": [R - 1] * n,
     }
-    for name, k in cases.items():
-        k_h = native.scalars_load(native.fr_vec_bytes(k), n)
-        want = bn254.g1_mul(bn254.G1, native.fr_dot_dev(k_h, 0, s_h, 0, n))
-        assert native.g1_msm_dev(table, 0, k_h, 0, n) == want, name
-        k_h.free()
+    same_h = native.scalars_load(native.fr_vec_bytes([k0] * n), n)
+    same = grp.table_dev(same_h, n, {0: k0, n - 1: k0})      # every entry k0 * G
+    for pre in (0, 17):
+        if pre:
+            native.table_precompute(table, pre)
+            native.table_precompute(same, pre)
+        for name, k in cases.items():
+            k_h = native.scalars_load(native.fr_vec_bytes(k), n)
+            want = grp.mul(native.fr_dot_dev(k_h, 0, s_h, 0, n))
+            assert grp.msm_dev(table, 0, k_h, 0, n) == want, (name, pre)
+            k_h.free()
+        # all points equal, all scalars equal: n k0^2 * G
+        assert grp.msm_dev(same, 0, same_h, 0, n) == grp.mul(n * k0 * k0), ("all points equal", pre)
 
 
 def test_groth16_prove_sharded_equals_single_gpu(native, comm):
